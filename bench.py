@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- AAConv2d fwd+bwd throughput on B200 (BASELINE.json metric, configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision bf16|fp32] [--shape T1|T2|T3|T1_512]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision bf16|fp32] [--shape T1|T2|T3|T1_512] [--dump-outputs DIR]
     python bench.py --impl reference ...      # the reference algorithm's CPU port on the host cores
 
 A step = one forward + backward of the AAConv2d module at the Transition-1 shape (B=16 per GPU, 256 ch,
@@ -19,6 +19,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -82,6 +83,26 @@ class ClockSampler(threading.Thread):
         return {'sm_mhz': s[len(s) // 2] if s else None, 'sm_max_mhz': self.max_mhz, 'reasons': sorted(self.reasons)}
 
 
+DUMP_ELEMENTS = 15 << 20      # float32 elements written by --dump-outputs in all: 60 MiB
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each tensor of `arrays` (name -> tensor) as out_dir/<name>.npy in float32.  The smaller tensors are written
+    whole, in their shape; a tensor beyond its share of DUMP_ELEMENTS is written as a flat sample at a fixed set of flat indices
+    (torch.randperm seeded with 0, sorted), the same for every run with the same arguments, so two builds compare element for
+    element."""
+    os.makedirs(out_dir, exist_ok=True)
+    left, todo = DUMP_ELEMENTS, sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(todo):
+        cap = left // (len(todo) - i)
+        a = t.detach().float().cpu()
+        if a.numel() > cap:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + '.npy'), a.numpy())
+        left -= a.numel()
+
+
 def cpu_port(shape, B, steps, warmup, threads):
     """The reference algorithm (oracle port of attn_aug_conv.py:65-97 + autograd) on the host cores."""
     from oracle import aaconv_oracle as O
@@ -112,7 +133,7 @@ def run_reference(args):
     cin, hin, cout, dk, dv = SHAPES[args.shape]
     B = args.ref_batch
     W = min(args.warmup, 1)
-    K = min(args.steps, args.ref_max_steps)        # ~0.8 s per B=16 step on 16 threads: bounded so the arm ends within minutes
+    K = args.steps if args.ref_max_steps is None else min(args.steps, args.ref_max_steps)   # ~0.8 s per B=16 step on 16 threads
     sec = cpu_port(args.shape, B, K, W, threads)
     tf = 3 * flops_fwd(B, cin, hin, cout, dk, dv) / sec / 1e12
     line = {'impl': 'reference', 'metric': 'aaconv_fwd_bwd_tflops', 'value': tf, 'unit': 'TFLOP/s', 'n_gpus': args.gpus,
@@ -158,9 +179,10 @@ class Ctx:
         return t.tolist()
 
 
-def measure_model(ctx, args, K, W, cuda_graph, sampler=None):
+def measure_model(ctx, args, K, W, cuda_graph, sampler=None, dump_dir=None):
     """configs[2]: whole-model data-parallel training step of aadensenet121 (chexpert.py:152-165) on synthetic radiographs:
-    forward, BCE loss, backward with the bucketed NCCL gradient all-reduce, SGD-nesterov.  -> dict (rank 0 uses it)."""
+    forward, BCE loss, backward with the bucketed NCCL gradient all-reduce, SGD-nesterov.  -> dict (rank 0 uses it).
+    `dump_dir`: the loss of the last timed step and the parameters it left go there (dump_outputs)."""
     from chexpert_b200 import _lib
     from chexpert_b200.train import TrainStep, synthetic_batch
     dev, world, rank = ctx.dev, ctx.world, ctx.rank
@@ -190,15 +212,19 @@ def measure_model(ctx, args, K, W, cuda_graph, sampler=None):
         ts(x, t)
     ctx.barrier()
     l0 = _lib.launch_count()
-    ms = timed(lambda: ts(x, t), K)
+    last = {}
+    ms = timed(lambda: last.update(loss=ts(x, t)), K)
     launches = _lib.launch_count() - l0
     if cuda_graph:          # replays do not pass through the host-side launch counter: count what one replay holds
         launches = ts.graph_launches * K
+    if dump_dir and rank == 0:      # before the steps below overwrite the captured graph's output and the parameters
+        last.update(('param_' + n.replace('.', '_'), p) for n, p in ts.model.named_parameters())
+        dump_outputs(dump_dir, last)
     ctx.barrier()
     for _ in range(2):
         e2e_step()
     ctx.barrier()
-    ms_e2e = timed(e2e_step, max(3, K // 2))
+    ms_e2e = timed(e2e_step, K)
     ctx.barrier()
     ms, ms_e2e = ctx.max_over_ranks(ms, ms_e2e)
     out = {'images_per_s': B * world / (ms * 1e-3), 'ms_per_step': ms, 'steps': K, 'warmup': W, 'n_gpus': world,
@@ -220,7 +246,7 @@ def run_model(args):
     W, K = max(args.warmup, 3), args.steps
     sampler = ClockSampler(ctx.local)
     sampler.start()
-    m = measure_model(ctx, args, K, W, args.cuda_graph)
+    m = measure_model(ctx, args, K, W, args.cuda_graph, dump_dir=args.dump_outputs)
     sampler.stop_flag = True
     sampler.join(timeout=2)
     if ctx.rank == 0:
@@ -258,10 +284,11 @@ def ncu_traffic(kernel):
     return j.get('kernels', {}).get(kernel), j.get('source')
 
 
-def measure_layer(ctx, args, shape, K, W, want_e2e=True, sampler=None):
+def measure_layer(ctx, args, shape, K, W, want_e2e=True, sampler=None, dump_dir=None):
     # args.io_dtype: element type of x / dy / y at the module boundary ('fp32' as the reference module, or 'bf16' = the
     # activations torch.autocast hands the Transition in the bf16 training configuration, configs[2])
-    """One AAConv2d forward + backward at a Transition shape through the public nn.Module (configs[1]).  -> dict."""
+    """One AAConv2d forward + backward at a Transition shape through the public nn.Module (configs[1]).  -> dict.
+    `dump_dir`: y, dx and the (all-reduced) parameter gradients of the last timed step go there (dump_outputs)."""
     import chexpert_b200 as cb
     from chexpert_b200 import _lib
     dev, world, rank, dist = ctx.dev, ctx.world, ctx.rank, ctx.dist
@@ -285,15 +312,17 @@ def measure_layer(ctx, args, shape, K, W, want_e2e=True, sampler=None):
     flush_buf = torch.empty(256 << 20, dtype=torch.uint8, device=dev)   # > 126 MB L2
 
     def step(xin, dyin):
+        """-> y and the all-reduced parameter gradients (one flat tensor; None on one GPU, where p.grad is the result)."""
         for p in params:
             p.grad = None
         xin.grad = None
         y = m(xin)
         y.backward(dyin)
+        flat = None
         if world > 1:   # data-parallel exchange step: one bucket with every parameter gradient of the module, averaged by NCCL
             flat = torch.cat([p.grad.reshape(-1) for p in params])
             dist.all_reduce(flat, op=dist.ReduceOp.AVG)
-        return y
+        return y, flat
 
     def timed(fn, n):
         """n calls, each bracketed by its own CUDA events on the current stream; L2 flushed in between."""
@@ -313,11 +342,19 @@ def measure_layer(ctx, args, shape, K, W, want_e2e=True, sampler=None):
         step(x, dy)
     ctx.barrier()
     l0 = _lib.launch_count()
+    last = {}
     t_wall = time.perf_counter()
-    ms = timed(lambda: step(x, dy), K)
+    ms = timed(lambda: last.update(out=step(x, dy)), K)
     ctx.barrier()
     t_wall = time.perf_counter() - t_wall
     launches = _lib.launch_count() - l0
+    if dump_dir and rank == 0:
+        y, flat = last['out']
+        grads = ([p.grad for p in params] if flat is None else
+                 [g.view_as(p) for g, p in zip(flat.split([p.numel() for p in params]), params)])
+        outs = {'y': y, 'grad_x': x.grad}
+        outs.update(('grad_' + n.replace('.', '_'), g) for (n, _), g in zip(m.named_parameters(), grads))
+        dump_outputs(dump_dir, outs)
     out = {'shape': shape, 'ms': ms, 'launches': launches, 't_wall': t_wall, 'h2d': 0, 'd2h': 0, 'ms_e2e': None,
            'io_dtype': 'bf16' if io_t == torch.bfloat16 else 'fp32'}
 
@@ -354,7 +391,7 @@ def measure_layer(ctx, args, shape, K, W, want_e2e=True, sampler=None):
             if k + 1 < state['n']:
                 upload(i ^ 1)                                # next step's inputs travel while this step computes
             cur.wait_event(ready[i])
-            y = step(xbuf[i].detach().requires_grad_(True), dybuf[i])
+            y, _ = step(xbuf[i].detach().requires_grad_(True), dybuf[i])
             freed[i].record(cur)
             cur.wait_event(drained[i])
             ystage[i].copy_(y.detach())
@@ -387,7 +424,7 @@ def measure_layer(ctx, args, shape, K, W, want_e2e=True, sampler=None):
 
         e2e_timed(3)
         ctx.barrier()
-        out['ms_e2e'] = e2e_timed(max(6, K // 2))
+        out['ms_e2e'] = e2e_timed(K)
         ctx.barrier()
         out['h2d'] = x_host.numel() * x_host.element_size() + dy_host.numel() * dy_host.element_size()
         out['d2h'] = y_host.numel() * y_host.element_size() + sum(t.numel() * 4 for t in g_host)
@@ -469,7 +506,8 @@ def main():
     ap.add_argument('--shape', default='T1', choices=list(SHAPES))
     ap.add_argument('--batch', type=int, default=16)
     ap.add_argument('--ref-batch', type=int, default=16, help='per-step batch of the CPU reference arm (same config as ours)')
-    ap.add_argument('--ref-max-steps', type=int, default=20, help='cap on the timed steps of the CPU reference arm')
+    ap.add_argument('--ref-max-steps', type=int, default=None,
+                    help='optional cap on the timed steps of the CPU reference arm (default: --steps, ~0.8 s each at B=16)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-flush', action='store_true')
     ap.add_argument('--no-model', action='store_true', help='skip the whole-model training measurement (`model` field)')
@@ -485,7 +523,15 @@ def main():
     ap.add_argument('--size', type=int, default=320)
     ap.add_argument('--channels-last', action='store_true', help='model workload: channels_last memory format for the dense blocks')
     ap.add_argument('--cuda-graph', action='store_true', help='model workload: capture the whole training step in a CUDA graph')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed to DIR/<name>.npy (float32; layer: y, grad_x and the parameter '
+                         'gradients, model: loss and the updated parameters); inputs are seeded, so runs with the same arguments '
+                         'compare output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the CUDA path (--impl ours)')
     if args.impl == 'reference':
         return run_reference(args)
     if args.workload == 'model':
@@ -495,18 +541,18 @@ def main():
     W, K = max(args.warmup, 3), args.steps
     sampler = ClockSampler(ctx.local)
     sampler.start()
-    layer = measure_layer(ctx, args, args.shape, K, W, want_e2e=True)
+    layer = measure_layer(ctx, args, args.shape, K, W, want_e2e=True, dump_dir=args.dump_outputs)
     other = None                                     # the same layer through the other boundary element type (reported beside)
     if args.precision == 'bf16' and ctx.world == 1:
         keep = args.io_dtype
         args.io_dtype = 'fp32' if keep == 'bf16' else 'bf16'
-        other = measure_layer(ctx, args, args.shape, max(5, K // 2), 3, want_e2e=True)
+        other = measure_layer(ctx, args, args.shape, K, 3, want_e2e=True)
         args.io_dtype = keep
     shapes = {}
     if ctx.world == 1 and not args.no_shapes:
         for sh in ('T2', 'T3', 'T1_512'):
             if sh != args.shape:
-                shapes[sh] = measure_layer(ctx, args, sh, max(5, K // 2), 3, want_e2e=False)
+                shapes[sh] = measure_layer(ctx, args, sh, K, 3, want_e2e=False)
     sampler.stop_flag = True
     sampler.join(timeout=2)
     clocks = sampler.summary()
@@ -514,7 +560,7 @@ def main():
     graph = not args.model_eager
     if not args.no_model:
         try:
-            model = measure_model(ctx, args, max(10, K), max(W, 4), cuda_graph=graph)
+            model = measure_model(ctx, args, K, max(W, 4), cuda_graph=graph)
         except Exception as e:   # the headline layer numbers are still printed
             model = {'error': f'{type(e).__name__}: {e}'[:300]}
 
@@ -528,7 +574,7 @@ def main():
         for sh, r in shapes.items():
             rf = roofline_of(r, args, clocks, 1)
             srows[sh] = {'ms_per_step': r['ms'], 'tflops': r['flops'] / (r['ms'] * 1e-3) / 1e12,
-                         'frac_of_bf16_peak': r['flops'] / (r['ms'] * 1e-3) / 1e12 / peak_tf, 'launches_per_step': r['launches'] / max(5, K // 2),
+                         'frac_of_bf16_peak': r['flops'] / (r['ms'] * 1e-3) / 1e12 / peak_tf, 'launches_per_step': r['launches'] / K,
                          'dominant_kernel': rf['kernel'] if rf else None, 'dominant_us': rf['us_per_launch'] if rf else None,
                          'dominant_frac': rf['frac'] if rf else None}
         line = {'metric': 'aaconv_fwd_bwd_tflops', 'value': tf, 'unit': 'TFLOP/s', 'n_gpus': world, 'steps': K, 'warmup': W,

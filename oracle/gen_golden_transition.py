@@ -56,7 +56,10 @@ def main():
     for name, cfg in CASES.items():
         for dtype, tag in ((torch.float64, 'f64'),):
             rec = run_case(name, cfg, dtype)
-            np.savez_compressed(os.path.join(OUT, f'transition_{name}_{tag}.npz'), **rec)
+            # the inputs (x, dy, parameters) go to a second part so that no file exceeds 1 MB (tests/helpers.py: load_fixture)
+            inputs = {k: v for k, v in rec.items() if k in ('x', 'dy') or k.startswith('p.')}
+            np.savez_compressed(os.path.join(OUT, f'transition_{name}_{tag}.npz'), **{k: v for k, v in rec.items() if k not in inputs})
+            np.savez_compressed(os.path.join(OUT, f'transition_{name}_{tag}.part2.npz'), **inputs)
             print(name, tag, {k: v.shape for k, v in rec.items()})
 
 

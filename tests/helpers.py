@@ -16,6 +16,16 @@ def golden_cases(tag):
                   for f in glob.glob(os.path.join(GOLDEN, f'aaconv_*_{tag}.npz')))
 
 
+def load_fixture(stem):
+    """tests/golden/<stem>.npz together with its parts <stem>.part*.npz -> {name: array}.  A fixture whose arrays would make one
+    file larger than 1 MB is stored split across such parts; the arrays themselves are the generator's, unchanged."""
+    z = {}
+    for f in [os.path.join(GOLDEN, stem + '.npz')] + sorted(glob.glob(os.path.join(GOLDEN, stem + '.part*.npz'))):
+        with np.load(f) as part:
+            z.update((k, part[k]) for k in part.files)
+    return z
+
+
 def load_case(name, tag):
     z = np.load(os.path.join(GOLDEN, f'aaconv_{name}_{tag}.npz'))
     B, Cin, Hin, Win, Cout, ks, st, dk, dv, nh, rel = (int(v) for v in z['cfg'])

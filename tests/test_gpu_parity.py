@@ -5,7 +5,7 @@ import pytest
 import torch
 
 from oracle import aaconv_oracle as O
-from tests.helpers import GOLDEN, autocast_reference, golden_cases, load_case, rel_err, rel_l2
+from tests.helpers import GOLDEN, autocast_reference, golden_cases, load_case, load_fixture, rel_err, rel_l2
 
 pytestmark = pytest.mark.gpu
 
@@ -305,10 +305,10 @@ def test_tiny_densenet_matches_reference_fixture():
     import chexpert_b200 as cb
     torch.backends.cudnn.allow_tf32 = False          # the dense blocks are torch/cuDNN: keep them in true fp32
     torch.backends.cuda.matmul.allow_tf32 = False
-    z = np.load(os.path.join(GOLDEN, 'tiny_densenet.npz'))
+    z = load_fixture('tiny_densenet')
     m = DenseNet(16, (2, 2, 2, 2), 32, num_classes=5,
                  attn_params={'k': 0.5, 'v': 0.5, 'nh': 8, 'relative': True, 'input_dims': (64, 64)}, precision='fp32')
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith('sd.')}
+    sd = {k[3:]: torch.from_numpy(z[k]) for k in z if k.startswith('sd.')}
     m.load_state_dict(sd, strict=True)
     m = m.cuda().train()
     out = m(torch.from_numpy(z['x']).cuda())
@@ -317,7 +317,7 @@ def test_tiny_densenet_matches_reference_fixture():
     assert torch.allclose(out.cpu(), torch.from_numpy(z['out']), rtol=1e-3, atol=1e-4)
     assert torch.allclose(loss.cpu(), torch.from_numpy(z['loss']), rtol=1e-4)
     for k, prm in m.named_parameters():
-        if 'g.' + k in z.files:
+        if 'g.' + k in z:
             assert rel_err(prm.grad.cpu(), torch.from_numpy(z['g.' + k])) < 2e-3, k
 
 

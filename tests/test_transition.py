@@ -8,17 +8,16 @@
 import glob
 import os
 
-import numpy as np
 import pytest
 import torch
 
-from tests.helpers import GOLDEN, rel_err, rel_l2
+from tests.helpers import GOLDEN, load_fixture, rel_err, rel_l2
 
 CASES = sorted(os.path.basename(f)[len('transition_'):-len('_f64.npz')] for f in glob.glob(os.path.join(GOLDEN, 'transition_*_f64.npz')))
 
 
 def _load(name):
-    z = np.load(os.path.join(GOLDEN, f'transition_{name}_f64.npz'))
+    z = load_fixture(f'transition_{name}_f64')
     B, Cin, Hin, Win, Cout, dk, dv, nh = (int(v) for v in z['cfg'])
     return z, (B, Cin, Hin, Win, Cout, dk, dv, nh)
 
@@ -30,7 +29,7 @@ def _transition(z, cfg, precision, fused):
     attn = {'k': 0.0, 'v': dv / Cout, 'nh': nh, 'relative': True, 'input_dims': (Hin, Win)}
     m = AATransition(Cin, Cout, attn, precision=precision, fused_prologue=fused)
     assert (m.conv.dk, m.conv.dv) == (dk, dv)
-    sd = {k[2:]: torch.from_numpy(z[k]).float() for k in z.files if k.startswith('p.')}
+    sd = {k[2:]: torch.from_numpy(z[k]).float() for k in z if k.startswith('p.')}
     m.load_state_dict(sd, strict=True)        # same keys as the reference _Transition: conv.conv.weight, conv.key_rel_h, ...
     return m.cuda()
 
@@ -157,11 +156,11 @@ def test_tiny_densenet_buffered_fused_matches_reference_fixture():
     import chexpert_b200 as cb
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
-    z = np.load(os.path.join(GOLDEN, 'tiny_densenet.npz'))
+    z = load_fixture('tiny_densenet')
     m = DenseNet(16, (2, 2, 2, 2), 32, num_classes=5,
                  attn_params={'k': 0.5, 'v': 0.5, 'nh': 8, 'relative': True, 'input_dims': (64, 64)}, precision='fp32',
                  feature_buffer=True, fused_prologue=True)
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith('sd.')}
+    sd = {k[3:]: torch.from_numpy(z[k]) for k in z if k.startswith('sd.')}
     m.load_state_dict(sd, strict=True)
     m = m.cuda().train()
     out = m(torch.from_numpy(z['x']).cuda())
@@ -170,7 +169,7 @@ def test_tiny_densenet_buffered_fused_matches_reference_fixture():
     assert torch.allclose(out.cpu(), torch.from_numpy(z['out']), rtol=1e-3, atol=1e-4)
     assert torch.allclose(loss.cpu(), torch.from_numpy(z['loss']), rtol=1e-4)
     for k, prm in m.named_parameters():
-        if 'g.' + k in z.files:
+        if 'g.' + k in z:
             assert rel_err(prm.grad.cpu(), torch.from_numpy(z['g.' + k])) < 2e-3, k
 
 
