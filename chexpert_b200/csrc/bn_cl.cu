@@ -128,6 +128,8 @@ __global__ void __launch_bounds__(256) bn_fin_bwd_kernel(const float2* __restric
 // hidden by CTAs, not inside one (300 CTAs: 19 us per call on average; see profiles/r02_b_scaling.md)
 constexpr int T_RED_CTAS = 2368;
 constexpr int CL_ROWS = 256;   // most rows per CTA of the reduction kernels (the host picks 32..256 so that every SM gets a few CTAs)
+// most channels of an NHWC input: cl_stats keeps a thread's segment means in registers, 4 quads of at most 256 threads per row
+constexpr int CL_MAX_C = 4 * 4 * 256;
 
 // red[slot][c] -> fixed-order sum over the 256 / TPR row slots for channel c (c < C), result broadcast through red[0][c]
 __device__ __forceinline__ void reduce_slots(float* red, int C, int nslot) {
@@ -154,7 +156,7 @@ __global__ void __launch_bounds__(256) cl_stats_kernel(const T* __restrict__ x, 
     *reinterpret_cast<float4*>(red + slot * C + 4 * q) = s;
   }
   reduce_slots(red, C, nslot);
-  float4 mean[4];                                         // up to 4 quads per thread (C <= 4 * 4 * TPR)
+  float4 mean[4];                                         // up to 4 quads per thread (C <= 4 * 4 * TPR <= CL_MAX_C)
   const float inv = 1.f / (float)nr;
   int k = 0;
   for (int q = q0; q < Q; q += TPR, ++k) {
@@ -615,6 +617,7 @@ int aaconv_bn_relu_cl_forward(const void* x, int dtype, int B, int C, int HW, in
   if (!x || !weight || !bias || !y_cl || !saved || !workspace || B <= 0 || C <= 0 || HW <= 0 || (C & 3) || (HW & 3))
     return fail(AACONV_E_ARG, "bad bn_relu_cl_forward arguments (C and HW must be multiples of 4)");
   if (dtype != AACONV_FP32 && dtype != AACONV_BF16) return fail(AACONV_E_ARG, "bad bn_relu_cl dtype");
+  if (x_is_cl && C > CL_MAX_C) return fail(AACONV_E_ARG, "bn_relu_cl_forward: an NHWC input has at most 4096 channels");
   if (!x_is_cl && (!nchw_stats || stats_groups <= 0 || planes_per_group <= 0 || x_batch_stride < (int64_t)C * HW))
     return fail(AACONV_E_ARG, "bn_relu_cl_forward: NCHW input needs its group statistics and batch stride");
   const size_t elt = dtype == AACONV_BF16 ? 2 : 4;
@@ -638,6 +641,7 @@ int aaconv_bn_relu_cl_backward(const void* x, int dtype, int B, int C, int HW, i
   if (!x || !dy_cl || !saved || !weight || !bias || !workspace || B <= 0 || C <= 0 || HW <= 0 || (C & 3) || (HW & 3))
     return fail(AACONV_E_ARG, "bad bn_relu_cl_backward arguments (C and HW must be multiples of 4)");
   if (dtype != AACONV_FP32 && dtype != AACONV_BF16) return fail(AACONV_E_ARG, "bad bn_relu_cl dtype");
+  if (x_is_cl && C > CL_MAX_C) return fail(AACONV_E_ARG, "bn_relu_cl_backward: an NHWC input has at most 4096 channels");
   const size_t elt = dtype == AACONV_BF16 ? 2 : 4;
   if (!aligned4(x, elt) || !aligned4(dy_cl, elt) || (dx && !aligned4(dx, elt)) ||
       (!x_is_cl && (((size_t)x_batch_stride * elt) % (4 * elt) || (dx && ((size_t)dx_batch_stride * elt) % (4 * elt)))))

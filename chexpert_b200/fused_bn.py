@@ -140,11 +140,15 @@ def _is_cl(t):
     return t.dim() == 4 and t.is_contiguous(memory_format=_CL)
 
 
+CL_MAX_C = 4096   # channels of an NHWC input the statistics kernel keeps in registers (csrc/bn_cl.cu, CL_MAX_C)
+
+
 def cl_ok(bn, x):
-    """The channels-last kernels cover training-mode BatchNorm2d on CUDA with C and H*W multiples of 4."""
+    """The channels-last kernels cover training-mode BatchNorm2d on CUDA with C and H*W multiples of 4, and at most CL_MAX_C
+    channels when x itself is channels-last."""
     B, C, H, W = x.shape
     return (bn.training and x.is_cuda and x.dtype in _DT and bn.affine and bn.track_running_stats and bn.momentum is not None
-            and C % 4 == 0 and (H * W) % 4 == 0 and B <= 65535)
+            and C % 4 == 0 and (H * W) % 4 == 0 and B <= 65535 and (C <= CL_MAX_C or not _is_cl(x)))
 
 
 def _bump(bn):

@@ -169,7 +169,7 @@ int aaconv_bn_relu_backward_acc(const void* x, int dtype, int B, int C, int HW, 
 
 /* Channels-last side of the dense layers (chexpert_b200/csrc/bn_cl.cu): cuDNN's tensor-core convolutions are NHWC kernels, so the
  * BatchNorm + ReLU passes hand them NHWC tensors and take NHWC gradients back instead of leaving ~10 layout transposes per layer
- * to cuDNN.  C and HW multiples of 4, tensors aligned for four-element accesses.
+ * to cuDNN.  C and HW multiples of 4, tensors aligned for four-element accesses, C <= 4096 when x is NHWC.
  *   aaconv_bn_stats_nchw        group statistics of channels [stats_valid_channels, C) of an NCHW (batch-strided) input into the
  *                               shared per-block buffer (layout of aaconv_bn_relu_forward); returns the group geometry
  *   aaconv_bn_relu_cl_forward   y (NHWC) = relu(bn(x)); x NHWC dense (x_is_cl = 1: statistics computed here) or NCHW with a batch

@@ -258,14 +258,9 @@ def test_channels_last_bn_relu_kernels_match_torch(dt, tol, geom):
     ya.backward(g)
     torch.autograd.backward([fb, yb], [gbuf[:, :C], g.to(dt).contiguous(memory_format=torch.channels_last)])
     want = xa.grad + g_prefix0
-    g_rest0 = None
     assert float((want - gbuf[:, :C].float()).abs().max()) < tol * float(want.abs().max()) * 2      # accumulated in place
     assert float((want - xb.grad.float()).abs().max()) < tol * float(want.abs().max()) * 2
     assert rel_err(ours.weight.grad, ref.weight.grad) < tol and rel_err(ours.bias.grad, ref.bias.grad) < tol
-    # the same statistics shared: a second layer that has `C` valid channels reduces nothing new and must give the same output
-    _, yb2 = tap_bn_relu_cl(pair()[1], buf[:, :C].detach().requires_grad_(True), (stats, C))
-    # (weights differ between the two modules; compare through the normalised values: same mean / rstd means same zero pattern)
-    assert torch.equal(yb2 == 0, yb2 == 0)
 
     # ---- (b) NHWC -> NHWC ----
     ref, ours = pair()
