@@ -10,6 +10,8 @@
 //                    gradient of the buffer:  t_bwd_reduce -> finalize -> t_bwd_dx
 //   norm2 -> relu2   x, y NHWC (the 128-channel bottleneck):  cl_stats -> finalize -> cl_apply;  cl_bwd_reduce -> finalize -> cl_bwd_dx
 //   append           new features NHWC -> their channel slice of the NCHW buffer, and the slice of the buffer gradient -> NHWC
+//   eval mode        t_apply / cl_apply alone (EVAL instantiations), their per-channel affine maps from the running statistics
+//                    (aaconv_bn_relu_eval; inference only, no backward)
 //
 // All reductions run in a fixed order (bit-reproducible).  Reference: torchvision densenet.py:31-95,120-124 under
 // models/attn_aug_conv.py:479-482.
@@ -188,9 +190,12 @@ __global__ void __launch_bounds__(256) cl_stats_kernel(const T* __restrict__ x, 
     }
 }
 
-template <class T>
+// EVAL: BatchNorm2d in eval mode, the channel's affine map from the running statistics (`saved` unused); else from saved (mean, rstd)
+template <class T, bool EVAL>
 __global__ void __launch_bounds__(256) cl_apply_kernel(const T* __restrict__ x, long long nquads, int C, const float2* __restrict__ saved,
-                                                       const float* __restrict__ weight, const float* __restrict__ bias, T* __restrict__ y) {
+                                                       const float* __restrict__ weight, const float* __restrict__ bias, T* __restrict__ y,
+                                                       const float* __restrict__ running_mean, const float* __restrict__ running_var,
+                                                       float eps) {
   // the quad's channels repeat with period C / 4: a grid-stride loop with a stride that is a multiple of C / 4 keeps them fixed
   const int Q = C >> 2;
   const long long stride = ((long long)gridDim.x * 256 / Q) * Q;
@@ -199,7 +204,14 @@ __global__ void __launch_bounds__(256) cl_apply_kernel(const T* __restrict__ x, 
   const int c = (int)(i % Q) * 4;
   float sc[4], sh[4];
 #pragma unroll
-  for (int u = 0; u < 4; ++u) { const float2 st = saved[c + u]; sc[u] = weight[c + u] * st.y; sh[u] = bias[c + u] - st.x * sc[u]; }
+  for (int u = 0; u < 4; ++u) {
+    if constexpr (EVAL) {
+      const float2 a = bn_eval_affine(weight, bias, running_mean, running_var, eps, c + u);
+      sc[u] = a.x; sh[u] = a.y;
+    } else {
+      const float2 st = saved[c + u]; sc[u] = weight[c + u] * st.y; sh[u] = bias[c + u] - st.x * sc[u];
+    }
+  }
   for (; i < nquads; i += stride) {
     const float4 v = ldv(x + 4 * i);
     stv(y + 4 * i, make_float4(fmaxf(fmaf(v.x, sc[0], sh[0]), 0.f), fmaxf(fmaf(v.y, sc[1], sh[1]), 0.f), fmaxf(fmaf(v.z, sc[2], sh[2]), 0.f),
@@ -297,7 +309,9 @@ __device__ __forceinline__ void tile_load_nchw(const T* __restrict__ src /* plan
 
 // y (NHWC) = relu(bn(x (NCHW, batch stride))).  The G <= 16 group statistics of the tile's 64 channels are merged here (the separate
 // finalize launch cost 5 us per layer); the CTAs of pixel tile 0 / sample 0 also write saved (mean, rstd) and the running statistics.
-template <class T>
+// EVAL: BatchNorm2d in eval mode instead -- the tile's affine maps come from the running statistics, which are only read (partial,
+// G, n_*, momentum and saved unused).
+template <class T, bool EVAL>
 __global__ void __launch_bounds__(256) t_apply_kernel(const T* __restrict__ x, long long xbs, int C, int HW, const float2* __restrict__ partial,
                                                       int G, float n_each, float n_last, float eps, float momentum,
                                                       float2* __restrict__ saved, float* __restrict__ running_mean,
@@ -306,7 +320,13 @@ __global__ void __launch_bounds__(256) t_apply_kernel(const T* __restrict__ x, l
   __shared__ float t[64][65];                                   // [pixel][channel]
   __shared__ float ssc[64], ssh[64];
   const int b = blockIdx.z, c0 = blockIdx.y * 64, p0 = blockIdx.x * 64;
-  {   // four threads per channel, then two shuffle steps (fixed order); measured: with 64 threads merging serially through IEEE
+  if constexpr (EVAL) {
+    if (threadIdx.x < 64 && c0 + (int)threadIdx.x < C) {
+      const float2 a = bn_eval_affine(weight, bias, running_mean, running_var, eps, c0 + threadIdx.x);
+      ssc[threadIdx.x] = a.x;
+      ssh[threadIdx.x] = a.y;
+    }
+  } else {   // four threads per channel, then two shuffle steps (fixed order); measured: with 64 threads merging serially through IEEE
       // divisions half of the kernel's samples sat in the barrier below
     const int ch = threadIdx.x >> 2, sub = threadIdx.x & 3, c = min(c0 + ch, C - 1);
     Chan acc = {0.f, 0.f, 0.f};
@@ -546,14 +566,33 @@ int cl_fwd(const T* x, int B, int C, int HW, int x_is_cl, long long xbs, const f
     AACONV_LAUNCH_OK("bn_fin_fwd");
     const long long nquads = rows * (C / 4);
     const int grid = (int)std::min<long long>((nquads + 255) / 256, 148 * 16);
-    cl_apply_kernel<T><<<std::max(grid, cdiv(C / 4, 256)), 256, 0, AACONV_ST(st)>>>(x, nquads, C, reinterpret_cast<const float2*>(saved), w, b, y);
+    cl_apply_kernel<T, false><<<std::max(grid, cdiv(C / 4, 256)), 256, 0, AACONV_ST(st)>>>(x, nquads, C, reinterpret_cast<const float2*>(saved),
+                                                                                          w, b, y, nullptr, nullptr, 0.f);
     AACONV_LAUNCH_OK("bn_cl_apply");
     return 0;
   }
-  t_apply_kernel<T><<<dim3(cdiv(HW, 64), cdiv(C, 64), B), 256, 0, AACONV_ST(st)>>>(x, xbs, C, HW, reinterpret_cast<const float2*>(nchw_partial), G,
-                                                                                  n_each, n_last, eps, momentum, reinterpret_cast<float2*>(saved),
-                                                                                  rm, rv, w, b, y);
+  t_apply_kernel<T, false><<<dim3(cdiv(HW, 64), cdiv(C, 64), B), 256, 0, AACONV_ST(st)>>>(x, xbs, C, HW, reinterpret_cast<const float2*>(nchw_partial),
+                                                                                         G, n_each, n_last, eps, momentum,
+                                                                                         reinterpret_cast<float2*>(saved), rm, rv, w, b, y);
   AACONV_LAUNCH_OK("bn_t_apply");
+  return 0;
+}
+
+// eval mode: the apply passes alone, their affine maps from the running statistics (read only: the const_casts below feed a kernel
+// parameter that the EVAL instantiation never writes through)
+template <class T>
+int cl_eval(const T* x, int B, int C, int HW, int x_is_cl, long long xbs, const float* w, const float* b, const float* rm, const float* rv,
+            float eps, T* y, cudaStream_t st) {
+  if (x_is_cl) {
+    const long long nquads = (long long)B * HW * (C / 4);
+    const int grid = (int)std::min<long long>((nquads + 255) / 256, 148 * 16);
+    cl_apply_kernel<T, true><<<std::max(grid, cdiv(C / 4, 256)), 256, 0, AACONV_ST(st)>>>(x, nquads, C, nullptr, w, b, y, rm, rv, eps);
+    AACONV_LAUNCH_OK("bn_cl_eval");
+    return 0;
+  }
+  t_apply_kernel<T, true><<<dim3(cdiv(HW, 64), cdiv(C, 64), B), 256, 0, AACONV_ST(st)>>>(x, xbs, C, HW, nullptr, 0, 0.f, 0.f, eps, 0.f, nullptr,
+                                                                                        const_cast<float*>(rm), const_cast<float*>(rv), w, b, y);
+  AACONV_LAUNCH_OK("bn_t_eval");
   return 0;
 }
 
@@ -674,6 +713,31 @@ int aaconv_slice_layout(const void* src, void* dst, int dtype, int B, int C, int
   }
   AACONV_LAUNCH_OK(to_nchw ? "slice_cl_to_nchw" : "slice_nchw_to_cl");
   return 0;
+}
+
+// relu(BatchNorm2d in eval mode): NCHW (batch stride) -> NCHW (bn_relu.cu), NCHW (batch stride) -> NHWC (t_apply tiles), NHWC -> NHWC
+int aaconv_bn_relu_eval(const void* x, int dtype, int B, int C, int HW, int x_is_cl, int64_t x_batch_stride, const float* weight,
+                        const float* bias, const float* running_mean, const float* running_var, float eps, void* y, int y_is_cl,
+                        void* stream) {
+  if (!x || !weight || !bias || !running_mean || !running_var || !y || B <= 0 || C <= 0 || HW <= 0 || B > 65535)
+    return fail(AACONV_E_ARG, "bad bn_relu_eval arguments");
+  if (dtype != AACONV_FP32 && dtype != AACONV_BF16) return fail(AACONV_E_ARG, "bad bn_relu_eval dtype");
+  if (x_is_cl && !y_is_cl)
+    return fail(AACONV_E_ARG, "bn_relu_eval: an NHWC input needs an NHWC output (pairs: NCHW -> NCHW, NCHW -> NHWC, NHWC -> NHWC)");
+  if (!x_is_cl && x_batch_stride < (int64_t)C * HW) return fail(AACONV_E_ARG, "bn_relu_eval: an NCHW input needs a batch stride >= C*HW");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (!y_is_cl)
+    return bn_relu_eval_nchw(x, dtype, B, C, HW, x_batch_stride, weight, bias, running_mean, running_var, eps, y, st);
+  if ((C & 3) || (HW & 3)) return fail(AACONV_E_ARG, "bn_relu_eval: an NHWC side needs C and HW multiples of 4");
+  if (x_is_cl && C > CL_MAX_C) return fail(AACONV_E_ARG, "bn_relu_eval: an NHWC input has at most 4096 channels");
+  const size_t elt = dtype == AACONV_BF16 ? 2 : 4;
+  if (!aligned4(x, elt) || !aligned4(y, elt) || (!x_is_cl && ((size_t)x_batch_stride * elt) % (4 * elt)))
+    return fail(AACONV_E_ARG, "bn_relu_eval: an NHWC side needs tensors aligned for four-element accesses");
+  return dtype == AACONV_BF16
+             ? cl_eval(static_cast<const bf16*>(x), B, C, HW, x_is_cl, x_batch_stride, weight, bias, running_mean, running_var, eps,
+                       static_cast<bf16*>(y), st)
+             : cl_eval(static_cast<const float*>(x), B, C, HW, x_is_cl, x_batch_stride, weight, bias, running_mean, running_var, eps,
+                       static_cast<float*>(y), st);
 }
 
 }  // extern "C"

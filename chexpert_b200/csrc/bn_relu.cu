@@ -18,6 +18,8 @@
 //             bn_bwd_dx  grid (C, G): merges the partials (fixed order), dx = w rstd (g - mean(g) - x^ mean(g x^)), optionally ADDED
 //                        into the gradient of the feature buffer; the group-0 block writes dweight = sum g x^ and dbias = sum g
 // 3 / 5 passes, all reductions in a fixed order (bit-reproducible), x read through its strides, y / dx dense.
+//   eval      bn_eval    grid (C, G): BatchNorm2d in eval mode, relu(x s + t) from the running statistics, the apply loop of bn_apply
+//                        (aaconv_bn_relu_eval's NCHW -> NCHW variant: stem norm0, norm5, layers the channels-last tiles cannot take)
 #include <algorithm>
 #include <cstdlib>
 #include <cuda_bf16.h>
@@ -164,6 +166,25 @@ __device__ __forceinline__ float2 merge_sums(const float2* __restrict__ partial,
   return sh[256];
 }
 
+// y (dense NCHW) = relu(x sc + sh) over channel c of group grp (this thread's share), x read through its batch stride
+template <class T>
+__device__ __forceinline__ void apply_relu_group(const T* __restrict__ x, T* __restrict__ y, const Geo& g, int c, int C, int grp, float sc,
+                                                 float sh) {
+  const int np = planes_of(g, grp), b0 = grp * g.bpb;
+  const T* px = x + (size_t)b0 * g.xbs + (size_t)c * g.HW;
+  T* py = y + ((size_t)b0 * C + c) * g.HW;
+  const size_t ybs = (size_t)C * g.HW;
+  if (g.unit == 4) {
+    for_each(g, np, [&](int p, int o) {
+      const float4 v = ld4(px + (size_t)p * g.xbs + o);
+      st4(py + p * ybs + o, make_float4(fmaxf(fmaf(v.x, sc, sh), 0.f), fmaxf(fmaf(v.y, sc, sh), 0.f), fmaxf(fmaf(v.z, sc, sh), 0.f),
+                                        fmaxf(fmaf(v.w, sc, sh), 0.f)));
+    });
+  } else {
+    for_each(g, np, [&](int p, int o) { st1(py + p * ybs + o, fmaxf(fmaf(ld1(px + (size_t)p * g.xbs + o), sc, sh), 0.f)); });
+  }
+}
+
 template <class T>
 __global__ void __launch_bounds__(256) bn_apply_kernel(const T* __restrict__ x, const Geo g, const float2* __restrict__ partial,
                                                        const float* __restrict__ weight, const float* __restrict__ bias,
@@ -171,7 +192,7 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const T* __restrict__ x, 
                                                        float eps, T* __restrict__ y, float2* __restrict__ saved, int c_from,
                                                        float2* __restrict__ partial_out) {
   __shared__ float2 shm[257];
-  const int c = blockIdx.x, grp = blockIdx.y, C = gridDim.x, np = planes_of(g, grp), b0 = grp * g.bpb;
+  const int c = blockIdx.x, grp = blockIdx.y, C = gridDim.x, np = planes_of(g, grp);
   float2 st;
   if (g.G == 1 && c >= c_from) {
     // one CTA owns the whole channel: its statistics are computed here (two more passes over data that stays in L1 / L2) and the
@@ -207,18 +228,16 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(const T* __restrict__ x, 
     }
   }
   const float sc = weight[c] * rstd, sh = bias[c] - st.x * sc;
-  const T* px = x + (size_t)b0 * g.xbs + (size_t)c * g.HW;
-  T* py = y + ((size_t)b0 * C + c) * g.HW;
-  const size_t ybs = (size_t)C * g.HW;
-  if (g.unit == 4) {
-    for_each(g, np, [&](int p, int o) {
-      const float4 v = ld4(px + (size_t)p * g.xbs + o);
-      st4(py + p * ybs + o, make_float4(fmaxf(fmaf(v.x, sc, sh), 0.f), fmaxf(fmaf(v.y, sc, sh), 0.f), fmaxf(fmaf(v.z, sc, sh), 0.f),
-                                        fmaxf(fmaf(v.w, sc, sh), 0.f)));
-    });
-  } else {
-    for_each(g, np, [&](int p, int o) { st1(py + p * ybs + o, fmaxf(fmaf(ld1(px + (size_t)p * g.xbs + o), sc, sh), 0.f)); });
-  }
+  apply_relu_group(x, y, g, c, C, grp, sc, sh);
+}
+
+// relu(BatchNorm2d eval) from the running statistics, NCHW -> NCHW: one pass, nothing to reduce.  Grid (C, G) as bn_apply.
+template <class T>
+__global__ void __launch_bounds__(256) bn_eval_kernel(const T* __restrict__ x, const Geo g, const float* __restrict__ weight,
+                                                      const float* __restrict__ bias, const float* __restrict__ running_mean,
+                                                      const float* __restrict__ running_var, float eps, T* __restrict__ y) {
+  const float2 a = bn_eval_affine(weight, bias, running_mean, running_var, eps, blockIdx.x);
+  apply_relu_group(x, y, g, blockIdx.x, gridDim.x, blockIdx.y, a.x, a.y);
 }
 
 // g = dy where the ReLU output is positive (recomputed from x and the saved statistics: y itself is not kept)
@@ -393,7 +412,25 @@ int bwd_t(const T* x, long long xbs, int B, int C, int HW, const T* dy, const fl
   return 0;
 }
 
+template <class T>
+int eval_t(const T* x, long long xbs, int B, int C, int HW, const float* w, const float* b, const float* rm, const float* rv, float eps, T* y,
+           cudaStream_t st) {
+  const Geo g = make_geo<T>(B, C, HW, xbs, x, y, nullptr);
+  bn_eval_kernel<T><<<dim3(C, g.G), 256, 0, AACONV_ST(st)>>>(x, g, w, b, rm, rv, eps, y);
+  AACONV_LAUNCH_OK("bn_relu_eval");
+  return 0;
+}
+
 }  // namespace
+
+int bn_relu_eval_nchw(const void* x, int dtype, int B, int C, int HW, long long xbs, const float* weight, const float* bias,
+                      const float* running_mean, const float* running_var, float eps, void* y, cudaStream_t st) {
+  return dtype == AACONV_BF16 ? eval_t(static_cast<const bf16*>(x), xbs, B, C, HW, weight, bias, running_mean, running_var, eps,
+                                       static_cast<bf16*>(y), st)
+                              : eval_t(static_cast<const float*>(x), xbs, B, C, HW, weight, bias, running_mean, running_var, eps,
+                                       static_cast<float*>(y), st);
+}
+
 }  // namespace aaconv
 
 using namespace aaconv;

@@ -95,6 +95,14 @@ __device__ __forceinline__ void store_y(void* y, size_t idx, float v, int bf16_o
   if (bf16_out) static_cast<__nv_bfloat16*>(y)[idx] = __float2bfloat16(v);
   else static_cast<float*>(y)[idx] = v;
 }
+// BatchNorm2d in eval mode as one affine map per channel: (s_c, t_c) with y = x s_c + t_c, s_c = weight_c / sqrt(running_var_c + eps)
+// (IEEE division and square root), t_c = bias_c - running_mean_c s_c
+__device__ __forceinline__ float2 bn_eval_affine(const float* __restrict__ weight, const float* __restrict__ bias,
+                                                 const float* __restrict__ running_mean, const float* __restrict__ running_var, float eps,
+                                                 int c) {
+  const float s = weight[c] / sqrtf(running_var[c] + eps);
+  return make_float2(s, bias[c] - running_mean[c] * s);
+}
 #endif
 
 inline size_t align256(size_t n) { return (n + 255) & ~size_t(255); }
@@ -113,5 +121,9 @@ struct Carver {
 };
 
 inline int cdiv(int a, int b) { return (a + b - 1) / b; }
+
+// relu(BatchNorm2d eval) NCHW (batch stride xbs) -> dense NCHW, any C / HW / alignment (bn_relu.cu; aaconv_bn_relu_eval dispatches)
+int bn_relu_eval_nchw(const void* x, int dtype, int B, int C, int HW, long long xbs, const float* weight, const float* bias,
+                      const float* running_mean, const float* running_var, float eps, void* y, cudaStream_t st);
 
 }  // namespace aaconv

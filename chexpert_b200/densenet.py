@@ -21,7 +21,8 @@ import torch.nn.functional as F
 from torchvision.models.densenet import _DenseBlock, _DenseLayer
 
 from .aaconv import AAConv2d
-from .fused_bn import bn_relu, tap_bn_relu, tap_bn_relu_cl, bn_relu_cl, cl_ok, slice_layout, _is_cl
+from .fused_bn import (bn_relu, tap_bn_relu, tap_bn_relu_cl, bn_relu_cl, cl_ok, slice_layout, _is_cl, bn_relu_eval, eval_ok,
+                       eval_cl_ok)
 
 
 def transition_attn_dims(num_output_features, attn_params):
@@ -149,9 +150,13 @@ class BufferedDenseBlock(nn.ModuleDict):
     [0, c_i) of the buffer and writes its output behind them, so the per-layer ``torch.cat`` (O(layers^2) copy traffic and
     saved activations) disappears.  If ``init_features`` already lives in such a buffer (an AAConv2d called with ``out_total``),
     it is adopted without a copy.  The gradient of the concatenated features is accumulated along the chain
-    (one add per layer over contiguous tensors) instead of per (producer, consumer) pair."""
+    (one add per layer over contiguous tensors) instead of per (producer, consumer) pair.
 
-    def __init__(self, num_layers, num_input_features, bn_size, growth_rate, drop_rate):
+    ``fused_eval=True``: in eval mode on CUDA with autograd off, every norm -> relu pair runs as relu(BatchNorm2d eval) through
+    fused_bn.bn_relu_eval (running statistics; the same layout plan as training: NCHW prefix -> NHWC for conv1, NHWC -> NHWC for
+    conv2).  Anything else -- training, grad enabled (e.g. Grad-CAM), CPU -- takes the path below unchanged."""
+
+    def __init__(self, num_layers, num_input_features, bn_size, growth_rate, drop_rate, fused_eval=False):
         super().__init__()
         for i in range(num_layers):
             self.add_module('denselayer%d' % (i + 1),
@@ -160,6 +165,23 @@ class BufferedDenseBlock(nn.ModuleDict):
         self.num_input_features, self.growth_rate, self.num_layers = num_input_features, growth_rate, num_layers
         self.out_channels = num_input_features + num_layers * growth_rate
         self.inner_channels_last = os.environ.get('AACONV_INNER_CL', '1') != '0'   # AACONV_INNER_CL=0: NCHW inside the layers (A/B, profiles/r02_b_scaling.md)
+        self.fused_eval = bool(fused_eval)
+
+    def _forward_eval(self, feats, buf):
+        """Inference through the eval-mode BatchNorm + ReLU kernels (no stats buffer: the running statistics are all they read)."""
+        H, W = buf.shape[2:]
+        growth_ok = self.growth_rate % 4 == 0 and (H * W) % 4 == 0
+        for layer in self.values():
+            norm1, norm2 = layer.norm1, layer.norm2
+            if self.inner_channels_last and growth_ok and eval_cl_ok(norm1, feats):
+                z = layer.conv1(bn_relu_eval(norm1, feats, out_cl=True))
+                y2 = bn_relu_eval(norm2, z, out_cl=True) if eval_cl_ok(norm2, z) else bn_relu_eval(norm2, z)
+                new = layer.conv2(y2).to(buf.dtype)
+            else:
+                new = layer.conv2(bn_relu_eval(norm2, layer.conv1(bn_relu_eval(norm1, feats)))).to(buf.dtype)
+            feats = (_AppendCL.apply(feats, new, buf) if _is_cl(new) and growth_ok and _nchw_slice_ok(feats)
+                     else _Append.apply(feats, new.contiguous(), buf))
+        return feats
 
     def forward(self, init_features):
         B, C0, H, W = init_features.shape
@@ -168,6 +190,8 @@ class BufferedDenseBlock(nn.ModuleDict):
                 or not buf.is_contiguous() or buf.data_ptr() != init_features.data_ptr()):
             buf = torch.empty(B, self.out_channels, H, W, dtype=init_features.dtype, device=init_features.device)
         feats = _Adopt.apply(init_features, buf)
+        if self.fused_eval and all(eval_ok(layer.norm1, feats) and eval_ok(layer.norm2, feats) for layer in self.values()):
+            return self._forward_eval(feats, buf)
         # per-(channel, sample) plane statistics of the buffer, shared by the norm1 of every layer: layer i only reduces the channels
         # layer i-1 has not seen (its own 32 new ones); the first layer reduces the block's input channels
         stats = torch.empty(2 * B * self.out_channels, device=buf.device, dtype=torch.float32) if buf.is_cuda else None
@@ -206,9 +230,10 @@ class DenseNet(nn.Module):
     ``precision`` ('fp32' | 'bf16') for the AAConv2d kernels.  Unlike the reference, ``attn_params`` is not mutated."""
 
     def __init__(self, growth_rate=32, block_config=(6, 12, 24, 16), num_init_features=64, bn_size=4, drop_rate=0,
-                 num_classes=1000, attn_params=None, precision=None, feature_buffer=False, fused_prologue=False):
+                 num_classes=1000, attn_params=None, precision=None, feature_buffer=False, fused_prologue=False, fused_eval=False):
         super().__init__()
         self.feature_buffer = bool(feature_buffer)
+        self.fused_eval = bool(fused_eval)
         attn = dict(attn_params) if attn_params is not None else None
         if len(block_config) == 4:    # ImageNet stem: /4 before the first block (:460-468)
             stem = [('conv0', nn.Conv2d(3, num_init_features, kernel_size=7, stride=2, padding=3, bias=False)),
@@ -224,7 +249,7 @@ class DenseNet(nn.Module):
         self.features = nn.Sequential(OrderedDict(stem))
         width = num_init_features
         for i, num_layers in enumerate(block_config):
-            block = (BufferedDenseBlock(num_layers, width, bn_size, growth_rate, drop_rate) if feature_buffer else
+            block = (BufferedDenseBlock(num_layers, width, bn_size, growth_rate, drop_rate, fused_eval) if feature_buffer else
                      _DenseBlock(num_layers=num_layers, num_input_features=width, bn_size=bn_size, growth_rate=growth_rate,
                                  drop_rate=drop_rate))
             self.features.add_module(f'denseblock{i + 1}', block)
@@ -245,6 +270,13 @@ class DenseNet(nn.Module):
             elif isinstance(m, nn.Linear):
                 nn.init.constant_(m.bias, 0)
 
+    def _bn_relu(self, bn, x):
+        """Stem norm0 -> relu0 and norm5 -> F.relu: the eval-mode kernel when fused_eval asks for it and it applies (eval mode, CUDA,
+        autograd off), the training-mode kernels / the module otherwise."""
+        if self.fused_eval and eval_ok(bn, x):
+            return bn_relu_eval(bn, x)
+        return bn_relu(bn, x)
+
     def _features(self, x):
         """-> relu(features(x)) (models/attn_aug_conv.py:513-514)."""
         if not self.feature_buffer:
@@ -259,10 +291,10 @@ class DenseNet(nn.Module):
             if isinstance(m, AATransition) and isinstance(nxt, BufferedDenseBlock):
                 x = m(x, out_total=nxt.out_channels)      # the AAConv2d epilogues write into the next block's buffer
             elif isinstance(m, nn.BatchNorm2d) and isinstance(nxt, nn.ReLU):
-                x = bn_relu(m, x)                         # stem: norm0 -> relu0 as one fused op (grid (C, B) instead of one CTA per channel)
+                x = self._bn_relu(m, x)                   # stem: norm0 -> relu0 as one fused op (grid (C, B) instead of one CTA per channel)
                 skip = True
             elif isinstance(m, nn.BatchNorm2d) and nxt is None:
-                return bn_relu(m, x)                      # norm5 followed by forward()'s F.relu
+                return self._bn_relu(m, x)                # norm5 followed by forward()'s F.relu
             else:
                 x = m(x)
         return F.relu(x, inplace=True)
@@ -276,9 +308,11 @@ class DenseNet(nn.Module):
         return [m for m in self.modules() if isinstance(m, AAConv2d)]
 
 
-def aadensenet121(num_classes=5, input_dims=(320, 320), precision=None, feature_buffer=False, fused_prologue=False):
+def aadensenet121(num_classes=5, input_dims=(320, 320), precision=None, feature_buffer=False, fused_prologue=False, fused_eval=False):
     """The model behind ``--model aadensenet121`` (chexpert.py:474-476); ``input_dims`` is the image size.
-    ``feature_buffer`` / ``fused_prologue``: the B200 execution options of rows f3 / f1 (same parameters, same state_dict)."""
+    ``feature_buffer`` / ``fused_prologue``: the B200 execution options of rows f3 / f1 (same parameters, same state_dict).
+    ``fused_eval``: inference of the feature-buffer model (eval mode, CUDA, autograd off) runs its BatchNorm + ReLU pairs through
+    the eval-mode kernels (fused_bn.bn_relu_eval); it has no effect without ``feature_buffer`` and adds no parameters."""
     return DenseNet(32, (6, 12, 24, 16), 64, num_classes=num_classes,
                     attn_params={'k': 0.2, 'v': 0.1, 'nh': 8, 'relative': True, 'input_dims': tuple(input_dims)},
-                    precision=precision, feature_buffer=feature_buffer, fused_prologue=fused_prologue)
+                    precision=precision, feature_buffer=feature_buffer, fused_prologue=fused_prologue, fused_eval=fused_eval)

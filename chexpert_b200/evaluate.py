@@ -18,6 +18,7 @@ import torch.nn.functional as F
 
 from . import _lib
 from .aaconv import AAConv2d, _ptr, _stream
+from .densenet import aadensenet121
 from .loss import BCEWithLogitsLoss
 
 PIXEL_MEAN, PIXEL_STD = 0.5330, 0.0349        # chexpert.py:70-72
@@ -104,16 +105,114 @@ def auroc_per_class(logits, targets):
     return out
 
 
+class Predictor:
+    """Inference counterpart of train.TrainStep: uint8 images (N, H, W), on the host or the device -> (N, num_classes) float32 logits
+    on the device, with the arithmetic of predict_logits (normalise_u8, then the model in eval mode under no_grad).
+
+    The model is aadensenet121(feature_buffer=True, fused_prologue=True, fused_eval=True): the dense blocks write into one feature
+    buffer, the Transitions' InstanceNorm + ReLU run inside the AAConv2d kernels, and every BatchNorm + ReLU runs through the
+    eval-mode kernels with the dense layers' convolutions channels-last.  Only uint8 images cross PCIe.
+
+    ``autocast=True`` (opt-in; None or False: off) runs the torch/cuDNN layers under bf16 autocast.  The stem and dense-block
+    convolution weights are then kept in bf16 inside this model (the dense blocks' k x k weights channels-last), so no per-call cast
+    kernels run; load_state_dict converts the fp32 checkpoint values as it copies them.  AAConv2d and BatchNorm parameters stay fp32
+    (the kernels read fp32).  Measured on a B200 over the 10 seed-initialised checkpoints of tests/golden/eval_ensemble.npz, autocast
+    keeps the logits within rtol 2e-2 / atol 1e-2 of the fp32 reference (max error 0.012) but misses the bf16 mode's AUROC gate: up to
+    3.6e-3 per class on the ensemble, against 2e-3.  So it is not the default, even for precision='bf16': without it the dense blocks
+    stay fp32, as in predict_logits.
+
+    ``cuda_graph``: after WARMUP eager batches (cuDNN picks its algorithms) one graph of the whole step at ``batch_size`` is
+    captured and replayed.  A ragged last batch is padded to ``batch_size`` (samples are independent in eval mode) and sliced.
+    load_state_dict writes parameters and buffers in place, so one capture serves every checkpoint of an ensemble;
+    ``captures`` counts the captures made."""
+
+    WARMUP = 2
+
+    def __init__(self, num_classes=5, size=320, precision='bf16', batch_size=16, device='cuda', autocast=False, cuda_graph=True):
+        self.device = torch.device(device)
+        if self.device.type != 'cuda':
+            raise RuntimeError('chexpert_b200.evaluate.Predictor runs on CUDA only; there is no CPU fallback')
+        self.num_classes, self.size, self.batch_size = num_classes, size, int(batch_size)
+        self.autocast = bool(autocast)
+        model = aadensenet121(num_classes, (size, size), precision=precision, feature_buffer=True, fused_prologue=True, fused_eval=True)
+        model.requires_grad_(False)
+        # the dense layers' convolutions see NHWC activations, so their k x k weights are kept channels-last (in fp32 too: cuDNN would
+        # otherwise transpose an NCHW weight on every call); 1 x 1 weights are the same bytes in both formats
+        own = {id(p) for m in model.modules() if isinstance(m, AAConv2d) for p in m.parameters()}
+        for name, m in model.named_modules():
+            if isinstance(m, torch.nn.Conv2d) and id(m.weight) not in own:
+                cl = 'denseblock' in name and m.weight.shape[2] * m.weight.shape[3] > 1
+                m.weight.data = m.weight.data.to(torch.bfloat16 if self.autocast else torch.float32,
+                                                 memory_format=torch.channels_last if cl else torch.contiguous_format)
+        self.model = model.to(self.device).eval()
+        self.cuda_graph = bool(cuda_graph)
+        self._warm = 0
+        self._graph = self._sx = self._sy = None
+        self.captures = 0
+
+    def load_state_dict(self, state_dict):
+        """Strict, in place (a reference checkpoint loads unchanged); a captured graph stays valid."""
+        with torch.no_grad():
+            self.model.load_state_dict(state_dict, strict=True)
+
+    def _forward(self, u8):
+        with torch.autocast('cuda', dtype=torch.bfloat16, enabled=self.autocast, cache_enabled=False):
+            return self.model(normalise_u8(u8)).float()
+
+    def _capture(self):
+        torch.cuda.synchronize(self.device)
+        self._graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self._graph):
+            self._sy = self._forward(self._sx)
+        self.captures += 1
+
+    def _batch(self, chunk):
+        n = chunk.shape[0]
+        if not self.cuda_graph:
+            return self._forward(chunk.to(self.device, non_blocking=True))
+        if self._sx is None:
+            self._sx = torch.zeros(self.batch_size, *chunk.shape[1:], dtype=torch.uint8, device=self.device)
+        self._sx[:n].copy_(chunk, non_blocking=True)       # rows [n, batch_size) keep earlier images: padding, sliced off below
+        if self._graph is None:
+            if self._warm < self.WARMUP:
+                self._warm += 1
+                return self._forward(self._sx)[:n]
+            self._capture()
+        self._graph.replay()
+        return self._sy[:n]
+
+    @torch.no_grad()
+    def __call__(self, images_u8):
+        """uint8 (N, H, W) -> (N, num_classes) float32 logits on the device, batch by batch."""
+        if images_u8.dtype != torch.uint8 or images_u8.dim() != 3:
+            raise RuntimeError(f'Predictor takes uint8 (N, H, W) images, got {images_u8.dtype} {tuple(images_u8.shape)}')
+        with torch.cuda.device(self.device):
+            N = images_u8.shape[0]
+            out = torch.empty(N, self.num_classes, device=self.device, dtype=torch.float32)
+            for i in range(0, N, self.batch_size):
+                chunk = images_u8[i:i + self.batch_size]
+                out[i:i + chunk.shape[0]].copy_(self._batch(chunk))
+            return out
+
+
 @torch.no_grad()
 def evaluate_ensemble(model, state_dicts, images_u8, targets, batch_size=16, device='cuda'):
     """The reference's ensemble evaluation (chexpert.py:217-236): every checkpoint's state_dict is loaded strictly into
     `model`, its logits and element losses over the whole set are kept, the ensemble output / loss are their means over the
     checkpoints (chexpert.py:233-234; note mean-of-losses, not loss-of-mean); metrics as compute_metrics (chexpert.py:130-146)
-    minus the plotting inputs.  -> dict(outputs, per_model, auroc, loss)."""
+    minus the plotting inputs.  -> dict(outputs, per_model, auroc, loss).
+    `model` may be a Predictor; it then runs on its own device with its own batch size (`batch_size` / `device` are not used)."""
+    if isinstance(model, Predictor):
+        device = model.device
     t = targets.to(device)
     loss_fn = BCEWithLogitsLoss('none').to(device)
     per_model, losses = [], []
     for sd in state_dicts:
+        if isinstance(model, Predictor):
+            model.load_state_dict(sd)
+            per_model.append(model(images_u8))
+            losses.append(loss_fn(per_model[-1], t))
+            continue
         model.load_state_dict(sd, strict=True)
         per_model.append(predict_logits(model, images_u8, batch_size, device))
         losses.append(loss_fn(per_model[-1], t))       # element losses of THIS checkpoint (chexpert.py:205,229-231)

@@ -1,7 +1,8 @@
 """BatchNorm2d (training mode) + ReLU as one op that reads its input through a batch stride -- the normalisation of a channel
 slice of the pre-allocated DenseBlock feature buffer (SURVEY.md section 8 row f3; torchvision densenet.py:36-41 under
 models/attn_aug_conv.py:479-482).  Parameters, buffers and the arithmetic are nn.BatchNorm2d's (same state_dict, same running
-statistics update); eval mode and CPU tensors go through the module's own forward.
+statistics update); eval mode and CPU tensors go through the module's own forward.  bn_relu_eval is the eval-mode counterpart
+(running statistics, no backward) that the dense blocks take only when asked to (DenseNet(fused_eval=True)) and autograd is off.
 """
 import ctypes
 
@@ -253,6 +254,54 @@ def tap_bn_relu_cl(bn, x, stats=None):
 def bn_relu_cl(bn, x):
     _bump(bn)
     return _BNReLUCL.apply(x, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.momentum, bn.eps)
+
+
+# ------------------------------------------------------------------------------------------------
+# eval mode (running statistics): aaconv_bn_relu_eval, inference only -- no autograd, no backward
+# ------------------------------------------------------------------------------------------------
+def eval_ok(bn, x):
+    """relu(bn(x)) may run through bn_relu_eval: an eval-mode, affine BatchNorm2d with running statistics, a CUDA tensor in fp32 /
+    bf16, and no autograd graph being recorded (the eval kernels have no backward)."""
+    return (not bn.training and not torch.is_grad_enabled() and x.is_cuda and x.dim() == 4 and x.dtype in _DT and bn.affine
+            and bn.track_running_stats and bn.running_mean is not None and x.shape[0] <= 65535
+            and all(t.dtype == torch.float32 and t.is_contiguous() for t in (bn.weight, bn.bias, bn.running_mean, bn.running_var)))
+
+
+def eval_cl_ok(bn, x):
+    """bn_relu_eval(bn, x, out_cl=True) is supported: C and H*W multiples of 4, x a channels-last tensor of at most CL_MAX_C channels
+    or an NCHW tensor with dense samples, both aligned for four-element accesses."""
+    B, C, H, W = x.shape
+    if not (eval_ok(bn, x) and C % 4 == 0 and (H * W) % 4 == 0 and x.data_ptr() % (4 * x.element_size()) == 0):
+        return False
+    return (_is_cl(x) and C <= CL_MAX_C) or (_strided_ok(x) and x.stride(0) % 4 == 0)
+
+
+def bn_relu_eval(bn, x, out_cl=False):
+    """relu(bn(x)) for an eval-mode nn.BatchNorm2d from its running statistics (which are read, never written; num_batches_tracked is
+    not touched).  x: an NCHW tensor with dense samples (e.g. a channel prefix of the feature buffer) or a channels-last tensor;
+    -> a new tensor, channels-last when `out_cl` (see eval_cl_ok for when that is supported), contiguous NCHW otherwise."""
+    if not x.is_cuda:
+        raise RuntimeError('fused_bn.bn_relu_eval runs on CUDA only; there is no CPU fallback')
+    if not eval_ok(bn, x):
+        raise RuntimeError('fused_bn.bn_relu_eval needs an eval-mode affine BatchNorm2d with running statistics, an fp32 / bf16 4-d '
+                           'input with B <= 65535, and autograd off (the eval kernels have no backward)')
+    if out_cl and not eval_cl_ok(bn, x):
+        raise RuntimeError('fused_bn.bn_relu_eval: channels-last output needs C and H*W multiples of 4, four-element alignment and '
+                           f'at most {CL_MAX_C} channels for a channels-last input')
+    x_is_cl = not _strided_ok(x) and _is_cl(x)
+    if not x_is_cl and not _strided_ok(x):
+        x = x.contiguous()
+    if x_is_cl and not out_cl:                 # no NHWC -> NCHW variant
+        x, x_is_cl = x.contiguous(), False
+    lib = _lib.load()
+    B, C, H, W = x.shape
+    w, b = bn.weight.detach(), bn.bias.detach()
+    with torch.cuda.device(x.device):
+        y = torch.empty((B, C, H, W), device=x.device, dtype=x.dtype, memory_format=_CL if out_cl else torch.contiguous_format)
+        _lib.check(lib.aaconv_bn_relu_eval(_ptr(x), _DT[x.dtype], B, C, H * W, int(x_is_cl), C * H * W if x_is_cl else x.stride(0),
+                                           _ptr(w), _ptr(b), _ptr(bn.running_mean), _ptr(bn.running_var), float(bn.eps), _ptr(y),
+                                           int(out_cl), _stream()), 'aaconv_bn_relu_eval')
+    return y
 
 
 def slice_layout(src, dst, to_nchw):

@@ -188,6 +188,15 @@ int aaconv_bn_relu_cl_backward(const void* x, int dtype, int B, int C, int HW, i
                                int dx_accumulate, float* dweight, float* dbias, void* workspace, void* stream);
 int aaconv_slice_layout(const void* src, void* dst, int dtype, int B, int C, int HW, int64_t nchw_batch_stride, int to_nchw, void* stream);
 
+/* relu(BatchNorm2d in EVAL mode): y = max(x * s_c + t_c, 0), s_c = weight_c / sqrt(running_var_c + eps), t_c = bias_c - running_mean_c * s_c.
+ * x: (B, C, HW) NCHW with x_batch_stride >= C*HW (a channel prefix of the feature buffer), or NHWC dense (x_is_cl = 1).
+ * y: dense, NCHW (y_is_cl = 0) or NHWC (y_is_cl = 1), same dtype as x (AACONV_FP32 | AACONV_BF16).  Supported pairs:
+ * NCHW -> NCHW (any C, HW, alignment), NCHW -> NHWC and NHWC -> NHWC (C, HW multiples of 4, four-element aligned, NHWC C <= 4096).
+ * Reads the running statistics, never writes them; no workspace. */
+int aaconv_bn_relu_eval(const void* x, int dtype, int B, int C, int HW, int x_is_cl, int64_t x_batch_stride,
+                        const float* weight, const float* bias, const float* running_mean, const float* running_var,
+                        float eps, void* y, int y_is_cl, void* stream);
+
 /* Accounting / measurement helpers used by bench.py (no reference counterpart).
  *   aaconv_launch_count   kernels launched by this library since it was loaded (all threads).
  *   aaconv_profile_begin  start recording a (start, stop) CUDA-event pair around every launch (`stream` is unused, kept for ABI).
