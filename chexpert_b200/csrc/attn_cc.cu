@@ -1048,6 +1048,11 @@ int launch_bwd_dq_cc(const Dims& d, const AugLayout& a, const CUtensorMap& tq_st
   return 0;
 }
 
+// the dQa staging tile is OUTW >= KD floats wide; a narrower one leaves room for one more streamed stage at 3 atoms
+template <int KATOMS> struct CcOutw {
+  static constexpr int MAX = KATOMS * 64 - 16, MID = KATOMS == 3 ? 152 : MAX;
+};
+
 template <int KATOMS, int DVH>
 int launch_bwd_cc(const Dims& d, const AugLayout& a, const void* qa, const void* ka, const float* v, const float* d_o,
                   const float* delta, float* dqa, float* dk, float* dv, void* dqkvh, int KPq, cudaStream_t st) {
@@ -1074,18 +1079,53 @@ int launch_bwd_cc(const Dims& d, const AugLayout& a, const void* qa, const void*
                                          nqt, nitems);
     AACONV_LAUNCH_OK("attn_bwd_dkv_cc");
   }
-  // the dQa staging tile is OUTW >= KD floats wide; a narrower one leaves room for one more streamed stage at 3 atoms
-  constexpr int OUTW_MAX = KATOMS * 64 - 16, OUTW_MID = KATOMS == 3 ? 152 : OUTW_MAX;
-  if (a.KD <= OUTW_MID) return launch_bwd_dq_cc<KATOMS, DVH, OUTW_MID>(d, a, tq_stat, tk_strm, v, d_o, delta, dqa, nqt, nitems, grid, st);
-  return launch_bwd_dq_cc<KATOMS, DVH, OUTW_MAX>(d, a, tq_stat, tk_strm, v, d_o, delta, dqa, nqt, nitems, grid, st);
+  typedef CcOutw<KATOMS> W;
+  if (a.KD <= W::MID) return launch_bwd_dq_cc<KATOMS, DVH, W::MID>(d, a, tq_stat, tk_strm, v, d_o, delta, dqa, nqt, nitems, grid, st);
+  return launch_bwd_dq_cc<KATOMS, DVH, W::MAX>(d, a, tq_stat, tk_strm, v, d_o, delta, dqa, nqt, nitems, grid, st);
+}
+
+// every kernel one (KATOMS, DVH) instance launches at this KD (forward, dK/dV, dQa) gets its dynamic shared memory next to
+// its static shared memory within the per-block limit
+template <class Kern>
+bool smem_fits(Kern kern, size_t dyn) {
+  static int optin = 0;
+  if (optin == 0) {
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
+      optin = 232448;
+  }
+  cudaFuncAttributes fa;
+  if (cudaFuncGetAttributes(&fa, kern) != cudaSuccess) { (void)cudaGetLastError(); return false; }
+  return fa.sharedSizeBytes + dyn <= (size_t)optin;
+}
+
+template <int KATOMS, int DVH>
+bool cc_smem_fits(int KD) {
+  typedef CcOutw<KATOMS> W;
+  static int ok[2] = {-1, -1};                     // per dQa staging width; the answer does not change within a process
+  int& r = ok[KD > W::MID];
+  if (r < 0) {
+    const bool dq = KD <= W::MID
+                        ? smem_fits(attn_bwd_dq_cc_kernel<KATOMS, DVH, W::MID>, sizeof(CbSmem<KATOMS, CB_BN * DVH, CB_BM * W::MID, DVH + 1>) + 1024)
+                        : smem_fits(attn_bwd_dq_cc_kernel<KATOMS, DVH, W::MAX>, sizeof(CbSmem<KATOMS, CB_BN * DVH, CB_BM * W::MAX, DVH + 1>) + 1024);
+    r = dq && smem_fits(attn_fwd_cc_kernel<KATOMS, DVH>, sizeof(CfSmem<KATOMS, DVH>) + 1024) &&
+        smem_fits(attn_bwd_dkv_cc_kernel<KATOMS, DVH, 0>, sizeof(CbSmem<KATOMS, CB_BN * (DVH + 1), 0, DVH>) + 1024);
+  }
+  return r;
 }
 
 }  // namespace
 
-// value width 1..2 and 16-byte-aligned fp32 side tiles (L % 4 == 0)
+// value width 1..2, 16-byte-aligned fp32 side tiles (L % 4 == 0), and every kernel of the instance within the 227 KB of
+// shared memory a block can have (dv/nh = 2 at three operand atoms is not: its dK/dV kernel needs more; the tc kernels run it)
 int cc_attn_supported(const Dims& d) {
   if (aug_supported(d)) return AACONV_E_UNSUPPORTED;
   if (d.dvh < 1 || d.dvh > 2 || (d.L & 3)) return AACONV_E_UNSUPPORTED;
+  const AugLayout a = aug_layout(d);
+  const int K = a.KP / 64;
+  const bool fits = d.dvh == 1 ? (K == 1 ? cc_smem_fits<1, 1>(a.KD) : K == 2 ? cc_smem_fits<2, 1>(a.KD) : cc_smem_fits<3, 1>(a.KD))
+                               : (K == 1 ? cc_smem_fits<1, 2>(a.KD) : K == 2 ? cc_smem_fits<2, 2>(a.KD) : cc_smem_fits<3, 2>(a.KD));
+  if (!fits) return AACONV_E_UNSUPPORTED;
   return 0;
 }
 

@@ -16,12 +16,16 @@ namespace aaconv {
 std::string& last_error_ref();
 int fail(int code, const char* fmt, ...);
 
+// A failed runtime call also leaves its error in the thread's last-error slot; it is consumed here, so that it is reported
+// once, by this call, and not again by the next launch check (AACONV_LAUNCH_OK) of a later, unrelated call.
 #define AACONV_CUDA_OK(expr)                                                                       \
   do {                                                                                             \
     cudaError_t e__ = (expr);                                                                      \
-    if (e__ != cudaSuccess)                                                                        \
+    if (e__ != cudaSuccess) {                                                                      \
+      (void)cudaGetLastError();                                                                    \
       return ::aaconv::fail(AACONV_E_CUDA, "%s:%d %s -> %s", __FILE__, __LINE__, #expr,          \
                             cudaGetErrorString(e__));                                              \
+    }                                                                                              \
   } while (0)
 
 // Called right after every kernel launch of this library: error check + launch accounting (+ optional

@@ -232,9 +232,9 @@ def aaconv_backward_closed(x, p, s: AAConvShape, dy):
         dAh = dS6.sum(5)                              # [b,n,y,x,y']  summed over key columns
         ix = _rel_index(W, x.device)
         iy = _rel_index(H, x.device)
-        dRw = torch.zeros(B, s.nh, H, W, 2 * W - 1, dtype=x.dtype).scatter_add_(
+        dRw = torch.zeros(B, s.nh, H, W, 2 * W - 1, dtype=x.dtype, device=x.device).scatter_add_(
             4, ix[None, None, None].expand(B, s.nh, H, W, W), dAw)
-        dRh = torch.zeros(B, s.nh, H, W, 2 * H - 1, dtype=x.dtype).scatter_add_(
+        dRh = torch.zeros(B, s.nh, H, W, 2 * H - 1, dtype=x.dtype, device=x.device).scatter_add_(
             4, iy[None, None, :, None, :].expand(B, s.nh, H, W, H), dAh)
         dRw = dRw.reshape(B, s.nh, H * W, -1)
         dRh = dRh.reshape(B, s.nh, H * W, -1)
@@ -266,7 +266,7 @@ def aaconv_backward_closed_by_head(x, p, s: AAConvShape, dy, return_weights_head
     Wo = p['out_proj.weight'][:, :, 0, 0]
     dya = dy[:, nconv:]
     dO_all = torch.einsum('oc,bohw->bchw', Wo, dya).reshape(B, s.nh, s.dvh, L)
-    O = torch.zeros(B, s.nh, s.dvh, L, dtype=x.dtype)
+    O = torch.zeros(B, s.nh, s.dvh, L, dtype=x.dtype, device=x.device)
     dq, dk, dV = torch.zeros_like(q), torch.zeros_like(k), torch.zeros_like(v)
     g = {}
     if s.relative:
@@ -291,8 +291,8 @@ def aaconv_backward_closed_by_head(x, p, s: AAConvShape, dy, return_weights_head
         if s.relative:
             dS6 = dS.reshape(B, 1, H, W, H, W)
             dAw, dAh = dS6.sum(4), dS6.sum(5)
-            dRw = torch.zeros(B, 1, H, W, 2 * W - 1, dtype=x.dtype).scatter_add_(4, ix[None, None, None].expand(B, 1, H, W, W), dAw)
-            dRh = torch.zeros(B, 1, H, W, 2 * H - 1, dtype=x.dtype).scatter_add_(
+            dRw = torch.zeros(B, 1, H, W, 2 * W - 1, dtype=x.dtype, device=x.device).scatter_add_(4, ix[None, None, None].expand(B, 1, H, W, W), dAw)
+            dRh = torch.zeros(B, 1, H, W, 2 * H - 1, dtype=x.dtype, device=x.device).scatter_add_(
                 4, iy[None, None, :, None, :].expand(B, 1, H, W, H), dAh)
             dRw, dRh = dRw.reshape(B, 1, L, -1), dRh.reshape(B, 1, L, -1)
             g['key_rel_w'] += torch.einsum('bndq,bnqr->dr', qn, dRw)
