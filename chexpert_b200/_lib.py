@@ -74,6 +74,12 @@ SYMBOLS = {
     'aaconv_slice_layout': (ctypes.c_int, [_P, _P, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int64, ctypes.c_int, _P]),
     'aaconv_bn_relu_eval': (ctypes.c_int, [_P, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int64,
                                            _P, _P, _P, _P, ctypes.c_float, _P, ctypes.c_int, _P]),
+    'aaconv_bn_relu_pool_workspace_bytes': (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int]),
+    'aaconv_bn_relu_pool_forward': (ctypes.c_int, [_P, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int64,
+                                                   ctypes.c_int, _P, _P, _P, _P, ctypes.c_float, ctypes.c_float, _P, _P, _P, ctypes.c_int,
+                                                   ctypes.c_int, _P]),
+    'aaconv_bn_relu_pool_backward': (ctypes.c_int, [_P, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int64,
+                                                    _P, _P, _P, _P, _P, ctypes.c_int64, ctypes.c_int, _P, _P, _P, _P]),
     'aaconv_launch_count': (ctypes.c_longlong, []),
     'aaconv_debug_set_timeline': (None, [_P]),
     'aaconv_debug_set_mode': (None, [ctypes.c_int]),

@@ -12,6 +12,9 @@
 //   append           new features NHWC -> their channel slice of the NCHW buffer, and the slice of the buffer gradient -> NHWC
 //   eval mode        t_apply / cl_apply alone (EVAL instantiations), their per-channel affine maps from the running statistics
 //                    (aaconv_bn_relu_eval; inference only, no backward)
+//   Transition       densenet121's BatchNorm -> ReLU -> 1x1 conv -> AvgPool2d(2), the pool moved ahead of the conv: NCHW block buffer
+//                    -> pooled NHWC operand (pool_apply, training or EVAL); backward pool_bwd_reduce -> finalize -> pool_bwd_dx
+//                    (aaconv_bn_relu_pool_*)
 //
 // All reductions run in a fixed order (bit-reproducible).  Reference: torchvision densenet.py:31-95,120-124 under
 // models/attn_aug_conv.py:479-482.
@@ -307,19 +310,17 @@ __device__ __forceinline__ void tile_load_nchw(const T* __restrict__ src /* plan
   }
 }
 
-// y (NHWC) = relu(bn(x (NCHW, batch stride))).  The G <= 16 group statistics of the tile's 64 channels are merged here (the separate
-// finalize launch cost 5 us per layer); the CTAs of pixel tile 0 / sample 0 also write saved (mean, rstd) and the running statistics.
-// EVAL: BatchNorm2d in eval mode instead -- the tile's affine maps come from the running statistics, which are only read (partial,
-// G, n_*, momentum and saved unused).
-template <class T, bool EVAL>
-__global__ void __launch_bounds__(256) t_apply_kernel(const T* __restrict__ x, long long xbs, int C, int HW, const float2* __restrict__ partial,
-                                                      int G, float n_each, float n_last, float eps, float momentum,
-                                                      float2* __restrict__ saved, float* __restrict__ running_mean,
-                                                      float* __restrict__ running_var, const float* __restrict__ weight,
-                                                      const float* __restrict__ bias, T* __restrict__ y) {
-  __shared__ float t[64][65];                                   // [pixel][channel]
-  __shared__ float ssc[64], ssh[64];
-  const int b = blockIdx.z, c0 = blockIdx.y * 64, p0 = blockIdx.x * 64;
+// The per-channel affine maps (ssc, ssh) of the CTA's 64 channels [c0, c0 + 64), y = relu(x ssc + ssh).  The G group statistics of
+// a channel (NCHW layout of aaconv_bn_stats_nchw) are merged here (the separate finalize launch cost 5 us per layer); the CTAs of
+// pixel tile 0 / sample 0 (blockIdx.x == 0, blockIdx.z == 0) also write saved (mean, rstd) and the running statistics.
+// EVAL: BatchNorm2d in eval mode instead -- the affine maps come from the running statistics, which are only read (partial, G,
+// n_*, momentum and saved unused).  The caller synchronises before reading ssc / ssh.
+template <bool EVAL>
+__device__ __forceinline__ void tile_affine(int c0, int C, const float2* __restrict__ partial, int G, float n_each, float n_last, float eps,
+                                            float momentum, float2* __restrict__ saved, float* __restrict__ running_mean,
+                                            float* __restrict__ running_var, const float* __restrict__ weight,
+                                            const float* __restrict__ bias, float* ssc, float* ssh) {
+  const int b = blockIdx.z;
   if constexpr (EVAL) {
     if (threadIdx.x < 64 && c0 + (int)threadIdx.x < C) {
       const float2 a = bn_eval_affine(weight, bias, running_mean, running_var, eps, c0 + threadIdx.x);
@@ -357,6 +358,19 @@ __global__ void __launch_bounds__(256) t_apply_kernel(const T* __restrict__ x, l
     }
     }
   }
+}
+
+// y (NHWC) = relu(bn(x (NCHW, batch stride))), the affine maps from tile_affine.
+template <class T, bool EVAL>
+__global__ void __launch_bounds__(256) t_apply_kernel(const T* __restrict__ x, long long xbs, int C, int HW, const float2* __restrict__ partial,
+                                                      int G, float n_each, float n_last, float eps, float momentum,
+                                                      float2* __restrict__ saved, float* __restrict__ running_mean,
+                                                      float* __restrict__ running_var, const float* __restrict__ weight,
+                                                      const float* __restrict__ bias, T* __restrict__ y) {
+  __shared__ float t[64][65];                                   // [pixel][channel]
+  __shared__ float ssc[64], ssh[64];
+  const int b = blockIdx.z, c0 = blockIdx.y * 64, p0 = blockIdx.x * 64;
+  tile_affine<EVAL>(c0, C, partial, G, n_each, n_last, eps, momentum, saved, running_mean, running_var, weight, bias, ssc, ssh);
   __syncthreads();
   tile_load_nchw(x + (size_t)b * xbs + (size_t)c0 * HW, C, c0, HW, p0, t, [&](int c, float4 v) {
     const float sc = ssc[c - c0], sh = ssh[c - c0];
@@ -486,6 +500,193 @@ __global__ void __launch_bounds__(256) t_bwd_dx_kernel(const T* __restrict__ x, 
         float4 v = make_float4(t[pl][cl], t[pl + 1][cl], t[pl + 2][cl], t[pl + 3][cl]);
         if (ACC) { v.x += ga[i].x; v.y += ga[i].y; v.z += ga[i].z; v.w += ga[i].w; }
         stv(dstp + (size_t)cl * HW + px, v);
+      }
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// torchvision's Transition, BatchNorm2d -> ReLU -> Conv2d 1x1 -> AvgPool2d(2), with the pool moved ahead of the 1x1 convolution
+// (the convolution is per pixel and linear, so the two commute): x NCHW (batch stride) -> P (B, H/2, W/2, C) NHWC dense, the 2x2
+// window means of relu(bn(x)); the convolution then runs on a quarter of the pixels.  Floor mode: an odd last row / column is in
+// no window, but it is part of the batch statistics, and backward gives it the mean terms of dx.
+// A CTA covers 64 channels x 64 windows (flattened over the window grid); warp w owns channels c0 + 8w .. c0 + 8w + 7, lane l the
+// windows l and l + 32 -- the four source pixels of a window are two pairs of neighbouring elements of two NCHW rows.
+// ------------------------------------------------------------------------------------------------
+// the 2 x 2 window (hq, wq) of a plane: v = rows 2 hq, 2 hq + 1 x columns 2 wq, 2 wq + 1; elements outside the plane read as 0
+template <class T>
+__device__ __forceinline__ void win_load(const T* __restrict__ plane, int H, int W, int hq, int wq, float v[4]) {
+  const int h = 2 * hq, w = 2 * wq;
+  const T* p = plane + (size_t)h * W + w;
+  const bool r1 = h + 1 < H, c1 = w + 1 < W;
+  v[0] = ld1v(p);
+  v[1] = c1 ? ld1v(p + 1) : 0.f;
+  v[2] = r1 ? ld1v(p + W) : 0.f;
+  v[3] = r1 && c1 ? ld1v(p + W + 1) : 0.f;
+}
+
+// P = avgpool2(relu(bn(x))); the affine maps (and in training saved / running statistics) from tile_affine
+template <class T, bool EVAL>
+__global__ void __launch_bounds__(256) pool_apply_kernel(const T* __restrict__ x, long long xbs, int C, int H, int W,
+                                                         const float2* __restrict__ partial, int G, float n_each, float n_last, float eps,
+                                                         float momentum, float2* __restrict__ saved, float* __restrict__ running_mean,
+                                                         float* __restrict__ running_var, const float* __restrict__ weight,
+                                                         const float* __restrict__ bias, T* __restrict__ y) {
+  __shared__ float t[64][65];                                   // [window][channel]
+  __shared__ float ssc[64], ssh[64];
+  const int b = blockIdx.z, c0 = blockIdx.y * 64, p0 = blockIdx.x * 64;
+  const int Wp = W >> 1, P = (H >> 1) * Wp;
+  tile_affine<EVAL>(c0, C, partial, G, n_each, n_last, eps, momentum, saved, running_mean, running_var, weight, bias, ssc, ssh);
+  __syncthreads();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const int cl = warp * 8 + i, c = c0 + cl;
+    const T* plane = x + (size_t)b * xbs + (size_t)min(c, C - 1) * H * W;
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int pl = lane + 32 * k, p = p0 + pl;
+      float s = 0.f;
+      if (c < C && p < P) {
+        const int hq = p / Wp;
+        float v[4];
+        win_load(plane, H, W, hq, p - hq * Wp, v);
+        const float sc = ssc[cl], sh = ssh[cl];
+        s = 0.25f * ((fmaxf(fmaf(v[0], sc, sh), 0.f) + fmaxf(fmaf(v[1], sc, sh), 0.f)) +
+                     (fmaxf(fmaf(v[2], sc, sh), 0.f) + fmaxf(fmaf(v[3], sc, sh), 0.f)));
+      }
+      t[pl][cl] = s;
+    }
+  }
+  __syncthreads();
+  const int cq = (lane & 15) * 4;
+  T* dst = y + (size_t)b * P * C;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int pl = warp * 8 + i * 2 + (lane >> 4), p = p0 + pl;
+    if (p < P && c0 + cq < C) stv(dst + (size_t)p * C + c0 + cq, make_float4(t[pl][cq], t[pl][cq + 1], t[pl][cq + 2], t[pl][cq + 3]));
+  }
+}
+
+// the dP tile of windows [p0, p0 + 64) of the window grid (Hq, Wq) -> t[window][channel]; windows outside the pooled map
+// (Hp, Wp) -- the odd last row / column -- get 0
+template <class T>
+__device__ __forceinline__ void dp_tile(const T* __restrict__ dP, int b, int C, int c0, int Hp, int Wp, int Wq, int nwin, int p0,
+                                        float (*t)[65]) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, cq = (lane & 15) * 4;
+  float4 gq[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {                                 // every load issued before the first store
+    const int q = p0 + warp * 8 + i * 2 + (lane >> 4), hq = q / Wq, wq = q - hq * Wq;
+    gq[i] = (q < nwin && hq < Hp && wq < Wp && c0 + cq < C) ? ldv(dP + (((size_t)b * Hp + hq) * Wp + wq) * C + c0 + cq)
+                                                            : make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int pl = warp * 8 + i * 2 + (lane >> 4);
+    t[pl][cq] = gq[i].x; t[pl][cq + 1] = gq[i].y; t[pl][cq + 2] = gq[i].z; t[pl][cq + 3] = gq[i].w;
+  }
+}
+
+// partial[c * (B * nseg) + b * nseg + seg] = (sum g, sum g x^) over the source pixels of the segment's windows, g = dP / 4 where the
+// pre-activation is positive (the dropped row / column has g = 0 and adds nothing)
+template <class T>
+__global__ void __launch_bounds__(256) pool_bwd_reduce_kernel(const T* __restrict__ x, long long xbs, int C, int H, int W,
+                                                              const T* __restrict__ dP, const float2* __restrict__ saved,
+                                                              const float* __restrict__ weight, const float* __restrict__ bias,
+                                                              int chunks_per_seg, float2* __restrict__ partial) {
+  __shared__ float t[64][65];                                   // dP tile, [window][channel]
+  const int seg = blockIdx.x, nseg = gridDim.x, c0 = blockIdx.y * 64, b = blockIdx.z, B = gridDim.z;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int Hp = H >> 1, Wp = W >> 1, P = Hp * Wp;
+  float mu[8], rs[8], w[8], bb[8], s1[8], s2[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const int c = min(c0 + warp * 8 + i, C - 1);
+    const float2 st = saved[c];
+    mu[i] = st.x; rs[i] = st.y; w[i] = weight[c]; bb[i] = bias[c]; s1[i] = 0.f; s2[i] = 0.f;
+  }
+  const int nchunks = (P + 63) / 64;
+  for (int ch = seg * chunks_per_seg; ch < min(nchunks, (seg + 1) * chunks_per_seg); ++ch) {
+    const int p0 = ch * 64;
+    __syncthreads();                                            // the previous chunk's tile has been consumed
+    dp_tile(dP, b, C, c0, Hp, Wp, Wp, P, p0, t);
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const int cl = warp * 8 + i, c = c0 + cl;
+      if (c >= C) continue;
+      const T* plane = x + (size_t)b * xbs + (size_t)c * H * W;
+#pragma unroll
+      for (int k = 0; k < 2; ++k) {
+        const int pl = lane + 32 * k, p = p0 + pl;
+        if (p >= P) continue;
+        const int hq = p / Wp;
+        float v[4];
+        win_load(plane, H, W, hq, p - hq * Wp, v);
+        const float g = 0.25f * t[pl][cl];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const float xh = (v[u] - mu[i]) * rs[i];
+          const float gg = fmaf(w[i], xh, bb[i]) > 0.f ? g : 0.f;
+          s1[i] += gg;
+          s2[i] = fmaf(gg, xh, s2[i]);
+        }
+      }
+    }
+  }
+  // the 32 lanes of a channel, summed in a fixed shuffle-tree order
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      s1[i] += __shfl_down_sync(0xffffffffu, s1[i], o);
+      s2[i] += __shfl_down_sync(0xffffffffu, s2[i], o);
+    }
+    const int c = c0 + warp * 8 + i;
+    if (lane == 0 && c < C) partial[(size_t)c * ((size_t)B * nseg) + (size_t)b * nseg + seg] = make_float2(s1[i], s2[i]);
+  }
+}
+
+// dx (NCHW, batch stride dbs) (+)= w rstd (g - mean(g) - x^ mean(g x^)) for EVERY source pixel: the grid runs over the
+// ceil(H/2) x ceil(W/2) windows, those past the pooled map covering the dropped row / column with g = 0
+template <class T, bool ACC>
+__global__ void __launch_bounds__(256) pool_bwd_dx_kernel(const T* __restrict__ x, long long xbs, int C, int H, int W,
+                                                          const T* __restrict__ dP, const float2* __restrict__ saved,
+                                                          const float* __restrict__ weight, const float* __restrict__ bias,
+                                                          const float2* __restrict__ sums, float inv_n, T* __restrict__ dx, long long dbs) {
+  __shared__ float t[64][65];
+  const int b = blockIdx.z, c0 = blockIdx.y * 64, p0 = blockIdx.x * 64;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int Wq = (W + 1) >> 1, nwin = ((H + 1) >> 1) * Wq;
+  dp_tile(dP, b, C, c0, H >> 1, W >> 1, Wq, nwin, p0, t);
+  __syncthreads();
+#pragma unroll 2
+  for (int i = 0; i < 8; ++i) {
+    const int c = c0 + warp * 8 + i;
+    if (c >= C) continue;
+    const float2 st = saved[c], sm = sums[c];
+    const float mu = st.x, rs = st.y, w = weight[c], bb = bias[c], k = w * rs, m1 = sm.x * inv_n, m2 = sm.y * inv_n;
+    const T* plane = x + (size_t)b * xbs + (size_t)c * H * W;
+    T* dplane = dx + (size_t)b * dbs + (size_t)c * H * W;
+#pragma unroll
+    for (int kk = 0; kk < 2; ++kk) {
+      const int pl = lane + 32 * kk, q = p0 + pl;
+      if (q >= nwin) continue;
+      const int hq = q / Wq, wq = q - hq * Wq;
+      float v[4];
+      win_load(plane, H, W, hq, wq, v);
+      const float g = 0.25f * t[pl][warp * 8 + i];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int h = 2 * hq + (u >> 1), ww = 2 * wq + (u & 1);
+        if (h >= H || ww >= W) continue;
+        const float xh = (v[u] - mu) * rs;
+        const float gg = fmaf(w, xh, bb) > 0.f ? g : 0.f;
+        T* d = dplane + (size_t)h * W + ww;
+        float o = k * (gg - m1 - xh * m2);
+        if (ACC) o += ld1v(static_cast<const T*>(d));
+        st1v(d, o);
       }
     }
   }
@@ -635,6 +836,54 @@ int cl_bwd(const T* x, int B, int C, int HW, int x_is_cl, long long xbs, const T
   return 0;
 }
 
+// BatchNorm + ReLU + AvgPool2d(2) of a Transition: the segments of the backward reduction (as t_bwd_reduce's, over windows)
+static int pool_segments(int B, int C, int H, int W, int* chunks_per_seg) {
+  const int nchunks = cdiv((H / 2) * (W / 2), 64), ctiles = cdiv(C, 64);
+  const int nseg0 = std::max(1, std::min(nchunks, cdiv(T_RED_CTAS, ctiles * B)));
+  const int cps = cdiv(nchunks, nseg0);
+  if (chunks_per_seg) *chunks_per_seg = cps;
+  return cdiv(nchunks, cps);
+}
+
+template <class T>
+int pool_fwd(const T* x, int B, int C, int H, int W, long long xbs, int training, const float* w, const float* b, float* rm, float* rv,
+             float momentum, float eps, T* y, float* saved, const float* nchw_partial, int G, float n_each, float n_last, cudaStream_t st) {
+  const dim3 grid(cdiv((H / 2) * (W / 2), 64), cdiv(C, 64), B);
+  const float2* part = reinterpret_cast<const float2*>(nchw_partial);
+  if (training) {
+    pool_apply_kernel<T, false><<<grid, 256, 0, AACONV_ST(st)>>>(x, xbs, C, H, W, part, G, n_each, n_last, eps, momentum,
+                                                                 reinterpret_cast<float2*>(saved), rm, rv, w, b, y);
+    AACONV_LAUNCH_OK("bn_pool_apply");
+  } else {   // running statistics read only (the EVAL instantiation never writes through rm / rv)
+    pool_apply_kernel<T, true><<<grid, 256, 0, AACONV_ST(st)>>>(x, xbs, C, H, W, nullptr, 0, 0.f, 0.f, eps, 0.f, nullptr, rm, rv, w, b, y);
+    AACONV_LAUNCH_OK("bn_pool_eval");
+  }
+  return 0;
+}
+
+template <class T>
+int pool_bwd(const T* x, int B, int C, int H, int W, long long xbs, const T* dP, const float* saved, const float* w, const float* b, T* dx,
+             long long dbs, int acc, float* dw, float* db, float* ws, cudaStream_t st) {
+  float2* sums = reinterpret_cast<float2*>(ws);
+  float2* part = sums + C;
+  const float2* sv = reinterpret_cast<const float2*>(saved);
+  int cps = 0;
+  const int nseg = pool_segments(B, C, H, W, &cps), ctiles = cdiv(C, 64);
+  pool_bwd_reduce_kernel<T><<<dim3(nseg, ctiles, B), 256, 0, AACONV_ST(st)>>>(x, xbs, C, H, W, dP, sv, w, b, cps, part);
+  AACONV_LAUNCH_OK("bn_pool_bwd_reduce");
+  bn_fin_bwd_kernel<<<cdiv(C, 8), 256, 0, AACONV_ST(st)>>>(part, C, B * nseg, (long long)B * nseg, 1, sums, dw, db);
+  AACONV_LAUNCH_OK("bn_fin_bwd");
+  if (!dx) return 0;
+  const dim3 grid(cdiv(((H + 1) / 2) * ((W + 1) / 2), 64), ctiles, B);
+  const float inv_n = 1.f / ((float)B * H * W);
+  if (acc)
+    pool_bwd_dx_kernel<T, true><<<grid, 256, 0, AACONV_ST(st)>>>(x, xbs, C, H, W, dP, sv, w, b, sums, inv_n, dx, dbs);
+  else
+    pool_bwd_dx_kernel<T, false><<<grid, 256, 0, AACONV_ST(st)>>>(x, xbs, C, H, W, dP, sv, w, b, sums, inv_n, dx, dbs);
+  AACONV_LAUNCH_OK("bn_pool_bwd_dx");
+  return 0;
+}
+
 }  // namespace aaconv
 
 using namespace aaconv;
@@ -738,6 +987,61 @@ int aaconv_bn_relu_eval(const void* x, int dtype, int B, int C, int HW, int x_is
                        static_cast<bf16*>(y), st)
              : cl_eval(static_cast<const float*>(x), B, C, HW, x_is_cl, x_batch_stride, weight, bias, running_mean, running_var, eps,
                        static_cast<float*>(y), st);
+}
+
+// the limits the pooled kernels share: C % 4 == 0 (NHWC quads), at least one 2 x 2 window, four-element alignment of every tensor
+// and batch stride (checked before the null pointers: the workspace query returns 0 for a shape past them)
+static int pool_args_ok(const char* what, int dtype, int B, int C, int H, int W, int64_t xbs, const void* x, const void* p_cl,
+                        const void* dx, int64_t dbs) {
+  if (dtype != AACONV_FP32 && dtype != AACONV_BF16) return fail(AACONV_E_ARG, "%s: dtype must be fp32 or bf16", what);
+  if (B <= 0 || B > 65535 || H < 2 || W < 2 || C <= 0 || (C & 3))
+    return fail(AACONV_E_ARG, "%s: needs C a multiple of 4, H and W >= 2 and 1 <= B <= 65535 (got B=%d C=%d H=%d W=%d)", what, B, C, H, W);
+  if (xbs < (int64_t)C * H * W || (dx && dbs < (int64_t)C * H * W))
+    return fail(AACONV_E_ARG, "%s: batch strides must be >= C*H*W", what);
+  const size_t elt = dtype == AACONV_BF16 ? 2 : 4;
+  if (!aligned4(x, elt) || !aligned4(p_cl, elt) || (dx && !aligned4(dx, elt)) || ((size_t)xbs * elt) % (4 * elt) ||
+      (dx && ((size_t)dbs * elt) % (4 * elt)))
+    return fail(AACONV_E_ARG, "%s: tensors and batch strides must be aligned for four-element accesses", what);
+  return 0;
+}
+
+size_t aaconv_bn_relu_pool_workspace_bytes(int B, int C, int H, int W) {
+  if (B <= 0 || C <= 0 || H < 2 || W < 2) return 0;
+  return align256(sizeof(float) * 2 * ((size_t)C + (size_t)C * B * pool_segments(B, C, H, W, nullptr)));
+}
+
+int aaconv_bn_relu_pool_forward(const void* x, int dtype, int B, int C, int H, int W, int64_t x_batch_stride, int training,
+                                const float* weight, const float* bias, float* running_mean, float* running_var, float momentum, float eps,
+                                void* y_cl, float* saved, const void* nchw_stats, int stats_groups, int planes_per_group, void* stream) {
+  AACONV_TRY(pool_args_ok("bn_relu_pool_forward", dtype, B, C, H, W, x_batch_stride, x, y_cl, nullptr, 0));
+  if (!x || !weight || !bias || !y_cl) return fail(AACONV_E_ARG, "bn_relu_pool_forward: null tensor");
+  if (training && (!saved || !nchw_stats || stats_groups <= 0 || planes_per_group <= 0 ||
+                   stats_groups != (B + planes_per_group - 1) / planes_per_group || (running_mean == nullptr) != (running_var == nullptr)))
+    return fail(AACONV_E_ARG, "bn_relu_pool_forward: training needs saved and the group statistics of aaconv_bn_stats_nchw");
+  if (!training && (!running_mean || !running_var)) return fail(AACONV_E_ARG, "bn_relu_pool_forward: eval mode needs the running statistics");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int HW = H * W;
+  const float n_each = (float)planes_per_group * HW, n_last = (float)(B - (stats_groups - 1) * planes_per_group) * HW;
+  const float* part = static_cast<const float*>(nchw_stats);
+  return dtype == AACONV_BF16
+             ? pool_fwd(static_cast<const bf16*>(x), B, C, H, W, x_batch_stride, training, weight, bias, running_mean, running_var, momentum,
+                        eps, static_cast<bf16*>(y_cl), saved, part, stats_groups, n_each, n_last, st)
+             : pool_fwd(static_cast<const float*>(x), B, C, H, W, x_batch_stride, training, weight, bias, running_mean, running_var,
+                        momentum, eps, static_cast<float*>(y_cl), saved, part, stats_groups, n_each, n_last, st);
+}
+
+int aaconv_bn_relu_pool_backward(const void* x, int dtype, int B, int C, int H, int W, int64_t x_batch_stride, const void* dP_cl,
+                                 const float* saved, const float* weight, const float* bias, void* dx, int64_t dx_batch_stride,
+                                 int dx_accumulate, float* dweight, float* dbias, void* workspace, void* stream) {
+  AACONV_TRY(pool_args_ok("bn_relu_pool_backward", dtype, B, C, H, W, x_batch_stride, x, dP_cl, dx, dx_batch_stride));
+  if (!x || !dP_cl || !saved || !weight || !bias || !workspace) return fail(AACONV_E_ARG, "bn_relu_pool_backward: null tensor");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* ws = static_cast<float*>(workspace);
+  return dtype == AACONV_BF16
+             ? pool_bwd(static_cast<const bf16*>(x), B, C, H, W, x_batch_stride, static_cast<const bf16*>(dP_cl), saved, weight, bias,
+                        static_cast<bf16*>(dx), dx_batch_stride, dx_accumulate, dweight, dbias, ws, st)
+             : pool_bwd(static_cast<const float*>(x), B, C, H, W, x_batch_stride, static_cast<const float*>(dP_cl), saved, weight, bias,
+                        static_cast<float*>(dx), dx_batch_stride, dx_accumulate, dweight, dbias, ws, st);
 }
 
 }  // extern "C"

@@ -10,6 +10,7 @@ chexpert.py:90-123,504-518) loads strictly into this model and vice versa.  The 
     models/attn_aug_conv.py:411-446 _Transition -> transition()
     models/attn_aug_conv.py:448-517 DenseNet    -> DenseNet
     chexpert.py:474-476 'aadensenet121'         -> aadensenet121()
+    chexpert.py:24 torchvision densenet121      -> densenet121()  (Transitions: BNTransition with fused_transition)
 """
 from collections import OrderedDict
 
@@ -22,7 +23,7 @@ from torchvision.models.densenet import _DenseBlock, _DenseLayer
 
 from .aaconv import AAConv2d
 from .fused_bn import (bn_relu, tap_bn_relu, tap_bn_relu_cl, bn_relu_cl, cl_ok, slice_layout, _is_cl, bn_relu_eval, eval_ok,
-                       eval_cl_ok)
+                       eval_cl_ok, _fused_ok, pool_ok, bn_relu_pool, bn_relu_pool_eval)
 
 
 def transition_attn_dims(num_output_features, attn_params):
@@ -144,6 +145,73 @@ class _AppendCL(torch.autograd.Function):
         return g[:, :c], gn, None
 
 
+class _ToBuffer(torch.autograd.Function):
+    """A channels-last (B, Cout, H, W) tensor -> channels [0, Cout) of a new (B, out_total, H, W) NCHW feature buffer, which the next
+    BufferedDenseBlock adopts without a copy; backward hands the slice's gradient back channels-last (as _AppendCL does)."""
+
+    @staticmethod
+    def forward(ctx, z, out_total):
+        B, C, H, W = z.shape
+        buf = torch.empty(B, out_total, H, W, device=z.device, dtype=z.dtype)
+        view = _alias(buf, 0, C)
+        slice_layout(z.detach(), view, to_nchw=True)
+        ctx.mark_non_differentiable(buf)
+        return view, buf
+
+    @staticmethod
+    def backward(ctx, g, _gbuf):
+        B, C, H, W = g.shape
+        if _nchw_slice_ok(g) and g.is_cuda:
+            gn = torch.empty((B, C, H, W), device=g.device, dtype=g.dtype, memory_format=torch.channels_last)
+            slice_layout(g, gn, to_nchw=False)
+        else:
+            gn = g.contiguous(memory_format=torch.channels_last)
+        return gn, None
+
+
+class BNTransition(nn.Sequential):
+    """torchvision's ``_Transition`` (BatchNorm2d -> ReLU -> Conv2d 1x1 -> AvgPool2d(2), densenet.py:98-104) with its child names
+    ``norm`` / ``relu`` / ``conv`` / ``pool``, so state_dicts are interchangeable, and a fused route on CUDA.
+
+    There the BatchNorm + ReLU + 2x2 average run as one kernel (fused_bn.bn_relu_pool) that reads the finished feature buffer once
+    and writes the pooled operand channels-last; the 1x1 convolution (cuDNN, as in the dense layers) then runs on a quarter of the
+    pixels -- the pool and the per-pixel linear convolution commute.  In training the kernel reuses the block's shared BatchNorm
+    statistics (``x.bn_stats``, set by BufferedDenseBlock), so only the block's last layer's channels are reduced again.
+    ``forward(x, out_total=C)`` writes the result into channels [0, Cout) of a new (B, C, H/2, W/2) buffer, attached as
+    ``.feature_buffer`` for the next block to adopt.
+
+    The fused route is taken in training on CUDA, and in eval mode with autograd off when ``fused_eval``; C and Cout multiples of 4,
+    H and W >= 2, (H/2)(W/2) a multiple of 4 and four-element alignment are required (fused_bn.pool_ok).  Anything else -- CPU, eval
+    with grad enabled (Grad-CAM), a shape past those limits -- runs the four modules unchanged."""
+
+    def __init__(self, num_input_features, num_output_features, fused_eval=False):
+        super().__init__(OrderedDict([
+            ('norm', nn.BatchNorm2d(num_input_features)),
+            ('relu', nn.ReLU(inplace=True)),
+            ('conv', nn.Conv2d(num_input_features, num_output_features, kernel_size=1, stride=1, bias=False)),
+            ('pool', nn.AvgPool2d(kernel_size=2, stride=2)),
+        ]))
+        self.fused_eval = bool(fused_eval)
+
+    def _fused(self, x):
+        if x.dim() != 4 or not (self.training or self.fused_eval) or not pool_ok(self.norm, x):
+            return False
+        H, W = x.shape[2:]
+        return self.conv.out_channels % 4 == 0 and ((H // 2) * (W // 2)) % 4 == 0      # aaconv_slice_layout into the next buffer
+
+    def forward(self, x, out_total=None):
+        if not self._fused(x):
+            return super().forward(x)
+        if self.training:
+            p = bn_relu_pool(self.norm, x, getattr(x, 'bn_stats', None))
+        else:
+            p = bn_relu_pool_eval(self.norm, x)
+        z = F.conv2d(p, self.conv.weight).contiguous(memory_format=torch.channels_last)
+        y, buf = _ToBuffer.apply(z, int(out_total or z.shape[1]))
+        y.feature_buffer = buf
+        return y
+
+
 class BufferedDenseBlock(nn.ModuleDict):
     """torchvision's ``_DenseBlock`` (same ``denselayer%d`` children, parameters and arithmetic; the reference uses it at
     models/attn_aug_conv.py:479-482) over ONE pre-allocated (B, C_in + n * growth, H, W) feature buffer: layer i reads channels
@@ -197,6 +265,7 @@ class BufferedDenseBlock(nn.ModuleDict):
         stats = torch.empty(2 * B * self.out_channels, device=buf.device, dtype=torch.float32) if buf.is_cuda else None
         valid = 0
         growth_ok = self.growth_rate % 4 == 0 and (H * W) % 4 == 0 and stats is not None
+        shared = stats is not None          # every norm1 reduced its new channels into `stats` (the fused kernels ran)
         for layer in self.values():
             # norm -> relu pairs: fused strided kernels in training on CUDA (chexpert_b200.fused_bn), the torch modules otherwise
             c = feats.shape[1]
@@ -216,21 +285,28 @@ class BufferedDenseBlock(nn.ModuleDict):
                 feats = (_AppendCL.apply(feats, new, buf) if _is_cl(new) else _Append.apply(feats, new.contiguous(), buf))
                 continue
             # norm1 taps the concatenated features: backward adds its dx into the gradient of the concatenation in place
+            shared = shared and _fused_ok(layer.norm1, feats)
             feats, y1 = tap_bn_relu(layer.norm1, feats, None if stats is None else (stats, valid))
             new = layer.conv2(bn_relu(layer.norm2, layer.conv1(y1)))
             valid = c
             if layer.drop_rate > 0:
                 new = F.dropout(new, p=layer.drop_rate, training=self.training)
             feats = _Append.apply(feats, new.to(buf.dtype), buf)
+        if shared:
+            # the statistics of channels [0, valid) of the output are in `stats`: a BNTransition reduces only the last layer's channels
+            feats.bn_stats = (stats, valid)
         return feats
 
 
 class DenseNet(nn.Module):
     """DenseNet with attention-augmented transitions; constructor of models/attn_aug_conv.py:452-453 plus
-    ``precision`` ('fp32' | 'bf16') for the AAConv2d kernels.  Unlike the reference, ``attn_params`` is not mutated."""
+    ``precision`` ('fp32' | 'bf16') for the AAConv2d kernels.  Unlike the reference, ``attn_params`` is not mutated.
+    With ``attn_params=None`` it is torchvision's DenseNet (same state_dict); ``fused_transition=True`` with ``feature_buffer=True``
+    then builds BNTransition (fused BatchNorm + ReLU + pool kernel) in place of the module Transition."""
 
     def __init__(self, growth_rate=32, block_config=(6, 12, 24, 16), num_init_features=64, bn_size=4, drop_rate=0,
-                 num_classes=1000, attn_params=None, precision=None, feature_buffer=False, fused_prologue=False, fused_eval=False):
+                 num_classes=1000, attn_params=None, precision=None, feature_buffer=False, fused_prologue=False, fused_eval=False,
+                 fused_transition=False):
         super().__init__()
         self.feature_buffer = bool(feature_buffer)
         self.fused_eval = bool(fused_eval)
@@ -255,7 +331,11 @@ class DenseNet(nn.Module):
             self.features.add_module(f'denseblock{i + 1}', block)
             width += num_layers * growth_rate
             if i != len(block_config) - 1:
-                self.features.add_module(f'transition{i + 1}', transition(width, width // 2, attn, precision, fused_prologue))
+                if attn is None and feature_buffer and fused_transition:
+                    trans = BNTransition(width, width // 2, fused_eval)
+                else:
+                    trans = transition(width, width // 2, attn, precision, fused_prologue)
+                self.features.add_module(f'transition{i + 1}', trans)
                 width //= 2
             if attn is not None:      # every stage halves the map the next transition's attention sees (:491-493)
                 attn['input_dims'] = attn['input_dims'][0] // 2, attn['input_dims'][1] // 2
@@ -288,8 +368,8 @@ class DenseNet(nn.Module):
                 skip = False
                 continue
             nxt = mods[i + 1][1] if i + 1 < len(mods) else None
-            if isinstance(m, AATransition) and isinstance(nxt, BufferedDenseBlock):
-                x = m(x, out_total=nxt.out_channels)      # the AAConv2d epilogues write into the next block's buffer
+            if isinstance(m, (AATransition, BNTransition)) and isinstance(nxt, BufferedDenseBlock):
+                x = m(x, out_total=nxt.out_channels)      # the Transition writes into the next block's buffer
             elif isinstance(m, nn.BatchNorm2d) and isinstance(nxt, nn.ReLU):
                 x = self._bn_relu(m, x)                   # stem: norm0 -> relu0 as one fused op (grid (C, B) instead of one CTA per channel)
                 skip = True
@@ -316,3 +396,12 @@ def aadensenet121(num_classes=5, input_dims=(320, 320), precision=None, feature_
     return DenseNet(32, (6, 12, 24, 16), 64, num_classes=num_classes,
                     attn_params={'k': 0.2, 'v': 0.1, 'nh': 8, 'relative': True, 'input_dims': tuple(input_dims)},
                     precision=precision, feature_buffer=feature_buffer, fused_prologue=fused_prologue, fused_eval=fused_eval)
+
+
+def densenet121(num_classes=5, feature_buffer=False, fused_transition=False, fused_eval=False):
+    """The model behind ``--model densenet121`` (chexpert.py:24): torchvision's densenet121 -- same 727 state_dict keys and shapes,
+    6,958,981 parameters at 5 classes, so torchvision's state_dict (e.g. ImageNet-initialised weights with the classifier replaced)
+    loads strictly.  ``feature_buffer`` / ``fused_eval``: the dense-block execution options of aadensenet121;
+    ``fused_transition`` (with ``feature_buffer``): the Transitions run as BNTransition.  None of them adds parameters."""
+    return DenseNet(32, (6, 12, 24, 16), 64, num_classes=num_classes, attn_params=None, feature_buffer=feature_buffer,
+                    fused_eval=fused_eval, fused_transition=fused_transition)

@@ -18,7 +18,7 @@ import torch.nn.functional as F
 
 from . import _lib
 from .aaconv import AAConv2d, _ptr, _stream
-from .densenet import aadensenet121
+from .densenet import aadensenet121, densenet121
 from .loss import BCEWithLogitsLoss
 
 PIXEL_MEAN, PIXEL_STD = 0.5330, 0.0349        # chexpert.py:70-72
@@ -124,17 +124,26 @@ class Predictor:
     ``cuda_graph``: after WARMUP eager batches (cuDNN picks its algorithms) one graph of the whole step at ``batch_size`` is
     captured and replayed.  A ragged last batch is padded to ``batch_size`` (samples are independent in eval mode) and sliced.
     load_state_dict writes parameters and buffers in place, so one capture serves every checkpoint of an ensemble;
-    ``captures`` counts the captures made."""
+    ``captures`` counts the captures made.
+
+    ``arch='densenet121'``: the reference's baseline, torchvision's densenet121, as densenet121(feature_buffer=True,
+    fused_transition=True, fused_eval=True) -- its Transitions' BatchNorm + ReLU + pool run through the eval-mode pooled kernel."""
 
     WARMUP = 2
 
-    def __init__(self, num_classes=5, size=320, precision='bf16', batch_size=16, device='cuda', autocast=False, cuda_graph=True):
+    def __init__(self, num_classes=5, size=320, precision='bf16', batch_size=16, device='cuda', autocast=False, cuda_graph=True,
+                 arch='aadensenet121'):
         self.device = torch.device(device)
         if self.device.type != 'cuda':
             raise RuntimeError('chexpert_b200.evaluate.Predictor runs on CUDA only; there is no CPU fallback')
         self.num_classes, self.size, self.batch_size = num_classes, size, int(batch_size)
         self.autocast = bool(autocast)
-        model = aadensenet121(num_classes, (size, size), precision=precision, feature_buffer=True, fused_prologue=True, fused_eval=True)
+        if arch == 'aadensenet121':
+            model = aadensenet121(num_classes, (size, size), precision=precision, feature_buffer=True, fused_prologue=True, fused_eval=True)
+        elif arch == 'densenet121':
+            model = densenet121(num_classes, feature_buffer=True, fused_transition=True, fused_eval=True)
+        else:
+            raise ValueError(f"Predictor: arch must be 'aadensenet121' or 'densenet121', got {arch!r}")
         model.requires_grad_(False)
         # the dense layers' convolutions see NHWC activations, so their k x k weights are kept channels-last (in fp32 too: cuDNN would
         # otherwise transpose an NCHW weight on every call); 1 x 1 weights are the same bytes in both formats

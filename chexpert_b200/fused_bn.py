@@ -3,6 +3,7 @@ slice of the pre-allocated DenseBlock feature buffer (SURVEY.md section 8 row f3
 models/attn_aug_conv.py:479-482).  Parameters, buffers and the arithmetic are nn.BatchNorm2d's (same state_dict, same running
 statistics update); eval mode and CPU tensors go through the module's own forward.  bn_relu_eval is the eval-mode counterpart
 (running statistics, no backward) that the dense blocks take only when asked to (DenseNet(fused_eval=True)) and autograd is off.
+bn_relu_pool / bn_relu_pool_eval add the 2x2 average pool of torchvision's Transition (densenet.BNTransition).
 """
 import ctypes
 
@@ -301,6 +302,95 @@ def bn_relu_eval(bn, x, out_cl=False):
         _lib.check(lib.aaconv_bn_relu_eval(_ptr(x), _DT[x.dtype], B, C, H * W, int(x_is_cl), C * H * W if x_is_cl else x.stride(0),
                                            _ptr(w), _ptr(b), _ptr(bn.running_mean), _ptr(bn.running_var), float(bn.eps), _ptr(y),
                                            int(out_cl), _stream()), 'aaconv_bn_relu_eval')
+    return y
+
+
+# ------------------------------------------------------------------------------------------------
+# BatchNorm2d + ReLU + AvgPool2d(2) of torchvision's Transition (csrc/bn_cl.cu, pool_* kernels): the pool runs ahead of the 1x1
+# convolution, on the channels-last operand the convolution reads
+# ------------------------------------------------------------------------------------------------
+def pool_ok(bn, x):
+    """bn_relu_pool (bn training) / bn_relu_pool_eval (bn in eval mode, autograd off: see eval_ok) take x: a CUDA fp32 / bf16
+    (B, C, H, W) tensor with dense samples (e.g. a dense block's feature buffer), C a multiple of 4, H and W >= 2, and x and its
+    batch stride aligned for four-element accesses."""
+    if not (x.is_cuda and x.dim() == 4 and x.dtype in _DT):
+        return False
+    B, C, H, W = x.shape
+    shape_ok = (C % 4 == 0 and H >= 2 and W >= 2 and B <= 65535 and _strided_ok(x) and x.stride(0) % 4 == 0
+                and x.data_ptr() % (4 * x.element_size()) == 0)
+    if bn.training:
+        return shape_ok and bn.affine and bn.track_running_stats and bn.momentum is not None
+    return shape_ok and eval_ok(bn, x)
+
+
+class _BNReLUPool(torch.autograd.Function):
+    """P = avgpool2(relu(bn(x))) channels-last (B, C, H // 2, W // 2) for a training-mode BatchNorm2d; backward takes dP
+    channels-last and returns dx for every pixel of x."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, running_mean, running_var, momentum, eps, stats):
+        lib = _lib.load()
+        B, C, H, W = x.shape
+        xs = x.detach()
+        w, b = weight.detach().float().contiguous(), bias.detach().float().contiguous()
+        with torch.cuda.device(x.device):
+            y = torch.empty((B, C, H // 2, W // 2), device=x.device, dtype=x.dtype, memory_format=_CL)
+            saved = torch.empty(C, 2, device=x.device, dtype=torch.float32)
+            # stats = (buffer, n_valid): the dense block's shared plane statistics; channels [0, n_valid) of x are already in it
+            if stats is not None and stats[0].numel() * 4 >= 8 * B * C:
+                pst, valid = stats[0], min(int(stats[1]), C)
+            else:
+                pst, valid = torch.empty(lib.aaconv_bn_relu_workspace_bytes(B, C) // 4, device=x.device, dtype=torch.float32), 0
+            G, bpb = ctypes.c_int(0), ctypes.c_int(0)
+            _lib.check(lib.aaconv_bn_stats_nchw(_ptr(xs), _DT[x.dtype], B, C, H * W, xs.stride(0), _ptr(pst), valid, ctypes.byref(G),
+                                                ctypes.byref(bpb), _stream()), 'aaconv_bn_stats_nchw')
+            _lib.check(lib.aaconv_bn_relu_pool_forward(_ptr(xs), _DT[x.dtype], B, C, H, W, xs.stride(0), 1, _ptr(w), _ptr(b),
+                                                       _ptr(running_mean), _ptr(running_var), float(momentum), float(eps), _ptr(y),
+                                                       _ptr(saved), _ptr(pst), G.value, bpb.value, _stream()), 'aaconv_bn_relu_pool_forward')
+        ctx.save_for_backward(xs, saved, w, b)
+        return y
+
+    @staticmethod
+    def backward(ctx, dP):
+        lib = _lib.load()
+        xs, saved, w, b = ctx.saved_tensors
+        B, C, H, W = xs.shape
+        g = dP.detach().to(xs.dtype).contiguous(memory_format=_CL)
+        need = ctx.needs_input_grad
+        with torch.cuda.device(xs.device):
+            dx = torch.empty(B, C, H, W, device=xs.device, dtype=xs.dtype) if need[0] else None
+            dw = torch.empty(C, device=xs.device, dtype=torch.float32) if need[1] else None
+            db = torch.empty(C, device=xs.device, dtype=torch.float32) if need[2] else None
+            ws = torch.empty(lib.aaconv_bn_relu_pool_workspace_bytes(B, C, H, W), device=xs.device, dtype=torch.uint8)
+            _lib.check(lib.aaconv_bn_relu_pool_backward(_ptr(xs), _DT[xs.dtype], B, C, H, W, xs.stride(0), _ptr(g), _ptr(saved), _ptr(w),
+                                                        _ptr(b), _ptr(dx), C * H * W, 0, _ptr(dw), _ptr(db), _ptr(ws), _stream()),
+                       'aaconv_bn_relu_pool_backward')
+        return dx, dw, db, None, None, None, None, None
+
+
+def bn_relu_pool(bn, x, stats=None):
+    """avgpool2(relu(bn(x))) as a channels-last (B, C, H // 2, W // 2) tensor for a training-mode nn.BatchNorm2d `bn` (batch statistics
+    over all H x W pixels, running statistics and num_batches_tracked updated as the module does).  ``stats = (float32 buffer of
+    >= 2*B*C elements, n_valid_channels)``: a dense block's shared plane statistics (see bn_relu).  See pool_ok for what x may be."""
+    if not (bn.training and pool_ok(bn, x)):
+        raise RuntimeError('fused_bn.bn_relu_pool needs a training-mode affine BatchNorm2d with running statistics and a CUDA fp32 / bf16 '
+                           'input with dense samples, C a multiple of 4, H and W >= 2, aligned for four-element accesses')
+    _bump(bn)
+    return _BNReLUPool.apply(x, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.momentum, bn.eps, stats)
+
+
+def bn_relu_pool_eval(bn, x):
+    """bn_relu_pool for an eval-mode nn.BatchNorm2d under no_grad: the running statistics are read, never written; no backward."""
+    if bn.training or not pool_ok(bn, x):
+        raise RuntimeError('fused_bn.bn_relu_pool_eval needs an eval-mode affine BatchNorm2d with running statistics, autograd off and '
+                           'a CUDA fp32 / bf16 input with dense samples, C a multiple of 4, H and W >= 2, aligned for four-element accesses')
+    lib = _lib.load()
+    B, C, H, W = x.shape
+    with torch.cuda.device(x.device):
+        y = torch.empty((B, C, H // 2, W // 2), device=x.device, dtype=x.dtype, memory_format=_CL)
+        _lib.check(lib.aaconv_bn_relu_pool_forward(_ptr(x), _DT[x.dtype], B, C, H, W, x.stride(0), 0, _ptr(bn.weight), _ptr(bn.bias),
+                                                   _ptr(bn.running_mean), _ptr(bn.running_var), 0.0, float(bn.eps), _ptr(y), None, None,
+                                                   0, 0, _stream()), 'aaconv_bn_relu_pool_forward')
     return y
 
 

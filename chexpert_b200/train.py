@@ -15,7 +15,7 @@ import torch.distributed as dist
 
 from . import _lib
 from .dataparallel import GradientBuckets
-from .densenet import aadensenet121
+from .densenet import aadensenet121, densenet121
 from .loss import BCEWithLogitsLoss
 
 # dataset normalisation constants of the reference transform (chexpert.py:70-72)
@@ -42,11 +42,18 @@ class TrainStep:
 
     def __init__(self, device, size=320, precision='bf16', lr=1e-4, raw_labels=True, bucket_mb=25.0, seed=0,
                  autocast=True, channels_last=False, cuda_graph=False, graph_after=2, buffered=False, fused_prologue=False,
-                 batched_casts=True):
+                 batched_casts=True, arch='aadensenet121'):
         torch.manual_seed(seed)
         self.device = torch.device(device)
-        self.model = aadensenet121(5, (size, size), precision=precision, feature_buffer=buffered,
-                                   fused_prologue=fused_prologue).to(self.device)
+        # arch: 'aadensenet121' or the reference's baseline 'densenet121' (torchvision's network; `precision` only concerns AAConv2d,
+        # and `fused_prologue` selects its fused BatchNorm + ReLU + pool Transitions).  The optimizer is the same for both.
+        if arch == 'aadensenet121':
+            model = aadensenet121(5, (size, size), precision=precision, feature_buffer=buffered, fused_prologue=fused_prologue)
+        elif arch == 'densenet121':
+            model = densenet121(5, feature_buffer=buffered, fused_transition=fused_prologue)
+        else:
+            raise ValueError(f"TrainStep: arch must be 'aadensenet121' or 'densenet121', got {arch!r}")
+        self.model = model.to(self.device)
         if channels_last:
             self.model = self.model.to(memory_format=torch.channels_last)
         self.loss_fn = BCEWithLogitsLoss('train', raw_labels=raw_labels).to(self.device)

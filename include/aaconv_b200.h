@@ -197,6 +197,29 @@ int aaconv_bn_relu_eval(const void* x, int dtype, int B, int C, int HW, int x_is
                         const float* weight, const float* bias, const float* running_mean, const float* running_var,
                         float eps, void* y, int y_is_cl, void* stream);
 
+/* The Transition of torchvision's DenseNet (BatchNorm2d -> ReLU -> Conv2d 1x1 -> AvgPool2d(2), tv densenet.py:98-104) with the pool
+ * moved ahead of the 1x1 convolution, which it commutes with: P = avgpool2(relu(bn(x))), the caller convolves P.
+ * x: (B, C, H, W) NCHW of `dtype` (AACONV_FP32 | AACONV_BF16) with x_batch_stride >= C*H*W elements between samples (the finished
+ * feature buffer of a dense block).  P, dP: (B, H/2, W/2, C) NHWC dense, floor mode (an odd last row / column is in no window).
+ * C a multiple of 4, H and W >= 2, B <= 65535, every tensor and batch stride aligned for four-element accesses.
+ *   aaconv_bn_relu_pool_forward   training != 0: batch statistics over ALL H*W pixels from the group statistics of
+ *                                 aaconv_bn_stats_nchw in nchw_stats (stats_groups, planes_per_group as it returns them; a dense block's
+ *                                 shared buffer with only the channels it has not reduced added); writes saved (C) x (mean, rstd) and
+ *                                 updates running_mean / running_var (may both be NULL) as nn.BatchNorm2d does (momentum, unbiased
+ *                                 variance).  training == 0: BatchNorm2d in eval mode from the running statistics, which are read,
+ *                                 never written (saved, nchw_stats unused).
+ *   aaconv_bn_relu_pool_backward  (training mode) dP -> dx for EVERY pixel of x (the dropped row / column gets the mean terms),
+ *                                 through dx_batch_stride, ADDED onto what is there when dx_accumulate; dx may be NULL.  dweight / dbias
+ *                                 (C) are WRITTEN (may be NULL).  Fixed-order reductions.
+ *   workspace: aaconv_bn_relu_pool_workspace_bytes(B, C, H, W) bytes (backward only). */
+size_t aaconv_bn_relu_pool_workspace_bytes(int B, int C, int H, int W);
+int aaconv_bn_relu_pool_forward(const void* x, int dtype, int B, int C, int H, int W, int64_t x_batch_stride, int training,
+                                const float* weight, const float* bias, float* running_mean, float* running_var, float momentum, float eps,
+                                void* y_cl, float* saved, const void* nchw_stats, int stats_groups, int planes_per_group, void* stream);
+int aaconv_bn_relu_pool_backward(const void* x, int dtype, int B, int C, int H, int W, int64_t x_batch_stride, const void* dP_cl,
+                                 const float* saved, const float* weight, const float* bias, void* dx, int64_t dx_batch_stride,
+                                 int dx_accumulate, float* dweight, float* dbias, void* workspace, void* stream);
+
 /* Accounting / measurement helpers used by bench.py (no reference counterpart).
  *   aaconv_launch_count   kernels launched by this library since it was loaded (all threads).
  *   aaconv_profile_begin  start recording a (start, stop) CUDA-event pair around every launch (`stream` is unused, kept for ABI).
