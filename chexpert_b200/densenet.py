@@ -23,7 +23,7 @@ from torchvision.models.densenet import _DenseBlock, _DenseLayer
 
 from .aaconv import AAConv2d
 from .fused_bn import (bn_relu, tap_bn_relu, tap_bn_relu_cl, bn_relu_cl, cl_ok, slice_layout, _is_cl, bn_relu_eval, eval_ok,
-                       eval_cl_ok, _fused_ok, pool_ok, bn_relu_pool, bn_relu_pool_eval)
+                       eval_cl_ok, _fused_ok, pool_ok, bn_relu_pool, bn_relu_pool_eval, module_bn)
 
 
 def transition_attn_dims(num_output_features, attn_params):
@@ -182,7 +182,8 @@ class BNTransition(nn.Sequential):
 
     The fused route is taken in training on CUDA, and in eval mode with autograd off when ``fused_eval``; C and Cout multiples of 4,
     H and W >= 2, (H/2)(W/2) a multiple of 4 and four-element alignment are required (fused_bn.pool_ok).  Anything else -- CPU, eval
-    with grad enabled (Grad-CAM), a shape past those limits -- runs the four modules unchanged."""
+    with grad enabled (Grad-CAM), a shape past those limits -- runs the four modules unchanged (the norm through fused_bn.module_bn,
+    so that a num_batches_tracked which TrainStep bumps is not bumped twice)."""
 
     def __init__(self, num_input_features, num_output_features, fused_eval=False):
         super().__init__(OrderedDict([
@@ -201,7 +202,7 @@ class BNTransition(nn.Sequential):
 
     def forward(self, x, out_total=None):
         if not self._fused(x):
-            return super().forward(x)
+            return self.pool(self.conv(self.relu(module_bn(self.norm, x))))
         if self.training:
             p = bn_relu_pool(self.norm, x, getattr(x, 'bn_stats', None))
         else:

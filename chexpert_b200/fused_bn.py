@@ -110,6 +110,15 @@ def _fused_ok(bn, x):
             and bn.momentum is not None and _strided_ok(x) and x.shape[0] <= 65535)
 
 
+def module_bn(bn, x):
+    """bn(x) through the module's own arithmetic, for the paths that do not run the fused kernels.  A counter that TrainStep bumps
+    itself (``_nbt_batched``) must not be bumped again by nn.BatchNorm2d.forward: for a training-mode module with a momentum that
+    forward is F.batch_norm with the module's buffers and parameters, plus the bump, so F.batch_norm is called without it."""
+    if getattr(bn, '_nbt_batched', False) and bn.training and bn.track_running_stats and bn.momentum is not None:
+        return F.batch_norm(x, bn.running_mean, bn.running_var, bn.weight, bn.bias, True, bn.momentum, bn.eps)
+    return bn(x)
+
+
 def tap_bn_relu(bn, x, stats=None):
     """-> (x handed on, relu(bn(x))): bn_relu for an input that has a second consumer (the concatenation of a dense block)."""
     if not (_fused_ok(bn, x) and torch.is_grad_enabled() and x.requires_grad):
@@ -126,7 +135,7 @@ def bn_relu(bn, x, stats=None):
     fused = (bn.training and x.is_cuda and x.dim() == 4 and x.dtype in _DT and bn.affine and bn.track_running_stats
              and bn.momentum is not None and _strided_ok(x) and x.shape[0] <= 65535)
     if not fused:
-        return F.relu(bn(x), inplace=True)
+        return F.relu(module_bn(bn, x), inplace=True)
     if bn.num_batches_tracked is not None and not getattr(bn, '_nbt_batched', False):   # TrainStep bumps all counters in one launch
         bn.num_batches_tracked.add_(1)
     return _BNReLU.apply(x, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.momentum, bn.eps, stats)

@@ -83,6 +83,31 @@ def test_bn_transition_on_cpu_is_the_module_path():
         assert torch.equal(t(x), ref(x))
 
 
+def test_module_fallbacks_leave_a_batched_counter_alone():
+    """TrainStep(buffered=True) bumps every num_batches_tracked once per step itself (one foreach add, `_nbt_batched`).  Where
+    bn_relu, tap_bn_relu and BNTransition run the modules (here: on the CPU; on the GPU for inputs the kernels do not take) the norm
+    must not count the batch a second time, and must otherwise be the module's own arithmetic, bit for bit."""
+    x = torch.randn(2, 64, 9, 8, generator=torch.Generator().manual_seed(1))
+    torch.manual_seed(0)
+    ref = torchvision.models.densenet._Transition(64, 32)
+    t = densenet.BNTransition(64, 32)
+    t.load_state_dict(ref.state_dict(), strict=True)
+    t.norm._nbt_batched = True
+    pairs = [('BNTransition', ref(x), t(x, out_total=48), ref.norm, t.norm)]
+    for name, fn in (('bn_relu', fused_bn.bn_relu), ('tap_bn_relu', lambda bn, v: fused_bn.tap_bn_relu(bn, v)[1])):
+        a = torch.nn.BatchNorm2d(64)
+        with torch.no_grad():
+            a.weight.uniform_(0.5, 1.5), a.bias.uniform_(-0.5, 0.5)
+        b = torch.nn.BatchNorm2d(64)
+        b.load_state_dict(a.state_dict())
+        b._nbt_batched = True
+        pairs.append((name, F.relu(a(x)), fn(b, x), a, b))
+    for name, want, got, a, b in pairs:
+        assert torch.equal(got, want), name
+        assert torch.equal(b.running_mean, a.running_mean) and torch.equal(b.running_var, a.running_var), name
+        assert int(a.num_batches_tracked) == 1 and int(b.num_batches_tracked) == 0, (name, int(b.num_batches_tracked))
+
+
 # ------------------------------------------------------------------------------------------------ GPU: the kernels against float64
 def _dt(dtype):
     return _lib.FP32 if dtype == torch.float32 else _lib.BF16
@@ -464,6 +489,24 @@ def test_train_step_densenet121(precision, no_tf32, monkeypatch):
     e, ec = float((du - dr).norm() / dr.norm()), float((dc - dr).norm() / dr.norm())
     print(f'{precision}: parameter updates {e:.3g} of their L2 norm (plain TrainStep: {ec:.3g})')
     assert e <= max(tol, CTL_FACTOR * ec), (e, ec)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize('channels_last', [False, True], ids=['nchw', 'channels_last'])
+def test_train_step_densenet121_counts_each_batch_once(channels_last):
+    """TrainStep(buffered=True) bumps every num_batches_tracked itself, so the BatchNorms that run as modules must not bump it again.
+    At 288 px transition3 sees 18 x 18 maps: their 9 x 9 pool is past the fused route's limit ((H/2)(W/2) a multiple of 4), so it
+    runs the four modules; with channels_last the stem's conv0 writes a channels-last map, which norm0 takes through the module."""
+    from chexpert_b200.train import TrainStep, synthetic_batch
+    ts = TrainStep('cuda', size=288, precision='bf16', lr=1e-3, seed=0, arch='densenet121', buffered=True, fused_prologue=True,
+                   channels_last=channels_last)
+    t3 = ts.model.features.transition3
+    assert isinstance(t3, densenet.BNTransition) and not t3._fused(torch.empty(2, 1024, 18, 18, device='cuda'))
+    x, t = synthetic_batch(2, size=288, seed=5, device='cuda')
+    for _ in range(2):
+        ts(x, t)
+    counts = {n: int(m.num_batches_tracked) for n, m in ts.model.named_modules() if isinstance(m, torch.nn.BatchNorm2d)}
+    assert len(counts) == 121 and all(c == 2 for c in counts.values()), {n: c for n, c in counts.items() if c != 2}
 
 
 @pytest.mark.gpu

@@ -7,7 +7,8 @@ import pytest
 import torch
 
 from oracle import aaconv_oracle as O
-from tests.helpers import GOLDEN, golden_cases, load_case, rel_err
+from oracle import model_oracle as M
+from tests.helpers import GOLDEN, golden_cases, load_case, load_fixture, rel_err
 
 
 def test_rel_to_abs_matches_reference():
@@ -123,3 +124,42 @@ def test_ensemble_mean_and_auroc():
     t[::2] = 1
     perfect = t * 2 - 1
     assert O.auroc_per_class(perfect, t) == [1.0] * 5
+
+
+# The reference model (oracle/model_oracle.py) in float64 against the reference's own fp32 forward / backward of the tiny DenseNet.
+# The fixture is fp32, so its rounding is the floor: measured 2.2e-6 (logits, of max), 4.4e-8 (loss) and 1.7e-5 (worst of the 17
+# gradients, transition2.conv.key_rel_h, of its max).  The gates sit ~5x above those; a wrong wiring (a missed stem /4, a swapped
+# dk / dv, a Transition without its InstanceNorm) moves the logits by O(1).
+TINY_OUT_TOL, TINY_LOSS_TOL, TINY_GRAD_TOL = 1e-5, 2e-7, 1e-4
+
+
+def test_reference_model_reproduces_the_tiny_densenet_fixture():
+    z = load_fixture('tiny_densenet')
+    m = M.RefDenseNet(16, (2, 2, 2, 2), 32, {'k': 0.5, 'v': 0.5, 'nh': 8, 'relative': True}, (64, 64))
+    m.load_state_dict({k[3:]: torch.from_numpy(z[k]) for k in z if k.startswith('sd.')}, strict=True)
+    m = m.double().train()
+    out = m(torch.from_numpy(z['x']).double())
+    loss = O.bce_with_logits(out, torch.from_numpy(z['t']).double()).sum(1).mean(0)
+    loss.backward()
+    assert rel_err(out.detach(), torch.from_numpy(z['out'])) < TINY_OUT_TOL
+    assert rel_err(loss.detach(), torch.from_numpy(z['loss'])) < TINY_LOSS_TOL
+    grads = {k: p.grad for k, p in m.named_parameters()}
+    names = [k[2:] for k in z if k.startswith('g.')]
+    assert len(names) == 17 and set(names) <= set(grads)
+    for k in names:
+        assert rel_err(grads[k], torch.from_numpy(z['g.' + k])) < TINY_GRAD_TOL, k
+
+
+def test_reference_aadensenet121_has_the_models_state_dict():
+    """The 320-px reference and chexpert_b200's aadensenet121: the same state_dict keys in the same order, the shapes of the
+    reference's own model (tests/golden/aadensenet121_meta.json), and strict loads both ways."""
+    from chexpert_b200.densenet import aadensenet121
+    meta = json.load(open(os.path.join(GOLDEN, 'aadensenet121_meta.json')))
+    ref, ours = M.ref_aadensenet121((320, 320)).state_dict(), aadensenet121(5, (320, 320)).state_dict()
+    assert list(ref) == list(ours) and set(ref) == set(meta['state_dict'])
+    for k, v in ref.items():
+        assert list(v.shape) == list(ours[k].shape) == meta['state_dict'][k], k
+    assert sum(v.numel() for k, v in ref.items() if not k.endswith(('running_mean', 'running_var', 'num_batches_tracked'))) \
+        == meta['n_params']
+    M.ref_aadensenet121((320, 320)).load_state_dict(ours, strict=True)
+    aadensenet121(5, (320, 320)).load_state_dict(ref, strict=True)
