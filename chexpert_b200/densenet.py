@@ -23,7 +23,7 @@ from torchvision.models.densenet import _DenseBlock, _DenseLayer
 
 from .aaconv import AAConv2d
 from .fused_bn import (bn_relu, tap_bn_relu, tap_bn_relu_cl, bn_relu_cl, cl_ok, slice_layout, _is_cl, bn_relu_eval, eval_ok,
-                       eval_cl_ok, _fused_ok, pool_ok, bn_relu_pool, bn_relu_pool_eval, module_bn)
+                       eval_cl_ok, _fused_ok, pool_ok, bn_relu_pool, bn_relu_pool_eval, module_bn, _alias, _strided_ok)
 
 
 def transition_attn_dims(num_output_features, attn_params):
@@ -75,14 +75,6 @@ def transition(num_input_features, num_output_features, attn_params=None, precis
 # ------------------------------------------------------------------------------------------------
 # pre-allocated DenseBlock feature buffer (SURVEY.md section 8 row f3)
 # ------------------------------------------------------------------------------------------------
-def _alias(buf, c0, c1):
-    """Tensor over channels [c0, c1) of the (B, C, H, W) buffer that shares its storage but NOT its autograd identity / version
-    counter: later layers write channels >= c1 of the same storage, which must not invalidate what earlier layers saved."""
-    B, C, H, W = buf.shape
-    return torch.empty(0, dtype=buf.dtype, device=buf.device).set_(
-        buf.untyped_storage(), buf.storage_offset() + c0 * H * W, (B, c1 - c0, H, W), (C * H * W, H * W, W, 1))
-
-
 class _Adopt(torch.autograd.Function):
     """init_features -> the first channels of the block's buffer (copied unless they were produced there)."""
 
@@ -115,10 +107,11 @@ class _Append(torch.autograd.Function):
         return g[:, :ctx.c], g[:, ctx.c:], None
 
 
-def _nchw_slice_ok(t):
-    B, C, H, W = t.shape
-    return (t.stride(3) == 1 and t.stride(2) == W and t.stride(1) == H * W and t.stride(0) % 4 == 0
-            and t.data_ptr() % (4 * t.element_size()) == 0)
+def _to_nhwc(g):
+    """The gradient of a channel slice of an NCHW buffer as a dense channels-last tensor (for a convolution's backward)."""
+    if g.is_cuda and _strided_ok(g, aligned=True):
+        return slice_layout(g, torch.empty(g.shape, device=g.device, dtype=g.dtype, memory_format=torch.channels_last), to_nchw=False)
+    return g.contiguous(memory_format=torch.channels_last)
 
 
 class _AppendCL(torch.autograd.Function):
@@ -134,15 +127,7 @@ class _AppendCL(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
-        c = ctx.c
-        gs = g[:, c:]
-        B, k, H, W = gs.shape
-        if _nchw_slice_ok(gs) and gs.is_cuda:
-            gn = torch.empty((B, k, H, W), device=g.device, dtype=g.dtype, memory_format=torch.channels_last)
-            slice_layout(gs, gn, to_nchw=False)
-        else:
-            gn = gs.contiguous(memory_format=torch.channels_last)
-        return g[:, :c], gn, None
+        return g[:, :ctx.c], _to_nhwc(g[:, ctx.c:]), None
 
 
 class _ToBuffer(torch.autograd.Function):
@@ -160,13 +145,15 @@ class _ToBuffer(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g, _gbuf):
-        B, C, H, W = g.shape
-        if _nchw_slice_ok(g) and g.is_cuda:
-            gn = torch.empty((B, C, H, W), device=g.device, dtype=g.dtype, memory_format=torch.channels_last)
-            slice_layout(g, gn, to_nchw=False)
-        else:
-            gn = g.contiguous(memory_format=torch.channels_last)
-        return gn, None
+        return _to_nhwc(g), None
+
+
+def _append(feats, new, buf, slice_ok):
+    """[feats | new] in buf: a channels-last `new` is transposed into its slice when ``slice_ok`` (see BufferedDenseBlock.forward),
+    anything else is copied."""
+    if slice_ok and _is_cl(new):
+        return _AppendCL.apply(feats, new, buf)
+    return _Append.apply(feats, new.contiguous(), buf)
 
 
 class BNTransition(nn.Sequential):
@@ -236,20 +223,17 @@ class BufferedDenseBlock(nn.ModuleDict):
         self.inner_channels_last = os.environ.get('AACONV_INNER_CL', '1') != '0'   # AACONV_INNER_CL=0: NCHW inside the layers (A/B, profiles/r02_b_scaling.md)
         self.fused_eval = bool(fused_eval)
 
-    def _forward_eval(self, feats, buf):
+    def _forward_eval(self, feats, buf, slice_ok):
         """Inference through the eval-mode BatchNorm + ReLU kernels (no stats buffer: the running statistics are all they read)."""
-        H, W = buf.shape[2:]
-        growth_ok = self.growth_rate % 4 == 0 and (H * W) % 4 == 0
         for layer in self.values():
             norm1, norm2 = layer.norm1, layer.norm2
-            if self.inner_channels_last and growth_ok and eval_cl_ok(norm1, feats):
+            if self.inner_channels_last and slice_ok and eval_cl_ok(norm1, feats):
                 z = layer.conv1(bn_relu_eval(norm1, feats, out_cl=True))
                 y2 = bn_relu_eval(norm2, z, out_cl=True) if eval_cl_ok(norm2, z) else bn_relu_eval(norm2, z)
                 new = layer.conv2(y2).to(buf.dtype)
             else:
                 new = layer.conv2(bn_relu_eval(norm2, layer.conv1(bn_relu_eval(norm1, feats)))).to(buf.dtype)
-            feats = (_AppendCL.apply(feats, new, buf) if _is_cl(new) and growth_ok and _nchw_slice_ok(feats)
-                     else _Append.apply(feats, new.contiguous(), buf))
+            feats = _append(feats, new, buf, slice_ok)
         return feats
 
     def forward(self, init_features):
@@ -259,19 +243,21 @@ class BufferedDenseBlock(nn.ModuleDict):
                 or not buf.is_contiguous() or buf.data_ptr() != init_features.data_ptr()):
             buf = torch.empty(B, self.out_channels, H, W, dtype=init_features.dtype, device=init_features.device)
         feats = _Adopt.apply(init_features, buf)
+        # every layer's features are a channel prefix of buf (the same strides and start): whether aaconv_slice_layout can write the
+        # growth channels of channels-last layers into the buffer holds for the whole block
+        slice_ok = buf.is_cuda and self.growth_rate % 4 == 0 and (H * W) % 4 == 0 and _strided_ok(feats, aligned=True)
         if self.fused_eval and all(eval_ok(layer.norm1, feats) and eval_ok(layer.norm2, feats) for layer in self.values()):
-            return self._forward_eval(feats, buf)
+            return self._forward_eval(feats, buf, slice_ok)
         # per-(channel, sample) plane statistics of the buffer, shared by the norm1 of every layer: layer i only reduces the channels
         # layer i-1 has not seen (its own 32 new ones); the first layer reduces the block's input channels
         stats = torch.empty(2 * B * self.out_channels, device=buf.device, dtype=torch.float32) if buf.is_cuda else None
         valid = 0
-        growth_ok = self.growth_rate % 4 == 0 and (H * W) % 4 == 0 and stats is not None
         shared = stats is not None          # every norm1 reduced its new channels into `stats` (the fused kernels ran)
         for layer in self.values():
             # norm -> relu pairs: fused strided kernels in training on CUDA (chexpert_b200.fused_bn), the torch modules otherwise
             c = feats.shape[1]
-            if (self.inner_channels_last and layer.drop_rate == 0 and torch.is_grad_enabled() and feats.requires_grad
-                    and cl_ok(layer.norm1, feats) and _nchw_slice_ok(feats) and growth_ok):
+            if (self.inner_channels_last and slice_ok and layer.drop_rate == 0 and torch.is_grad_enabled() and feats.requires_grad
+                    and cl_ok(layer.norm1, feats)):
                 # The two convolutions of the layer run channels-last (cuDNN's tensor-core kernels are NHWC; with NCHW tensors it
                 # transposes every operand of every fprop / dgrad / wgrad itself: 21 % of the step in the round-2 profile).  The
                 # layout change rides on the BatchNorm + ReLU passes (csrc/bn_cl.cu); the buffer itself stays NCHW.
@@ -282,8 +268,7 @@ class BufferedDenseBlock(nn.ModuleDict):
                 else:
                     new = layer.conv2(bn_relu(layer.norm2, z.contiguous()))
                 valid = c
-                new = new.to(buf.dtype)
-                feats = (_AppendCL.apply(feats, new, buf) if _is_cl(new) else _Append.apply(feats, new.contiguous(), buf))
+                feats = _append(feats, new.to(buf.dtype), buf, slice_ok)
                 continue
             # norm1 taps the concatenated features: backward adds its dx into the gradient of the concatenation in place
             shared = shared and _fused_ok(layer.norm1, feats)
@@ -406,3 +391,25 @@ def densenet121(num_classes=5, feature_buffer=False, fused_transition=False, fus
     ``fused_transition`` (with ``feature_buffer``): the Transitions run as BNTransition.  None of them adds parameters."""
     return DenseNet(32, (6, 12, 24, 16), 64, num_classes=num_classes, attn_params=None, feature_buffer=feature_buffer,
                     fused_eval=fused_eval, fused_transition=fused_transition)
+
+
+def build_model(arch, num_classes=5, size=320, precision=None, feature_buffer=False, fused=False, fused_eval=False):
+    """aadensenet121 or the reference's baseline densenet121 by name.  ``fused``: aadensenet121's fused_prologue / densenet121's
+    fused_transition (fused BatchNorm + ReLU + pool Transitions); ``size`` and ``precision`` only concern aadensenet121's AAConv2d."""
+    if arch == 'aadensenet121':
+        return aadensenet121(num_classes, (size, size), precision=precision, feature_buffer=feature_buffer, fused_prologue=fused,
+                             fused_eval=fused_eval)
+    if arch == 'densenet121':
+        return densenet121(num_classes, feature_buffer=feature_buffer, fused_transition=fused, fused_eval=fused_eval)
+    raise ValueError(f"arch must be 'aadensenet121' or 'densenet121', got {arch!r}")
+
+
+def conv_weight_plan(model):
+    """[(name, conv, channels_last)] for the nn.Conv2d modules of `model` that cuDNN runs: all but the parameter holders of the
+    AAConv2d modules, whose fp32 weights the library's kernels read.  channels_last: a k x k convolution of a BufferedDenseBlock whose
+    layers run channels-last (inner_channels_last) sees NHWC activations, so its weight is kept channels-last too, or cuDNN would
+    transpose it on every call.  1 x 1 weights are the same bytes in both formats; the stem's convolution stays NCHW."""
+    own = {id(p) for m in model.modules() if isinstance(m, AAConv2d) for p in m.parameters()}
+    cl = {id(m) for b in model.modules() if isinstance(b, BufferedDenseBlock) and b.inner_channels_last for m in b.modules()}
+    return [(name, m, id(m) in cl and m.weight.shape[2] * m.weight.shape[3] > 1) for name, m in model.named_modules()
+            if isinstance(m, nn.Conv2d) and id(m.weight) not in own]

@@ -18,7 +18,7 @@ import torch.nn.functional as F
 
 from . import _lib
 from .aaconv import AAConv2d, _ptr, _stream
-from .densenet import aadensenet121, densenet121
+from .densenet import build_model, conv_weight_plan
 from .loss import BCEWithLogitsLoss
 
 PIXEL_MEAN, PIXEL_STD = 0.5330, 0.0349        # chexpert.py:70-72
@@ -138,21 +138,11 @@ class Predictor:
             raise RuntimeError('chexpert_b200.evaluate.Predictor runs on CUDA only; there is no CPU fallback')
         self.num_classes, self.size, self.batch_size = num_classes, size, int(batch_size)
         self.autocast = bool(autocast)
-        if arch == 'aadensenet121':
-            model = aadensenet121(num_classes, (size, size), precision=precision, feature_buffer=True, fused_prologue=True, fused_eval=True)
-        elif arch == 'densenet121':
-            model = densenet121(num_classes, feature_buffer=True, fused_transition=True, fused_eval=True)
-        else:
-            raise ValueError(f"Predictor: arch must be 'aadensenet121' or 'densenet121', got {arch!r}")
+        model = build_model(arch, num_classes, size, precision, feature_buffer=True, fused=True, fused_eval=True)
         model.requires_grad_(False)
-        # the dense layers' convolutions see NHWC activations, so their k x k weights are kept channels-last (in fp32 too: cuDNN would
-        # otherwise transpose an NCHW weight on every call); 1 x 1 weights are the same bytes in both formats
-        own = {id(p) for m in model.modules() if isinstance(m, AAConv2d) for p in m.parameters()}
-        for name, m in model.named_modules():
-            if isinstance(m, torch.nn.Conv2d) and id(m.weight) not in own:
-                cl = 'denseblock' in name and m.weight.shape[2] * m.weight.shape[3] > 1
-                m.weight.data = m.weight.data.to(torch.bfloat16 if self.autocast else torch.float32,
-                                                 memory_format=torch.channels_last if cl else torch.contiguous_format)
+        for _, m, cl in conv_weight_plan(model):
+            m.weight.data = m.weight.data.to(torch.bfloat16 if self.autocast else torch.float32,
+                                             memory_format=torch.channels_last if cl else torch.contiguous_format)
         self.model = model.to(self.device).eval()
         self.cuda_graph = bool(cuda_graph)
         self._warm = 0

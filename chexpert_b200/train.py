@@ -15,7 +15,7 @@ import torch.distributed as dist
 
 from . import _lib
 from .dataparallel import GradientBuckets
-from .densenet import aadensenet121, densenet121
+from .densenet import build_model, conv_weight_plan
 from .loss import BCEWithLogitsLoss
 
 # dataset normalisation constants of the reference transform (chexpert.py:70-72)
@@ -45,15 +45,8 @@ class TrainStep:
                  batched_casts=True, arch='aadensenet121'):
         torch.manual_seed(seed)
         self.device = torch.device(device)
-        # arch: 'aadensenet121' or the reference's baseline 'densenet121' (torchvision's network; `precision` only concerns AAConv2d,
-        # and `fused_prologue` selects its fused BatchNorm + ReLU + pool Transitions).  The optimizer is the same for both.
-        if arch == 'aadensenet121':
-            model = aadensenet121(5, (size, size), precision=precision, feature_buffer=buffered, fused_prologue=fused_prologue)
-        elif arch == 'densenet121':
-            model = densenet121(5, feature_buffer=buffered, fused_transition=fused_prologue)
-        else:
-            raise ValueError(f"TrainStep: arch must be 'aadensenet121' or 'densenet121', got {arch!r}")
-        self.model = model.to(self.device)
+        # arch (densenet.build_model): 'aadensenet121' or the reference's baseline 'densenet121'; the optimizer is the same for both
+        self.model = build_model(arch, 5, size, precision, feature_buffer=buffered, fused=fused_prologue).to(self.device)
         if channels_last:
             self.model = self.model.to(memory_format=torch.channels_last)
         self.loss_fn = BCEWithLogitsLoss('train', raw_labels=raw_labels).to(self.device)
@@ -81,7 +74,7 @@ class TrainStep:
                     self._nbt.append(m.num_batches_tracked)
         self._sh = None
         if batched_casts and self.autocast:
-            self._setup_shadows(buffered_cl=bool(buffered))
+            self._setup_shadows()
         # Gradient exchange.  On CUDA: fresh gradients, packed (one multi-tensor copy per ~25 MB bucket) and all-reduced (NCCL, averaged)
         # AFTER backward.  Measured on 2 and 8 B200s under the CUDA graph: communication under backward is slower here --
         # AACONV_DP_OVERLAP=1 (one hook per bucket, GradientBuckets(overlap='bucket')) 2504 images/s vs 2777 at 2 GPUs, the
@@ -105,26 +98,17 @@ class TrainStep:
         self.graph_launches = 0
         self.model.train()
 
-    def _setup_shadows(self, buffered_cl=True):
-        from .aaconv import AAConv2d
-        own = {id(p) for m in self.model.modules() if isinstance(m, AAConv2d) for p in m.parameters()}   # fp32 into our kernels
-        names, params = [], []
-        for n, m in self.model.named_modules():
-            if isinstance(m, torch.nn.Conv2d) and id(m.weight) not in own:
-                names.append(n + '.weight')
-                params.append(m.weight)
-        self._sh_names, self._sh_params = names, params
-        # The convolutions inside the dense blocks see NHWC activations (csrc/bn_cl.cu), so their k x k weights live channels-last too --
-        # the fp32 MASTER weights themselves (values, state_dict and optimizer are layout-agnostic): with a contiguous master and a
-        # channels-last shadow torch._foreach_copy_ fell back to one strided copy kernel per tensor (1.1 ms per step in the profile).
-        # 1 x 1 weights are the same bytes in both formats and stay as they are; the stem keeps NCHW weights (its output must stay NCHW
-        # for the fused strided BN + ReLU).
-        if buffered_cl and os.environ.get('AACONV_INNER_CL', '1') != '0':
-            for n, p in zip(names, params):
-                if 'denseblock' in n and p.shape[2] * p.shape[3] > 1:
-                    p.data = p.data.contiguous(memory_format=torch.channels_last)
-        self._sh = [torch.empty_like(p, dtype=torch.bfloat16).requires_grad_(True) for p in params]     # preserve_format: strides of p
-        self._sh_grads = [torch.empty_like(p) for p in params]          # fp32, static: what the optimizer / buckets read
+    def _setup_shadows(self):
+        plan = conv_weight_plan(self.model)
+        self._sh_names, self._sh_params = [n + '.weight' for n, _, _ in plan], [m.weight for _, m, _ in plan]
+        # The weights the plan keeps channels-last are the fp32 MASTER weights themselves (values, state_dict and optimizer are
+        # layout-agnostic): with a contiguous master and a channels-last shadow torch._foreach_copy_ fell back to one strided copy
+        # kernel per tensor (1.1 ms per step in the profile).
+        for _, m, cl in plan:
+            if cl:
+                m.weight.data = m.weight.data.contiguous(memory_format=torch.channels_last)
+        self._sh = [torch.empty_like(p, dtype=torch.bfloat16).requires_grad_(True) for p in self._sh_params]   # preserve_format: strides of p
+        self._sh_grads = [torch.empty_like(p) for p in self._sh_params]          # fp32, static: what the optimizer / buckets read
 
     def _step(self, x, target):
         if self.buckets is not None:

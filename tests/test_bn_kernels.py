@@ -526,6 +526,34 @@ def test_bn_relu_cl_rejects_more_than_4096_channels(C):
         fused_bn.bn_relu_cl(bn, x)
 
 
+@pytest.mark.gpu
+@pytest.mark.parametrize('which', ['module', 'running_stats', 'weight_bias'])
+def test_route_predicates_refuse_a_batchnorm_that_is_not_fp32(which):
+    """The kernels read weight and bias and read or update the running statistics through float pointers, so every route predicate
+    refuses a BatchNorm2d with bf16 parameters or running statistics (e.g. after model.to(torch.bfloat16)): such a module takes the
+    module path.  Only the predicates run here; no kernel is launched."""
+    B, C, H, W = 4, 64, 8, 8
+    x = torch.empty(B, C, H, W, device='cuda', dtype=torch.bfloat16)
+    xl = torch.empty(B, C, H, W, device='cuda', dtype=torch.bfloat16, memory_format=CL)
+
+    def routes(bn):
+        bn.train()
+        ok = [fused_bn._fused_ok(bn, x), fused_bn.cl_ok(bn, x), fused_bn.cl_ok(bn, xl), fused_bn.pool_ok(bn, x)]
+        bn.eval()
+        with torch.no_grad():
+            ok += [fused_bn.eval_ok(bn, x), fused_bn.eval_cl_ok(bn, x), fused_bn.eval_cl_ok(bn, xl), fused_bn.pool_ok(bn, x)]
+        return ok
+    assert all(routes(torch.nn.BatchNorm2d(C).cuda()))                  # fp32: every route takes it
+    bn = torch.nn.BatchNorm2d(C)
+    if which == 'module':
+        bn.to(torch.bfloat16)
+    elif which == 'running_stats':
+        bn.running_mean, bn.running_var = bn.running_mean.bfloat16(), bn.running_var.bfloat16()
+    else:
+        bn.weight.data, bn.bias.data = bn.weight.data.bfloat16(), bn.bias.data.bfloat16()
+    assert not any(routes(bn.cuda())), routes(bn)
+
+
 @pytest.fixture
 def no_tf32():
     old = torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32
