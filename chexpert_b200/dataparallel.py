@@ -1,17 +1,17 @@
-"""Data-parallel training plumbing: one process per GPU, batch sharded across ranks, gradients exchanged as flat
-buckets with an NCCL all-reduce that overlaps the rest of backward.
+"""Data-parallel training plumbing: one process per GPU, batch sharded across ranks, gradients averaged over the ranks after
+backward as flat buckets, one all-reduce per bucket.
 
 The reference is single-process / single-device (chexpert.py:38,453); this is the one new subsystem SURVEY.md
 section 8(e) asks for.  The batch dimension is the only shard: every AAConv2d kernel runs unsharded on its rank.
 
 Design (deliberately small, no torch DDP wrapper):
   * parameters are laid out, in REVERSE registration order (the order backward produces gradients), into flat
-    fp32 buckets of ~``bucket_mb``; ``p.grad`` of every parameter is a view into its bucket, so autograd accumulates
-    straight into the communication buffer and no gather/scatter copies exist;
-  * a post-accumulate hook per parameter counts the bucket down; the last one issues ``all_reduce(async_op=True)``,
-    which NCCL runs on its own stream over NVLink 5 / NVSwitch while backward continues on the compute stream;
-  * ``finish()`` waits for the outstanding work and scales by 1/world (mean over the global batch, the reference's
-    ``.mean(0)``, chexpert.py:160).
+    fp32 buckets of ~``bucket_mb``;
+  * autograd writes fresh gradients; ``finish()`` packs each bucket with one multi-tensor copy, all-reduces it as a mean
+    over the global batch (the reference's ``.mean(0)``, chexpert.py:160) and points every ``p.grad`` at its slice of the
+    bucket.  There is no per-parameter accumulate kernel (360 small launches per step for aadensenet121, ~1 ms under a CUDA
+    graph); the price is an all-reduce that is not hidden under backward (~0.2 ms for 50 MB over NVLink 5 at 8 GPUs);
+  * every rank issues the all-reduces in the same bucket order, whichever parameters received a gradient on it.
 Works with the gloo backend on CPU, which is how tests/ covers world_size 2 without GPUs.
 """
 import torch
@@ -19,22 +19,13 @@ import torch.distributed as dist
 
 
 class GradientBuckets:
-    """``overlap=True``: gradients accumulate straight into the buckets and every bucket is all-reduced from the backward hooks as
-    soon as it is complete (communication under the rest of backward).  ``overlap=False``: autograd writes fresh gradients,
-    ``finish()`` packs them into the buckets with one multi-tensor copy per bucket, all-reduces (average) and points ``p.grad`` at
-    the bucket views -- no per-parameter accumulate kernel (360 small launches per step for aadensenet121, ~1 ms under a CUDA
-    graph) at the price of a 50 MB all-reduce that is not hidden (~0.2 ms over NVLink 5 at 8 GPUs)."""
+    """Averages the gradients of ``module``'s trainable parameters over the ranks of ``process_group``.
 
-    def __init__(self, module, bucket_mb=25.0, process_group=None, broadcast_from=0, overlap=True, grad_sources=None):
-        """``overlap='bucket'``: fresh gradients as with ``overlap=False``, but every bucket is packed (one multi-tensor copy) and
-        all-reduced from ONE hook that fires when the last gradient of the bucket has been computed
-        (``torch.autograd.graph.register_multi_grad_hook``): communication under the rest of backward without the per-parameter
-        accumulate kernels.  ``grad_sources`` maps a parameter to the tensor whose gradient stands in for it (TrainStep's bf16
-        weight shadows): the pack converts to the fp32 bucket on the way."""
+    One step is ``reset()``, one or more ``backward()`` calls, ``finish()``, then the optimizer step.  Gradients of several
+    ``backward()`` calls in one step add up in ``.grad`` as usual, and ``finish()`` exchanges their sum once."""
+
+    def __init__(self, module, bucket_mb=25.0, process_group=None, broadcast_from=0):
         self.group = process_group
-        self.bucket_hooks = overlap == 'bucket'
-        self.overlap = bool(overlap) and not self.bucket_hooks
-        self._src = dict(grad_sources or {})
         self.world = dist.get_world_size(process_group) if dist.is_initialized() else 1
         self.params = [p for p in module.parameters() if p.requires_grad]
         if not self.params:
@@ -44,7 +35,6 @@ class GradientBuckets:
                 dist.broadcast(t.data, broadcast_from, group=process_group)
         cap = max(1, int(bucket_mb * (1 << 20) / 4))
         self.buckets = []          # (flat tensor, [params])
-        self._bucket_of = {}
         self._view = {}
         cur, cur_n = [], 0
         for p in reversed(self.params):
@@ -55,18 +45,6 @@ class GradientBuckets:
             cur_n += p.numel()
         if cur:
             self._seal(cur)
-        self._pending = [0] * len(self.buckets)
-        self._works = []
-        self._next = 0            # buckets [0, _next) have had their all-reduce issued this step
-        self._state = 'finished'  # 'armed' between reset() and finish()
-        self._sync = True
-        self._hooks = [p.register_post_accumulate_grad_hook(self._on_grad) for p in self.params] if self.overlap else []
-        self._ready = [False] * len(self.buckets)
-        if self.bucket_hooks:
-            import functools
-            for bi, (_, params) in enumerate(self.buckets):
-                srcs = tuple(self._src.get(p, p) for p in params)
-                self._hooks.append(torch.autograd.graph.register_multi_grad_hook(srcs, functools.partial(self._on_bucket, bi), mode='all'))
         self.reset()
 
     def _seal(self, params):
@@ -79,159 +57,40 @@ class GradientBuckets:
             # the view has the parameter's own (dense) strides -- channels-last conv weights included -- so that packing its
             # gradient is part of one multi-tensor copy instead of a strided copy of its own
             seg = flat[off:off + p.numel()]
-            self._view[p] = p.grad = seg.view_as(p) if p.is_contiguous() else seg.as_strided(p.shape, p.stride())
+            self._view[p] = seg.view_as(p) if p.is_contiguous() else seg.as_strided(p.shape, p.stride())
             off += p.numel()
-            self._bucket_of[p] = len(self.buckets)
         self.buckets.append((flat, params))
 
     def reset(self):
-        """Zero the buckets (replaces optimizer.zero_grad(); keeps the grad views alive) and arm the step."""
-        if not self.overlap:                      # fresh gradients from autograd: nothing to zero, nothing to accumulate into
-            for p in self.params:
-                p.grad = None
-            self._ready = [False] * len(self.buckets)
-            self._works = []
-            self._next = 0
-            self._state = 'armed'
-            return
-        for flat, _ in self.buckets:
-            flat.zero_()
-        self._pending = [len(ps) for _, ps in self.buckets]
-        self._works = []
-        self._next = 0
-        self._state = 'armed'
-
-    def no_sync(self):
-        """Context manager for gradient accumulation: backward passes inside it only accumulate locally into the buckets;
-        the exchange happens in the first backward outside it (then finish()).  reset() once per accumulation window."""
-        return _NoSync(self)
-
-    def _issue_ready(self, upto=None):
-        # collectives are ALWAYS issued in bucket order 0, 1, 2, ... on every rank, whatever order the hooks fired in (a rank on
-        # which some parameter got no gradient must not reorder its all-reduces relative to the other ranks)
-        n = len(self.buckets) if upto is None else upto
-        while self._next < n and (upto is not None or self._pending[self._next] == 0):
-            if self.world > 1:
-                self._works.append(dist.all_reduce(self.buckets[self._next][0], group=self.group, async_op=True))
-            self._next += 1
-
-    def _avg_op(self):
-        return dist.ReduceOp.AVG if (self.world > 1 and dist.get_backend(self.group) == 'nccl') else None
-
-    def _pack(self, bi, grads):
-        """gradients of bucket bi (None = parameter without a gradient on this rank: zeros) -> its flat fp32 buffer"""
-        flat, params = self.buckets[bi]
-        views = [self._view[p] for p in params]
-        have = [(v, g) for v, g in zip(views, grads) if g is not None and g.data_ptr() != v.data_ptr()]
-        for v, g in zip(views, grads):
-            if g is None:
-                v.zero_()
-        if have:
-            torch._foreach_copy_([v for v, _ in have], [g for _, g in have])
-
-    def _issue_packed(self):
-        """all-reduce the packed buckets in bucket order 0, 1, 2, ... (identical on every rank)"""
-        avg = self._avg_op()
-        while self._next < len(self.buckets) and self._ready[self._next]:
-            flat = self.buckets[self._next][0]
-            if self.world > 1:
-                self._works.append(dist.all_reduce(flat, op=avg, group=self.group, async_op=True) if avg is not None
-                                   else dist.all_reduce(flat, group=self.group, async_op=True))
-            self._next += 1
-
-    def _on_bucket(self, bi, grads):
-        if not self._sync or self._state != 'armed' or self._ready[bi]:
-            return                                # accumulation window / stray backward: finish() packs from .grad
-        with torch.no_grad():
-            self._pack(bi, grads)
-        self._ready[bi] = True
-        self._issue_packed()
-
-    def _on_grad(self, p):
-        b = self._bucket_of[p]
-        view = self._view[p]
-        if p.grad.data_ptr() != view.data_ptr():     # someone replaced .grad (e.g. set_to_none): copy back in
-            view.copy_(p.grad)
-            p.grad = view
-        if not self._sync:
-            return
-        if self._state != 'armed':
-            raise RuntimeError('GradientBuckets: backward() after finish() without reset() -- the buckets hold reduced gradients; '
-                               'call reset() at the start of every step (use no_sync() for gradient accumulation)')
-        self._pending[b] -= 1
-        if self._pending[b] < 0:
-            raise RuntimeError('GradientBuckets: a parameter received a second gradient before finish(): its bucket has already '
-                               'been exchanged.  Wrap all but the last backward() of an accumulation window in no_sync().')
-        self._issue_ready()
+        """Drop the gradients (replaces optimizer.zero_grad(set_to_none=True)) and arm the step."""
+        for p in self.params:
+            p.grad = None
+        self._armed = True
 
     def finish(self):
-        """Wait for the exchange and turn sums into means.  Call once after backward(), before optimizer.step()."""
-        if self._state != 'armed':
-            raise RuntimeError('GradientBuckets: finish() called twice (or before reset())')
-        if self.bucket_hooks:
-            with torch.no_grad():
-                for bi, (flat, params) in enumerate(self.buckets):      # buckets whose hook did not fire (no gradient at all, no_sync)
-                    if not self._ready[bi]:
-                        self._pack(bi, [self._src.get(p, p).grad for p in params])
-                        self._ready[bi] = True
-                self._issue_packed()
-                for w in self._works:
-                    w.wait()
-                if self.world > 1 and self._avg_op() is None:
-                    for flat, _ in self.buckets:
-                        flat.div_(self.world)
-                for flat, params in self.buckets:
-                    for p in params:
-                        p.grad = self._view[p]
-            self._works = []
-            self._state = 'finished'
-            return
-        if not self.overlap:
-            avg = dist.ReduceOp.AVG if (self.world > 1 and dist.get_backend(self.group) == 'nccl') else None
-            for flat, params in self.buckets:
-                views = [self._view[p] for p in params]
-                have = [(v, p.grad) for v, p in zip(views, params) if p.grad is not None and p.grad.data_ptr() != v.data_ptr()]
-                for v, p in zip(views, params):
-                    if p.grad is None:
-                        v.zero_()                 # parameter without a gradient on this rank contributes zeros
-                if have:
-                    torch._foreach_copy_([v for v, _ in have], [g for _, g in have])
-                if self.world > 1:
-                    if avg is not None:
-                        dist.all_reduce(flat, op=avg, group=self.group)
-                    else:
-                        dist.all_reduce(flat, group=self.group)
-                        flat.div_(self.world)
-                for v, p in zip(views, params):
-                    p.grad = v
-            self._state = 'finished'
-            return
-        self._issue_ready(upto=len(self.buckets))     # buckets with parameters that received no gradient this step, in order
-        if self.world > 1:
-            for w in self._works:
-                w.wait()
-            for flat, _ in self.buckets:
-                flat.div_(self.world)
-        self._works = []
-        self._state = 'finished'
+        """Average the gradients over the ranks.  Call once after backward(), before optimizer.step()."""
+        if not self._armed:
+            raise RuntimeError('GradientBuckets: finish() called twice, or without reset() since the last finish() -- the '
+                               'gradients are already averaged; call reset() at the start of every step')
+        avg = dist.ReduceOp.AVG if (self.world > 1 and dist.get_backend(self.group) == 'nccl') else None
+        for flat, params in self.buckets:
+            views = [self._view[p] for p in params]
+            have = [(v, p.grad) for v, p in zip(views, params) if p.grad is not None]
+            for v, p in zip(views, params):
+                if p.grad is None:
+                    v.zero_()                 # parameter without a gradient on this rank contributes zeros
+            if have:
+                torch._foreach_copy_([v for v, _ in have], [g for _, g in have])
+            if self.world > 1:
+                if avg is not None:
+                    dist.all_reduce(flat, op=avg, group=self.group)
+                else:
+                    dist.all_reduce(flat, group=self.group)
+                    flat.div_(self.world)
+            for v, p in zip(views, params):
+                p.grad = v
+        self._armed = False
 
     @property
     def nbytes(self):
         return sum(f.numel() * 4 for f, _ in self.buckets)
-
-    def remove(self):
-        for h in self._hooks:
-            h.remove()
-
-
-class _NoSync:
-    def __init__(self, gb):
-        self.gb = gb
-
-    def __enter__(self):
-        self.gb._sync = False
-        return self.gb
-
-    def __exit__(self, *exc):
-        self.gb._sync = True
-        return False

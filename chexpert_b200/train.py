@@ -7,9 +7,6 @@ radiograph-shaped batches (SURVEY.md section 8d, configs 1/3/4).
 The loop around it (tqdm, tensorboard, checkpoint tracker, periodic eval; chexpert.py:167-193) is outside the hot
 path and not rebuilt; `TrainStep` is what bench.py times and what a user's own loop would call per batch.
 """
-import contextlib
-import os
-
 import torch
 import torch.distributed as dist
 
@@ -75,21 +72,10 @@ class TrainStep:
         self._sh = None
         if batched_casts and self.autocast:
             self._setup_shadows()
-        # Gradient exchange.  On CUDA: fresh gradients, packed (one multi-tensor copy per ~25 MB bucket) and all-reduced (NCCL, averaged)
-        # AFTER backward.  Measured on 2 and 8 B200s under the CUDA graph: communication under backward is slower here --
-        # AACONV_DP_OVERLAP=1 (one hook per bucket, GradientBuckets(overlap='bucket')) 2504 images/s vs 2777 at 2 GPUs, the
-        # per-parameter hook variant (overlap=True: 360 small accumulate kernels per step) 7.03x vs 7.62x at 8 GPUs in the first
-        # session: the ~0.5 ms all-reduce costs the concurrent convolutions more than it hides.
-        mode = True if self.device.type != 'cuda' else ('bucket' if os.environ.get('AACONV_DP_OVERLAP', '0') == '1' else False)
-        srcs = dict(zip(self._sh_params, self._sh)) if self._sh is not None else None
-        # The bucket hooks create the AccumulateGrad nodes of their tensors at registration, and such a node keeps the stream it was
-        # created under: registered under the default stream they would make it wait on the capturing stream during the graph capture
-        # (cudaErrorStreamCaptureImplicit).  So with bucket hooks EVERY step -- eager, capture, replay -- runs on one side stream.
-        self._stream = torch.cuda.Stream(self.device) if (self.world > 1 and mode == 'bucket') else None
-        with torch.cuda.stream(self._stream) if self._stream is not None else contextlib.nullcontext():
-            self.buckets = (GradientBuckets(self.model, bucket_mb=bucket_mb, overlap=mode, grad_sources=srcs if mode == 'bucket' else None)
-                            if self.world > 1 else None)
-        self._bucket_sources = self.buckets is not None and mode == 'bucket' and self._sh is not None
+        # Gradient exchange (world > 1): packed and all-reduced after backward, inside the CUDA graph.  Exchanging under backward
+        # measured slower on B200s under the CUDA graph (one hook per bucket: 2504 vs 2777 images/s at 2 GPUs; one hook per
+        # parameter: 7.03x vs 7.62x at 8 GPUs): the ~0.5 ms all-reduce costs the concurrent convolutions more than it hides.
+        self.buckets = GradientBuckets(self.model, bucket_mb=bucket_mb) if self.world > 1 else None
         self.cuda_graph = bool(cuda_graph and self.device.type == 'cuda')
         self.graph_after = graph_after
         self._calls = 0
@@ -128,7 +114,7 @@ class TrainStep:
                 out = self.model(x)
         loss = self.loss_fn(out.float(), target)
         loss.backward()
-        if self._sh is not None and not self._bucket_sources:      # (bucket hooks pack the shadows' gradients themselves)
+        if self._sh is not None:
             with torch.no_grad():
                 torch._foreach_copy_(self._sh_grads, [t.grad for t in self._sh])
             for p, g in zip(self._sh_params, self._sh_grads):
@@ -146,7 +132,7 @@ class TrainStep:
             self.opt.zero_grad(set_to_none=True)
         n0 = _lib.launch_count()
         mode = 'thread_local' if self.world > 1 else 'global'   # NCCL's watchdog thread polls events during the capture
-        with torch.cuda.graph(self._graph, stream=self._stream, capture_error_mode=mode):
+        with torch.cuda.graph(self._graph, capture_error_mode=mode):
             self._sloss = self._step(self._sx, self._st)
         self.graph_launches = _lib.launch_count() - n0      # kernels of libaaconv_b200 inside one replay
         self._graph_lr = [g['lr'] for g in self.opt.param_groups]
@@ -160,16 +146,6 @@ class TrainStep:
 
     def __call__(self, x, target):
         """-> loss (0-dim device tensor; no host sync, unlike loss.item() at chexpert.py:167)."""
-        if self._stream is None:
-            return self._call(x, target)
-        cur = torch.cuda.current_stream(self.device)
-        self._stream.wait_stream(cur)
-        with torch.cuda.stream(self._stream):
-            loss = self._call(x, target)
-        cur.wait_stream(self._stream)
-        return loss
-
-    def _call(self, x, target):
         self._calls += 1
         if not self.cuda_graph or self._calls <= self.graph_after:
             loss = self._step(x, target)
