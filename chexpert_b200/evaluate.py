@@ -20,6 +20,7 @@ from . import _lib
 from .aaconv import AAConv2d, _ptr, _stream
 from .densenet import build_model, conv_weight_plan
 from .loss import BCEWithLogitsLoss
+from .preprocess import Radiographs, pack_radiographs, prepare
 
 PIXEL_MEAN, PIXEL_STD = 0.5330, 0.0349        # chexpert.py:70-72
 
@@ -124,7 +125,9 @@ class Predictor:
     ``cuda_graph``: after WARMUP eager batches (cuDNN picks its algorithms) one graph of the whole step at ``batch_size`` is
     captured and replayed.  A ragged last batch is padded to ``batch_size`` (samples are independent in eval mode) and sliced.
     load_state_dict writes parameters and buffers in place, so one capture serves every checkpoint of an ensemble;
-    ``captures`` counts the captures made.
+    ``captures`` counts the captures made.  Raw radiographs (any sizes, see __call__) have a graph of their own, captured the same
+    way from a static prepared (batch_size, 3, S, S) input onward; the prep launch runs before each replay, so batches of any
+    geometries replay it.
 
     ``arch='densenet121'``: the reference's baseline, torchvision's densenet121, as densenet121(feature_buffer=True,
     fused_transition=True, fused_eval=True) -- its Transitions' BatchNorm + ReLU + pool run through the eval-mode pooled kernel."""
@@ -145,8 +148,9 @@ class Predictor:
                                              memory_format=torch.channels_last if cl else torch.contiguous_format)
         self.model = model.to(self.device).eval()
         self.cuda_graph = bool(cuda_graph)
-        self._warm = 0
-        self._graph = self._sx = self._sy = None
+        self._warm = {'u8': 0, 'raw': 0}
+        self._graphs = {}                   # input path -> (graph, static logits)
+        self._sx = self._rx = None          # static inputs: uint8 (batch_size, S, S); prepared float (batch_size, 3, S, S)
         self.captures = 0
 
     def load_state_dict(self, state_dict):
@@ -155,15 +159,27 @@ class Predictor:
             self.model.load_state_dict(state_dict, strict=True)
 
     def _forward(self, u8):
-        with torch.autocast('cuda', dtype=torch.bfloat16, enabled=self.autocast, cache_enabled=False):
-            return self.model(normalise_u8(u8)).float()
+        return self._model_forward(normalise_u8(u8))
 
-    def _capture(self):
-        torch.cuda.synchronize(self.device)
-        self._graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self._graph):
-            self._sy = self._forward(self._sx)
-        self.captures += 1
+    def _model_forward(self, x):
+        with torch.autocast('cuda', dtype=torch.bfloat16, enabled=self.autocast, cache_enabled=False):
+            return self.model(x).float()
+
+    def _run(self, path, forward, sx, n):
+        """forward(sx)[:n]: eager for the first WARMUP batches of this input path, then through the path's graph, captured once."""
+        if path not in self._graphs:
+            if self._warm[path] < self.WARMUP:
+                self._warm[path] += 1
+                return forward(sx)[:n]
+            torch.cuda.synchronize(self.device)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                sy = forward(sx)
+            self._graphs[path] = (graph, sy)
+            self.captures += 1
+        graph, sy = self._graphs[path]
+        graph.replay()
+        return sy[:n]
 
     def _batch(self, chunk):
         n = chunk.shape[0]
@@ -172,25 +188,44 @@ class Predictor:
         if self._sx is None:
             self._sx = torch.zeros(self.batch_size, *chunk.shape[1:], dtype=torch.uint8, device=self.device)
         self._sx[:n].copy_(chunk, non_blocking=True)       # rows [n, batch_size) keep earlier images: padding, sliced off below
-        if self._graph is None:
-            if self._warm < self.WARMUP:
-                self._warm += 1
-                return self._forward(self._sx)[:n]
-            self._capture()
-        self._graph.replay()
-        return self._sy[:n]
+        return self._run('u8', self._forward, self._sx, n)
+
+    def _raw_batch(self, rad):
+        """Radiographs on the device -> logits: one prep launch, then the model from the prepared tensor onward."""
+        n = len(rad)
+        if not self.cuda_graph:
+            return self._model_forward(prepare(rad))
+        if self._rx is None:
+            self._rx = torch.zeros(self.batch_size, 3, self.size, self.size, dtype=torch.float32, device=self.device)
+        prepare(rad, out=self._rx[:n])                      # rows [n, batch_size): padding, as in _batch
+        return self._run('raw', self._model_forward, self._rx, n)
 
     @torch.no_grad()
-    def __call__(self, images_u8):
-        """uint8 (N, H, W) -> (N, num_classes) float32 logits on the device, batch by batch."""
-        if images_u8.dtype != torch.uint8 or images_u8.dim() != 3:
-            raise RuntimeError(f'Predictor takes uint8 (N, H, W) images, got {images_u8.dtype} {tuple(images_u8.shape)}')
+    def __call__(self, images):
+        """-> (N, num_classes) float32 logits on the device, batch by batch, from either
+        - uint8 (N, S, S) images already at the model's size, on the host or the device, normalised by normalise_u8; or
+        - raw radiographs of any sizes: a list of 2-D uint8 host images (packed and uploaded batch by batch), or a
+          preprocess.Radiographs of side S (uploaded whole if on the host).  preprocess.prepare runs the reference's
+          Resize(S) + CenterCrop(S) + normalisation on the device, one launch per batch; its CUDA graph starts after it."""
+        raw = isinstance(images, (Radiographs, list, tuple))
+        if not raw and (images.dtype != torch.uint8 or images.dim() != 3):
+            raise RuntimeError(f'Predictor takes uint8 (N, H, W) images, got {images.dtype} {tuple(images.shape)}')
+        if isinstance(images, Radiographs) and images.size != self.size:
+            raise RuntimeError(f'Radiographs packed for size {images.size}, this Predictor takes {self.size}')
         with torch.cuda.device(self.device):
-            N = images_u8.shape[0]
+            if isinstance(images, Radiographs):
+                images = images.to(self.device)
+            N = len(images)
             out = torch.empty(N, self.num_classes, device=self.device, dtype=torch.float32)
             for i in range(0, N, self.batch_size):
-                chunk = images_u8[i:i + self.batch_size]
-                out[i:i + chunk.shape[0]].copy_(self._batch(chunk))
+                chunk = images[i:i + self.batch_size]
+                if isinstance(chunk, Radiographs):
+                    y = self._raw_batch(chunk)
+                elif raw:
+                    y = self._raw_batch(pack_radiographs(chunk, self.size).to(self.device))
+                else:
+                    y = self._batch(chunk)
+                out[i:i + y.shape[0]].copy_(y)
             return out
 
 
@@ -200,9 +235,12 @@ def evaluate_ensemble(model, state_dicts, images_u8, targets, batch_size=16, dev
     `model`, its logits and element losses over the whole set are kept, the ensemble output / loss are their means over the
     checkpoints (chexpert.py:233-234; note mean-of-losses, not loss-of-mean); metrics as compute_metrics (chexpert.py:130-146)
     minus the plotting inputs.  -> dict(outputs, per_model, auroc, loss).
-    `model` may be a Predictor; it then runs on its own device with its own batch size (`batch_size` / `device` are not used)."""
+    `model` may be a Predictor; it then runs on its own device with its own batch size (`batch_size` / `device` are not used),
+    and `images_u8` may also be raw radiographs (see Predictor.__call__): a list is packed and uploaded once for all checkpoints."""
     if isinstance(model, Predictor):
         device = model.device
+        if isinstance(images_u8, (list, tuple)):
+            images_u8 = pack_radiographs(images_u8, model.size).to(device)
     t = targets.to(device)
     loss_fn = BCEWithLogitsLoss('none').to(device)
     per_model, losses = [], []

@@ -14,6 +14,7 @@ from . import _lib
 from .dataparallel import GradientBuckets
 from .densenet import build_model, conv_weight_plan
 from .loss import BCEWithLogitsLoss
+from .preprocess import Radiographs, prepare
 
 # dataset normalisation constants of the reference transform (chexpert.py:70-72)
 PIXEL_MEAN, PIXEL_STD = 0.5330, 0.0349
@@ -145,14 +146,21 @@ class TrainStep:
             torch.cuda.synchronize(self.device)
 
     def __call__(self, x, target):
-        """-> loss (0-dim device tensor; no host sync, unlike loss.item() at chexpert.py:167)."""
+        """-> loss (0-dim device tensor; no host sync, unlike loss.item() at chexpert.py:167).
+        x: the float (B, 3, S, S) model input, or a preprocess.Radiographs batch of raw 8-bit radiographs, which
+        preprocess.prepare turns into that input on the device (under the CUDA graph: straight into its static input)."""
         self._calls += 1
+        rad = x.to(self.device) if isinstance(x, Radiographs) else None
         if not self.cuda_graph or self._calls <= self.graph_after:
-            loss = self._step(x, target)
+            loss = self._step(x if rad is None else prepare(rad), target)
         else:
-            if self._graph is None or self._graph_lr != [g['lr'] for g in self.opt.param_groups]:
-                self._capture(x, target)
-            self._sx.copy_(x, non_blocking=True)
+            recapture = self._graph is None or self._graph_lr != [g['lr'] for g in self.opt.param_groups]
+            if recapture:
+                self._capture(x if rad is None else prepare(rad), target)
+            if rad is None:
+                self._sx.copy_(x, non_blocking=True)
+            elif not recapture:                 # a capture's static input already holds this batch
+                prepare(rad, out=self._sx)
             self._st.copy_(target, non_blocking=True)
             self._graph.replay()
             loss = self._sloss.clone()       # the static tensor is overwritten by the next replay

@@ -220,6 +220,19 @@ int aaconv_bn_relu_pool_backward(const void* x, int dtype, int B, int C, int H, 
                                  const float* saved, const float* weight, const float* bias, void* dx, int64_t dx_batch_stride,
                                  int dx_accumulate, float* dweight, float* dbias, void* workspace, void* stream);
 
+/* The reference's input transform (chexpert.py:64-79: Resize(S), CenterCrop(S), ToTensor, Normalize(0.5330, 0.0349), grey -> 3
+ * channels) for a ragged batch of 8-bit grayscale images in one launch (chexpert_b200/csrc/prep.cu), bit-identical to torchvision's
+ * PIL path (bilinear, 8-bit) followed by evaluate.normalise_u8 on the device.
+ *   pixels     the images' rows back to back, total_bytes bytes; never read outside [0, total_bytes)
+ *   geometry   (B, 8) int64 rows: byte offset of the image, h, w, resized h, resized w, crop top, crop left, 0 -- the resized size and
+ *              crop offsets by torchvision's rules (chexpert_b200.preprocess.pack_radiographs computes them)
+ *   max_side   an upper bound of every h and w of the batch, 1..8192 (sizes the launch's shared memory)
+ *   S          16..2048; out (B, 3, S, S) fp32 contiguous NCHW, three equal channels
+ * A geometry row the kernel cannot honour (a side past max_side, pixels outside the buffer, a crop outside the resized image) yields
+ * NaN for that image instead of a read out of bounds; the host is expected to validate first. */
+int aaconv_radiograph_prep(const uint8_t* pixels, int64_t total_bytes, const int64_t* geometry, int B, int max_side, int S,
+                           float* out, void* stream);
+
 /* Accounting / measurement helpers used by bench.py (no reference counterpart).
  *   aaconv_launch_count   kernels launched by this library since it was loaded (all threads).
  *   aaconv_profile_begin  start recording a (start, stop) CUDA-event pair around every launch (`stream` is unused, kept for ABI).
