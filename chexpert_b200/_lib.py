@@ -81,6 +81,8 @@ SYMBOLS = {
     'aaconv_bn_relu_pool_backward': (ctypes.c_int, [_P, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int64,
                                                     _P, _P, _P, _P, _P, ctypes.c_int64, ctypes.c_int, _P, _P, _P, _P]),
     'aaconv_radiograph_prep': (ctypes.c_int, [_P, ctypes.c_int64, _P, ctypes.c_int, ctypes.c_int, ctypes.c_int, _P, _P]),
+    'aaconv_grad_cam': (ctypes.c_int, [_P, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int64, _P, _P,
+                                       _P, _P, ctypes.c_float, _P, ctypes.c_int, _P, _P, ctypes.c_int, _P, _P]),
     'aaconv_launch_count': (ctypes.c_longlong, []),
     'aaconv_debug_set_timeline': (None, [_P]),
     'aaconv_debug_set_mode': (None, [ctypes.c_int]),

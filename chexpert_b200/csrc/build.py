@@ -11,7 +11,7 @@ import sys
 from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ['api.cu', 'runtime.cu', 'prologue.cu', 'bn_relu.cu', 'bn_cl.cu', 'fp32_gemms.cu', 'fp32_attn.cu', 'fp32_path.cu', 'bce.cu', 'eval_ops.cu', 'bf16_path.cu', 'tc_host.cu', 'aug_ops.cu', 'aug_tc.cu', 'attn_tc.cu', 'attn_cc.cu', 'attn_tc_bwd.cu', 'gemm_tc.cu', 'prep.cu']
+SOURCES = ['api.cu', 'runtime.cu', 'prologue.cu', 'bn_relu.cu', 'bn_cl.cu', 'fp32_gemms.cu', 'fp32_attn.cu', 'fp32_path.cu', 'bce.cu', 'eval_ops.cu', 'bf16_path.cu', 'tc_host.cu', 'aug_ops.cu', 'aug_tc.cu', 'attn_tc.cu', 'attn_cc.cu', 'attn_tc_bwd.cu', 'gemm_tc.cu', 'prep.cu', 'cam.cu']
 LIB = os.path.join(HERE, os.environ.get('AACONV_BUILD_NAME', 'libaaconv_b200.so'))
 EXTRA = os.environ.get('AACONV_BUILD_FLAGS', '').split()     # experiment variants: AACONV_BUILD_NAME=libx.so AACONV_BUILD_FLAGS='-DAACONV_CF_NWG=4'
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')

@@ -24,6 +24,7 @@ from torchvision.models.densenet import _DenseBlock, _DenseLayer
 from .aaconv import AAConv2d
 from .fused_bn import (bn_relu, tap_bn_relu, tap_bn_relu_cl, bn_relu_cl, cl_ok, slice_layout, _is_cl, bn_relu_eval, eval_ok,
                        eval_cl_ok, _fused_ok, pool_ok, bn_relu_pool, bn_relu_pool_eval, module_bn, _alias, _strided_ok)
+from .gradcam import grad_cam
 
 
 def transition_attn_dims(num_output_features, attn_params):
@@ -343,31 +344,65 @@ class DenseNet(nn.Module):
             return bn_relu_eval(bn, x)
         return bn_relu(bn, x)
 
-    def _features(self, x):
-        """-> relu(features(x)) (models/attn_aug_conv.py:513-514)."""
+    def _norm5_input(self, x):
+        """-> the input of features.norm5: the last dense block's output (with feature_buffer, its whole buffer)."""
+        mods = list(self.features.children())[:-1]                  # norm5 is the last child
         if not self.feature_buffer:
-            return F.relu(self.features(x), inplace=True)
-        mods = list(self.features.named_children())
+            for m in mods:
+                x = m(x)
+            return x
         skip = False
-        for i, (name, m) in enumerate(mods):
+        for i, m in enumerate(mods):
             if skip:
                 skip = False
                 continue
-            nxt = mods[i + 1][1] if i + 1 < len(mods) else None
+            nxt = mods[i + 1] if i + 1 < len(mods) else None
             if isinstance(m, (AATransition, BNTransition)) and isinstance(nxt, BufferedDenseBlock):
                 x = m(x, out_total=nxt.out_channels)      # the Transition writes into the next block's buffer
             elif isinstance(m, nn.BatchNorm2d) and isinstance(nxt, nn.ReLU):
                 x = self._bn_relu(m, x)                   # stem: norm0 -> relu0 as one fused op (grid (C, B) instead of one CTA per channel)
                 skip = True
-            elif isinstance(m, nn.BatchNorm2d) and nxt is None:
-                return self._bn_relu(m, x)                # norm5 followed by forward()'s F.relu
             else:
                 x = m(x)
-        return F.relu(x, inplace=True)
+        return x
+
+    def _norm5_relu(self, x):
+        """relu(features.norm5(x)): norm5 followed by forward()'s F.relu."""
+        if not self.feature_buffer:
+            return F.relu(self.features.norm5(x), inplace=True)
+        return self._bn_relu(self.features.norm5, x)
+
+    def _features(self, x):
+        """-> relu(features(x)) (models/attn_aug_conv.py:513-514).  Without feature_buffer model.features runs as the module it is,
+        so hooks on it keep firing."""
+        if not self.feature_buffer:
+            return F.relu(self.features(x), inplace=True)
+        return self._norm5_relu(self._norm5_input(x))
+
+    def _head(self, f):
+        return self.classifier(F.adaptive_avg_pool2d(f, (1, 1)).flatten(1))
 
     def forward(self, x):
-        f = self._features(x)
-        return self.classifier(F.adaptive_avg_pool2d(f, (1, 1)).flatten(1))
+        return self._head(self._features(x))
+
+    def forward_grad_cam(self, x, size=None):
+        """-> (logits, maps): the logits of forward(x) and Grad-CAM of every class at model.features' output (the layer the reference
+        hooks, chexpert.py:260-361), computed in closed form by gradcam.grad_cam from norm5's input -- no backward pass.  maps: fp32
+        (B, K, h, w) at the feature map's resolution, or (B, K, size, size) upsampled bilinearly when `size` is given.
+        Inference only: eval mode, CUDA, autograd off, and a norm5 the eval kernels take (fused_bn.eval_ok); anything else raises."""
+        if self.training:
+            raise RuntimeError('forward_grad_cam runs in eval mode only (call model.eval()): Grad-CAM here uses the running statistics')
+        if torch.is_grad_enabled():
+            raise RuntimeError('forward_grad_cam runs with autograd off (torch.no_grad()): its gradient is computed in closed form')
+        if not x.is_cuda:
+            raise RuntimeError('forward_grad_cam runs on CUDA only; there is no CPU fallback')
+        h = self._norm5_input(x)
+        if not eval_ok(self.features.norm5, h):
+            raise RuntimeError('forward_grad_cam needs an affine norm5 with fp32 parameters and running statistics and an fp32 / bf16 '
+                               'feature map of at most 65535 samples')
+        logits = self._head(self._norm5_relu(h))
+        cam, up = grad_cam(h, self.features.norm5, self.classifier, size)
+        return logits, cam if up is None else up
 
     def attn_layers(self):
         """The AAConv2d modules the visualise path hooks (chexpert.py:478)."""

@@ -8,6 +8,7 @@ visualise path reads (chexpert.py:365,383-387).
                                                      through the C ABI: aaconv_ensemble_mean / aaconv_auroc / BCE kernel)
     chexpert.py:130-146  compute_metrics         ->  auroc_per_class
     chexpert.py:363-397  vis_attn (data part)    ->  attention_maps
+    chexpert.py:260-361  grad_cam (data part)    ->  Predictor.grad_cam  (closed form at norm5, aaconv_grad_cam; see gradcam.py)
 
 No sklearn, no host round trip per batch; plotting is out of scope (DESIGN.md section 8).
 """
@@ -129,6 +130,9 @@ class Predictor:
     way from a static prepared (batch_size, 3, S, S) input onward; the prep launch runs before each replay, so batches of any
     geometries replay it.
 
+    ``grad_cam(images)`` returns the same logits together with Grad-CAM maps of every class at the model's input size
+    (DenseNet.forward_grad_cam); each input form has a graph of its own for it, captured the same way.
+
     ``arch='densenet121'``: the reference's baseline, torchvision's densenet121, as densenet121(feature_buffer=True,
     fused_transition=True, fused_eval=True) -- its Transitions' BatchNorm + ReLU + pool run through the eval-mode pooled kernel."""
 
@@ -148,7 +152,7 @@ class Predictor:
                                              memory_format=torch.channels_last if cl else torch.contiguous_format)
         self.model = model.to(self.device).eval()
         self.cuda_graph = bool(cuda_graph)
-        self._warm = {'u8': 0, 'raw': 0}
+        self._warm = {'u8': 0, 'raw': 0, 'u8_cam': 0, 'raw_cam': 0}
         self._graphs = {}                   # input path -> (graph, static logits)
         self._sx = self._rx = None          # static inputs: uint8 (batch_size, S, S); prepared float (batch_size, 3, S, S)
         self.captures = 0
@@ -158,19 +162,26 @@ class Predictor:
         with torch.no_grad():
             self.model.load_state_dict(state_dict, strict=True)
 
-    def _forward(self, u8):
-        return self._model_forward(normalise_u8(u8))
+    def _forward(self, u8, cam=False):
+        return self._model_forward(normalise_u8(u8), cam)
 
-    def _model_forward(self, x):
+    def _model_forward(self, x, cam=False):
+        """-> logits, or (logits, Grad-CAM maps at the input size) when `cam`."""
         with torch.autocast('cuda', dtype=torch.bfloat16, enabled=self.autocast, cache_enabled=False):
-            return self.model(x).float()
+            if not cam:
+                return self.model(x).float()
+            logits, maps = self.model.forward_grad_cam(x, self.size)
+            return logits.float(), maps
 
     def _run(self, path, forward, sx, n):
-        """forward(sx)[:n]: eager for the first WARMUP batches of this input path, then through the path's graph, captured once."""
+        """forward(sx), each output sliced to [:n]: eager for the first WARMUP batches of this input path, then through the path's
+        graph, captured once."""
+        def head(y):
+            return tuple(t[:n] for t in y) if isinstance(y, tuple) else y[:n]
         if path not in self._graphs:
             if self._warm[path] < self.WARMUP:
                 self._warm[path] += 1
-                return forward(sx)[:n]
+                return head(forward(sx))
             torch.cuda.synchronize(self.device)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
@@ -179,34 +190,28 @@ class Predictor:
             self.captures += 1
         graph, sy = self._graphs[path]
         graph.replay()
-        return sy[:n]
+        return head(sy)
 
-    def _batch(self, chunk):
+    def _batch(self, chunk, cam=False):
         n = chunk.shape[0]
         if not self.cuda_graph:
-            return self._forward(chunk.to(self.device, non_blocking=True))
+            return self._forward(chunk.to(self.device, non_blocking=True), cam)
         if self._sx is None:
             self._sx = torch.zeros(self.batch_size, *chunk.shape[1:], dtype=torch.uint8, device=self.device)
         self._sx[:n].copy_(chunk, non_blocking=True)       # rows [n, batch_size) keep earlier images: padding, sliced off below
-        return self._run('u8', self._forward, self._sx, n)
+        return self._run('u8_cam' if cam else 'u8', lambda sx: self._forward(sx, cam), self._sx, n)
 
-    def _raw_batch(self, rad):
+    def _raw_batch(self, rad, cam=False):
         """Radiographs on the device -> logits: one prep launch, then the model from the prepared tensor onward."""
         n = len(rad)
         if not self.cuda_graph:
-            return self._model_forward(prepare(rad))
+            return self._model_forward(prepare(rad), cam)
         if self._rx is None:
             self._rx = torch.zeros(self.batch_size, 3, self.size, self.size, dtype=torch.float32, device=self.device)
         prepare(rad, out=self._rx[:n])                      # rows [n, batch_size): padding, as in _batch
-        return self._run('raw', self._model_forward, self._rx, n)
+        return self._run('raw_cam' if cam else 'raw', lambda rx: self._model_forward(rx, cam), self._rx, n)
 
-    @torch.no_grad()
-    def __call__(self, images):
-        """-> (N, num_classes) float32 logits on the device, batch by batch, from either
-        - uint8 (N, S, S) images already at the model's size, on the host or the device, normalised by normalise_u8; or
-        - raw radiographs of any sizes: a list of 2-D uint8 host images (packed and uploaded batch by batch), or a
-          preprocess.Radiographs of side S (uploaded whole if on the host).  preprocess.prepare runs the reference's
-          Resize(S) + CenterCrop(S) + normalisation on the device, one launch per batch; its CUDA graph starts after it."""
+    def _predict(self, images, cam):
         raw = isinstance(images, (Radiographs, list, tuple))
         if not raw and (images.dtype != torch.uint8 or images.dim() != 3):
             raise RuntimeError(f'Predictor takes uint8 (N, H, W) images, got {images.dtype} {tuple(images.shape)}')
@@ -217,16 +222,37 @@ class Predictor:
                 images = images.to(self.device)
             N = len(images)
             out = torch.empty(N, self.num_classes, device=self.device, dtype=torch.float32)
+            maps = torch.empty(N, self.num_classes, self.size, self.size, device=self.device, dtype=torch.float32) if cam else None
             for i in range(0, N, self.batch_size):
                 chunk = images[i:i + self.batch_size]
                 if isinstance(chunk, Radiographs):
-                    y = self._raw_batch(chunk)
+                    y = self._raw_batch(chunk, cam)
                 elif raw:
-                    y = self._raw_batch(pack_radiographs(chunk, self.size).to(self.device))
+                    y = self._raw_batch(pack_radiographs(chunk, self.size).to(self.device), cam)
                 else:
-                    y = self._batch(chunk)
+                    y = self._batch(chunk, cam)
+                if cam:
+                    y, m = y
+                    maps[i:i + m.shape[0]].copy_(m)
                 out[i:i + y.shape[0]].copy_(y)
-            return out
+            return out, maps
+
+    @torch.no_grad()
+    def __call__(self, images):
+        """-> (N, num_classes) float32 logits on the device, batch by batch, from either
+        - uint8 (N, S, S) images already at the model's size, on the host or the device, normalised by normalise_u8; or
+        - raw radiographs of any sizes: a list of 2-D uint8 host images (packed and uploaded batch by batch), or a
+          preprocess.Radiographs of side S (uploaded whole if on the host).  preprocess.prepare runs the reference's
+          Resize(S) + CenterCrop(S) + normalisation on the device, one launch per batch; its CUDA graph starts after it."""
+        return self._predict(images, cam=False)[0]
+
+    @torch.no_grad()
+    def grad_cam(self, images):
+        """-> (logits (N, num_classes), maps (N, num_classes, S, S)), both float32 on the device, from the inputs __call__ takes.
+        The logits are __call__'s, bit for bit; maps[:, c] is Grad-CAM of class c at model.features' output (the layer the reference
+        hooks, chexpert.py:260-361), upsampled bilinearly to the input size S (DenseNet.forward_grad_cam, gradcam.py).  Each input
+        form has a graph of its own for this step."""
+        return self._predict(images, cam=True)
 
 
 @torch.no_grad()

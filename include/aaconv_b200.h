@@ -233,6 +233,24 @@ int aaconv_bn_relu_pool_backward(const void* x, int dtype, int B, int C, int H, 
 int aaconv_radiograph_prep(const uint8_t* pixels, int64_t total_bytes, const int64_t* geometry, int B, int max_side, int S,
                            float* out, void* stream);
 
+/* Grad-CAM at features.norm5 of the DenseNets (the data part of chexpert.py:260-361) in closed form, from norm5's input
+ * (chexpert_b200/csrc/cam.cu).  The head is norm5 -> relu -> global average pool -> Linear, so with A = norm5(x) computed as the eval
+ * apply kernels compute it (fmaf(x, s_k, t_k), bn_eval_affine) and n = h*w:
+ *   cam[b, c, p] = max(0, sum_k W[c,k] m_k / n^2 * A_k[p]),  m_k = #{p : A_k[p] > 0}
+ * which is Grad-CAM (Selvaraju et al. 2017) with the gradient of logit c with respect to model.features' output.
+ *   x            (B, C, h, w) NCHW of `dtype` (AACONV_FP32 | AACONV_BF16), dense samples, x_batch_stride >= C*h*w elements between
+ *                samples (e.g. the last dense block's feature buffer); aligned to its element size
+ *   weight .. eps  norm5's affine and running statistics (fp32, C)
+ *   cls_weight   (K, C) fp32 contiguous: classifier.weight
+ *   cam          (B, K, h, w) fp32 contiguous out
+ *   up           NULL, or (B, K, S, S) fp32 contiguous out: cam upsampled as F.interpolate(mode='bilinear', align_corners=False)
+ *   workspace    B*C int32 elements (the counts m_k)
+ * Limits: 1 <= B <= 65535, 1 <= C <= 4096, h*w <= 4096 (64 x 64), 1 <= K <= 64, 1 <= S <= 4096.  Deterministic: fixed-order sums,
+ * no atomics; an image's maps do not depend on the other images of the batch. */
+int aaconv_grad_cam(const void* x, int dtype, int B, int C, int h, int w, int64_t x_batch_stride, const float* weight,
+                    const float* bias, const float* running_mean, const float* running_var, float eps, const float* cls_weight, int K,
+                    float* cam, float* up, int S, int32_t* workspace, void* stream);
+
 /* Accounting / measurement helpers used by bench.py (no reference counterpart).
  *   aaconv_launch_count   kernels launched by this library since it was loaded (all threads).
  *   aaconv_profile_begin  start recording a (start, stop) CUDA-event pair around every launch (`stream` is unused, kept for ABI).
