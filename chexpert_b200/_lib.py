@@ -7,7 +7,7 @@ import os
 import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get('AACONV_LIB_PATH') or os.path.join(_HERE, 'csrc', 'libaaconv_b200.so')   # env: experiment builds only
+LIB_PATH = os.path.join(_HERE, 'csrc', 'libaaconv_b200.so')
 
 FP32, BF16 = 0, 1
 PRECISIONS = {'fp32': FP32, 'bf16': BF16}

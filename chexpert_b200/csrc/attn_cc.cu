@@ -13,7 +13,6 @@
 // rings running on a global tile counter); the rules that keeps their mbarrier parity waits exact are next to cb_plan.
 // Reference rows a3-a8 (attn_aug_conv.py:75-91) and their adjoint; layouts as in attn_tc_bwd.cu.
 #include <algorithm>
-#include <cstdlib>
 #include "tc_common.cuh"
 #include "bf16_path.cuh"
 
@@ -22,15 +21,12 @@ namespace aaconv {
 using tc::smem_u32;
 typedef __nv_bfloat16 bf16;
 
-// ablation switches for tools/attn_ablate.py (0 in production): 1 no MUFU, 2 no global traffic after the first tiles,
-// 4 no gradient MMAs, 8 no math at all, 32 dQa drain by per-row stores; 16 = soft mbarrier timeouts (tools/dbg_shape.py)
-int g_attn_dbg_mode = 0;
 static unsigned long long* g_mbar_host_log = nullptr;
 extern long long* g_attn_dbg;      // attn_tc_bwd.cu: timeline buffer of TL_EVENTS x TL_COLS stamps (tools/attn_timeline.py)
 constexpr int TL_COLS = 96, TL_CTA = 40;
 #define TL_STAMP(tl, ev, col) do { if ((tl) && (col) < TL_COLS) (tl)[(ev) * TL_COLS + (col)] = clock64(); } while (0)
+// bit 16 of m: soft mbarrier timeouts (tools/dbg_shape.py); every other bit is ignored
 extern "C" void aaconv_debug_set_mode(int m) {
-  g_attn_dbg_mode = m & 47;            // bit 32: dQa drain by per-row stores instead of the bulk store
   const unsigned soft = (m >> 4) & 1;                    // bit 16: soft mbarrier timeouts in this file's kernels (see tc_common.cuh)
   static unsigned long long* host_log = nullptr;
   if (soft && !host_log) cudaHostAlloc(reinterpret_cast<void**>(&host_log), 65 * sizeof(unsigned long long), cudaHostAllocMapped);
@@ -137,7 +133,7 @@ __device__ __forceinline__ void fwd_cc_half(uint32_t (&r)[2][32], uint32_t vt, i
       }
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
-        const float p = tc::ex2_mixed(__uint_as_float(r[c][i + u]) + mneg, u);
+        const float p = tc::ex2f(__uint_as_float(r[c][i + u]) + mneg);
         if (u & 1) l2 += p; else l += p;
 #pragma unroll
         for (int e = 0; e < DVH; ++e) {
@@ -222,7 +218,7 @@ __device__ __forceinline__ void cf_score_loop(Smem& sm, uint32_t tmem, int ntile
 template <int KATOMS, int DVH>
 __global__ void __launch_bounds__(CF_THREADS, 1) attn_fwd_cc_kernel(
     const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k, const float* __restrict__ v,
-    float* __restrict__ o, float* __restrict__ lse, int L, int C1, int nqt, int nitems, int dbg) {
+    float* __restrict__ o, float* __restrict__ lse, int L, int C1, int nqt, int nitems) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   typedef CfSmem<KATOMS, DVH> Smem;
   Smem& sm = *reinterpret_cast<Smem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -325,16 +321,14 @@ __global__ void __launch_bounds__(CF_THREADS, 1) attn_fwd_cc_kernel(
         tc::tmem_ld_x32(tslot + 0, r[0]);
         tc::tmem_ld_x32(tslot + 32, r[1]);
         tc::tmem_ld_wait();
-        if (dbg & 8) l += __uint_as_float(r[0][0]);
-        else if (nvalid < 64) fwd_cc_half<DVH, true>(r, vt, nvalid, m, l, acc);
+        if (nvalid < 64) fwd_cc_half<DVH, true>(r, vt, nvalid, m, l, acc);
         else fwd_cc_half<DVH, false>(r, vt, nvalid, m, l, acc);
         tc::tmem_ld_x32(tslot + 64, r[0]);
         tc::tmem_ld_x32(tslot + 96, r[1]);
         tc::tmem_ld_wait();
         tc::tc_fence_before();
         tc::mbar_arrive(&sm.bar_slot_free[slot]);   // all scores of the tile have been read: the slot can be refilled
-        if (dbg & 8) l += __uint_as_float(r[0][0]);
-        else if (nvalid < CF_BN) { if (nvalid > 64) fwd_cc_half<DVH, true>(r, vt + 64 * DVH * 4, nvalid - 64, m, l, acc); }
+        if (nvalid < CF_BN) { if (nvalid > 64) fwd_cc_half<DVH, true>(r, vt + 64 * DVH * 4, nvalid - 64, m, l, acc); }
         else fwd_cc_half<DVH, false>(r, vt + 64 * DVH * 4, nvalid - 64, m, l, acc);
         tc::mbar_arrive(&sm.bar_empty[st]);          // value tile consumed
       }
@@ -388,7 +382,7 @@ __global__ void __launch_bounds__(CF_THREADS, 1) attn_fwd_cc_kernel(
 // ================================================================================================
 // backward
 // ================================================================================================
-constexpr int CB_BM = 128, CB_BN = 64, CB_MAXSLOTS = 7;
+constexpr int CB_BM = 128, CB_BN = 64, CB_MAXSLOTS = 5;
 // three math warpgroups (global tile t -> warpgroup t % 3): three warps per scheduler keep the MUFU pipe busy while the others sit
 // in TMEM load / store / barrier latencies;  then one TMA warp, the score-MMA issuer (+TMEM alloc) and the gradient-MMA issuer
 // (warp CB_W_G), and TWO score-MMA issuers (CB_W_S even global tiles + TMEM alloc, CB_W_S2 odd ones): the timeline showed a
@@ -398,15 +392,15 @@ constexpr int CB_NWG = 3, CB_W_TMA = 4 * CB_NWG, CB_W_S = CB_W_TMA + 1, CB_W_G =
 // Streamed-tile stages.  A stage is held from its TMA issue until the tile's GRADIENT MMA has completed (~3.5 tiles of
 // pipeline), so the prefetch lead is ST - 4.5 tiles; with 6 stages the score issuer waited 400-900 cycles per tile for the
 // K tile to land (timeline).  The dQa kernel also holds a 24-88 KB staging tile (sized by OUTW >= KD), the dK/dV kernel does not.
-template <int KATOMS, int OUT_FLOATS, int NSTAT = 1> struct CbStages {   // as many as fit beside the stationary tile(s) and the staging tile
-  static constexpr int fixed = 1024 /*alignment slack*/ + (NSTAT > 1 ? 8192 : 4096) /*side rows, barriers*/ + (NSTAT > 1 ? 4096 : 2048) /*static dV exchange*/;
-  static constexpr int avail = 232448 - fixed - NSTAT * KATOMS * CB_BM * 128 - OUT_FLOATS * 4;
+template <int KATOMS, int OUT_FLOATS> struct CbStages {   // as many as fit beside the stationary tile and the staging tile
+  static constexpr int fixed = 1024 /*alignment slack*/ + 4096 /*side rows, barriers*/ + 2048 /*static dV exchange*/;
+  static constexpr int avail = 232448 - fixed - KATOMS * CB_BM * 128 - OUT_FLOATS * 4;
   static constexpr int fit = avail / (KATOMS * CB_BN * 128);
   static constexpr int value = fit > 10 ? 10 : fit;
   static_assert(value >= 3, "not enough shared memory for three streamed stages");
 };
 
-// TMEM plan of a backward kernel whose accumulator needs ACC columns: QB stationary buffers, NS score slots of 64 columns
+// TMEM plan of a backward kernel whose accumulator needs ACC columns: one stationary buffer, NS score slots of 64 columns.
 // The pipeline is latency-bound by (tiles in flight) / (S' MMA + TMEM round trip + math + gradient MMA ~ 2700 cycles), i.e. by
 // the number of score slots: the stationary operand gets ONE buffer (it is refilled right after the item's last score MMA,
 // which is when a second buffer would have been filled too) and every remaining column goes to slots.
@@ -418,29 +412,26 @@ template <int KATOMS, int OUT_FLOATS, int NSTAT = 1> struct CbStages {   // as m
 // Two score issuers when there are enough stages for both to have a tile in flight; one otherwise.
 // (and an item of a single tile would leave one issuer without a commit on bar_s_done for that item)
 __host__ __device__ constexpr int cb_issuers(int stages, int ntiles) { return (stages >= 4 && ntiles >= 2) ? 2 : 1; }
-struct CbPlan { int QB, NS; uint32_t col_slot0, col_acc; };
-// qb = 1: the stationary operand lives in TMEM (TS-mode score MMAs, at most 5 slots); qb = 0: it stays in shared memory
-// (SS-mode, double-buffered by item parity) and its columns become score slots
-__device__ __forceinline__ CbPlan cb_plan(int katoms, int acc_cols, int stages, int ntiles, int qb = 1) {
+struct CbPlan { int NS; uint32_t col_slot0, col_acc; };
+// the stationary operand lives in TMEM at column 0 (TS-mode score MMAs, at most CB_MAXSLOTS slots)
+__device__ __forceinline__ CbPlan cb_plan(int katoms, int acc_cols, int stages, int ntiles) {
   CbPlan p;
-  p.QB = qb;
-  p.NS = min(qb ? 5 : CB_MAXSLOTS, (512 - p.QB * katoms * 32 - acc_cols) / 64);
+  p.NS = min(CB_MAXSLOTS, (512 - katoms * 32 - acc_cols) / 64);
   if (stages & 1) p.NS = min(p.NS, stages);
   // Math warpgroups: global tile t belongs to warpgroup t % 3, so before waiting for S'(t) on slot t % NS a warpgroup has
   // seen S'(t-3) complete; the slot's previous phase is S'(t-NS).  With ONE issuer the score MMAs complete in order and
   // NS >= 3 suffices; with TWO issuers (even / odd tiles) t-NS and t-3 must come from the same issuer, i.e. NS must be odd
   // (3 or 5).  NS = 4 with two issuers (512-px dQa kernel with 4 stages) let a warpgroup run ahead of the lagging issuer.
   if (cb_issuers(stages, ntiles) == 2 && !(p.NS & 1)) p.NS -= 1;
-  p.col_slot0 = p.QB * katoms * 32;
+  p.col_slot0 = katoms * 32;
   p.col_acc = p.col_slot0 + 64 * p.NS;
   return p;
 }
 
-template <int KATOMS, int SIDE_FLOATS, int OUT_FLOATS, int ROW_FLOATS, int NSTAT = 1>
+template <int KATOMS, int SIDE_FLOATS, int OUT_FLOATS, int ROW_FLOATS>
 struct __align__(1024) CbSmem {
-  static constexpr int ST = CbStages<KATOMS, OUT_FLOATS, NSTAT>::value;
-  static constexpr int NST = NSTAT;
-  bf16 stat[NSTAT * KATOMS][CB_BM * 64];         // NSTAT = 2 (SS mode): buffer (item parity) * KATOMS + atom
+  static constexpr int ST = CbStages<KATOMS, OUT_FLOATS>::value;
+  bf16 stat[KATOMS][CB_BM * 64];
   bf16 strm[ST][KATOMS][CB_BN * 64];
   float side[ST][SIDE_FLOATS];                 // fp32 side tile: v (dq kernel) or dO | delta (dkv kernel)
   float rowside[2][CB_BM * ROW_FLOATS];        // fp32 rows of the stationary tile (dO | delta, or v), by item parity
@@ -459,8 +450,7 @@ __device__ __forceinline__ void cb_load_stat(Smem& sm, const CUtensorMap* m_stat
   const int nrows = min(CB_BM, L - row0);
   const size_t g0 = (size_t)bn * L + row0;
   tc::mbar_arrive_expect_tx(&sm.bar_stat, KATOMS * CB_BM * 64 * 2 + nrows * (RW0 + RW1) * 4);
-  const int sb = (Smem::NST > 1 ? (parity & 1) : 0) * KATOMS;
-  for (int a = 0; a < KATOMS; ++a) tc::tma_load_3d(sm.stat[sb + a], m_stat, &sm.bar_stat, a * 64, row0, bn);
+  for (int a = 0; a < KATOMS; ++a) tc::tma_load_3d(sm.stat[a], m_stat, &sm.bar_stat, a * 64, row0, bn);
   bulk_g2s(sm.rowside[parity], r0 + g0 * RW0, nrows * RW0 * 4, &sm.bar_stat);
   if (RW1) bulk_g2s(sm.rowside[parity] + CB_BM * RW0, r1 + g0 * RW1, nrows * RW1 * 4, &sm.bar_stat);
 }
@@ -498,7 +488,7 @@ __device__ __forceinline__ void cb_init(Smem& sm, int warp, int lane, const CUte
 template <int KATOMS, class Smem>
 __device__ __forceinline__ void cb_producer(Smem& sm, const CUtensorMap* m_stat, const CUtensorMap* m_strm, const float* side0,
                                             int SW0, const float* side1, int SW1, const float* r0, int RW0, const float* r1, int RW1,
-                                            int L, int nqt, int ntiles, int my_items, int dbg, long long* tl = nullptr) {
+                                            int L, int nqt, int ntiles, int my_items, long long* tl = nullptr) {
   Ring rg;
   // the next item's stationary tile is requested half-way through the item: by then every warpgroup has started the item
   // (bar_stat_free), so this wait never holds up the tile stream, and the tile still lands long before it is needed
@@ -508,19 +498,14 @@ __device__ __forceinline__ void cb_producer(Smem& sm, const CUtensorMap* m_stat,
     for (int j = 0; j < ntiles; ++j, rg.next(Smem::ST)) {
       if (j == jq && it + 1 < my_items) {              // next item's stationary tile: the staging buffer is free once WG0
         const int nitem = item + gridDim.x, nbn = nitem / nqt, nrow0 = (nitem - nbn * nqt) * CB_BM;   // has moved this item's to TMEM
-        tc::hb(1, it * 1000 + j);
         tc::mbar_wait(&sm.bar_stat_free, it & 1);
-        if (Smem::NST > 1 && it > 0) tc::mbar_wait(&sm.bar_s_done, (it - 1) & 1);   // SS mode: item it-1's score MMAs have read stat[(it+1)&1]
-        tc::hb(1, 500000 + it * 1000 + j);
         cb_load_stat<KATOMS>(sm, m_stat, r0, RW0, r1, RW1, L, nbn, nrow0, (it + 1) & 1);
       }
       const int s = rg.i;
       const int nvalid = min(CB_BN, L - j * CB_BN);
       const size_t r0 = (size_t)bn * L + (size_t)j * CB_BN;
-      tc::hb(0, it * 1000 + j);
       tc::mbar_wait(&sm.bar_empty[s], rg.ph ^ 1);
       TL_STAMP(tl, 14, it * ntiles + j);
-      if ((dbg & 2) && (it > 0 || j >= Smem::ST)) { tc::mbar_arrive(&sm.bar_full[s]); continue; }     // ablation: no global traffic
       tc::mbar_arrive_expect_tx(&sm.bar_full[s], KATOMS * CB_BN * 64 * 2 + nvalid * (SW0 + SW1) * 4);
       for (int a = 0; a < KATOMS; ++a) tc::tma_load_3d(sm.strm[s][a], m_strm, &sm.bar_full[s], a * 64, j * CB_BN, bn);
       bulk_g2s(sm.side[s], side0 + r0 * SW0, nvalid * SW0 * 4, &sm.bar_full[s]);
@@ -540,36 +525,25 @@ __device__ __forceinline__ void cb_score_loop(Smem& sm, uint32_t tmem, CbPlan pl
   Ring rst, rsl;
   for (int i = 0; i < sidx; ++i) { rst.next(Smem::ST); rsl.next(NS); }
   int it = 0, j = sidx, a_it = -1;
-  uint32_t a_tmem = tmem, a_smem = 0;
-  constexpr uint32_t STAT_ATOM = (CB_BM * 128) >> 4;
   for (int t = sidx; t < total; t += nstep) {
     while (j >= ntiles) { j -= ntiles; ++it; }
     if (it != a_it) {                              // first tile of an item for this issuer: its stationary operand is in TMEM
-      if (Smem::NST > 1) {                           // (SS mode: in shared memory buffer it & 1, landed with bar_stat)
-        tc::mbar_wait(&sm.bar_stat, it & 1);
-        a_smem = tc::desc_lo_k(smem_u32(sm.stat[(it & 1) * KATOMS]));
-      } else {
-        tc::mbar_wait(&sm.bar_a_ready, it & 1);
-        a_tmem = tmem + (uint32_t)((it & (pl.QB - 1)) * KATOMS * 32);
-      }
+      tc::mbar_wait(&sm.bar_a_ready, it & 1);
       a_it = it;
     }
     const int st = rst.i, slot = rsl.i;
     TL_STAMP(tl, 0, t);
-    if (lane_id() == 0) tc::hb(2 + sidx, it * 1000 + j);
     tc::mbar_wait(&sm.bar_full[st], rst.ph);
     TL_STAMP(tl, 1, t);
     if (t >= NS) tc::mbar_wait(&sm.bar_slot_free[slot], rsl.ph ^ 1);
     tc::tc_fence_after();
     TL_STAMP(tl, 2, t);
     if (tc::elect_one()) {
-      if (Smem::NST > 1) tc::issue_ss_ksteps<NKS, STAT_ATOM, STRM_ATOM>(tmem + pl.col_slot0 + 64 * slot, a_smem, strm_lo + st * STAGE, idesc_s);
-      else tc::issue_ts_ksteps<NKS, 0, STRM_ATOM>(tmem + pl.col_slot0 + 64 * slot, 0u, a_tmem, strm_lo + st * STAGE, idesc_s);
+      tc::issue_ts_ksteps<NKS, 0, STRM_ATOM>(tmem + pl.col_slot0 + 64 * slot, 0u, tmem, strm_lo + st * STAGE, idesc_s);
       tc::mma_commit(&sm.bar_s_full[slot]);
       if (j + nstep >= ntiles) tc::mma_commit(&sm.bar_s_done);   // this issuer's last tile of the item
     }
     __syncwarp();
-    if (lane_id() == 0) tc::hb(2 + sidx, 500000 + it * 1000 + j);
     TL_STAMP(tl, 3, t);
     j += nstep;
     for (int i = 0; i < nstep; ++i) { rst.next(Smem::ST); rsl.next(NS); }
@@ -598,7 +572,7 @@ __device__ __forceinline__ void cb_score_issuer(Smem& sm, uint32_t tmem, CbPlan 
 
 // gradient-MMA issuer shared by both backward kernels: acc (+)= dS(t)[TMEM slot] . streamed tile (MN-major view), N = n_acc
 template <int KATOMS, class Smem>
-__device__ __forceinline__ void cb_grad_issuer(Smem& sm, uint32_t tmem, CbPlan pl, uint32_t idesc, int ntiles, int my_items, int dbg,
+__device__ __forceinline__ void cb_grad_issuer(Smem& sm, uint32_t tmem, CbPlan pl, uint32_t idesc, int ntiles, int my_items,
                                                long long* tl = nullptr) {
   constexpr uint32_t STRM_ATOM = (CB_BN * 128) >> 4, STAGE = KATOMS * STRM_ATOM;
   const uint32_t b_lo = tc::desc_lo_mn(smem_u32(sm.strm[0][0]), CB_BN * 128);
@@ -609,7 +583,6 @@ __device__ __forceinline__ void cb_grad_issuer(Smem& sm, uint32_t tmem, CbPlan p
       const int st = rst.i, slot = rsl.i;
       const uint32_t tslot = tmem + pl.col_slot0 + 64 * slot;
       TL_STAMP(tl, 4, it * ntiles + jj);
-      if (lane_id() == 0) tc::hb(4, it * 1000 + jj);
       tc::mbar_wait(&sm.bar_p_ready[slot], rsl.ph);
       if (jj == 0 && it > 0) tc::mbar_wait(&sm.bar_acc_free, (it - 1) & 1);   // previous item's accumulator has been drained
       tc::tc_fence_after();
@@ -618,13 +591,12 @@ __device__ __forceinline__ void cb_grad_issuer(Smem& sm, uint32_t tmem, CbPlan p
         const uint32_t bb = b_lo + st * STAGE;
 #pragma unroll
         for (int ks = 0; ks < CB_BN / 16; ++ks)
-          if (!(dbg & 4) || jj == 0) tc::mma_ts(tmem + pl.col_acc, tslot + ks * 8, tc::desc64(bb + ks * 128), idesc, (jj > 0 || ks > 0) ? 1u : 0u);
+          tc::mma_ts(tmem + pl.col_acc, tslot + ks * 8, tc::desc64(bb + ks * 128), idesc, (jj > 0 || ks > 0) ? 1u : 0u);
         tc::mma_commit(&sm.bar_empty[st]);
         tc::mma_commit(&sm.bar_slot_free[slot]);
         if (jj == ntiles - 1) tc::mma_commit(&sm.bar_final);
       }
       __syncwarp();
-      if (lane_id() == 0) tc::hb(4, 500000 + it * 1000 + jj);
       TL_STAMP(tl, 6, it * ntiles + jj);
     }
   }
@@ -648,7 +620,7 @@ __device__ __forceinline__ void dq_cc_chunk(const uint32_t (&rs)[32], uint32_t (
       float dp = ndelta;
 #pragma unroll
       for (int e = 0; e < DVH; ++e) dp = fmaf(go[e], vv[u * DVH + e], dp);
-      ds[u] = tc::ex2_mixed(__uint_as_float(rs[i + u]), u) * dp;
+      ds[u] = tc::ex2f(__uint_as_float(rs[i + u])) * dp;
       if (TAIL && C * 32 + i + u >= nvalid) ds[u] = 0.f;     // zero-filled keys past L
     }
     pd[C * 16 + (i >> 1)] = tc::pack_bf16x2(ds[0], ds[1]);
@@ -677,7 +649,7 @@ __device__ __forceinline__ void dkv_cc_chunk(const uint32_t (&rs)[32], uint32_t 
       float dp = -dls[u];
 #pragma unroll
       for (int e = 0; e < DVH; ++e) dp = fmaf(gg[u * DVH + e], vk[e], dp);
-      float p = tc::ex2_mixed(__uint_as_float(rs[i + u]), u);
+      float p = tc::ex2f(__uint_as_float(rs[i + u]));
       const bool dead = TAIL && C * 32 + i + u >= nvalid;    // zero-filled queries past L: the side tile holds stale data there
       if (dead) { p = 0.f; dp = 0.f; }
 #pragma unroll
@@ -690,12 +662,12 @@ __device__ __forceinline__ void dkv_cc_chunk(const uint32_t (&rs)[32], uint32_t 
 }
 
 // ---- query-stationary: dQa ------------------------------------------------------------------------
-// TMEM: Qa buffers [0, QB*32K); slot s: S' at col_slot0 + 64 s (dS, bf16, over its first 32 columns); dQa behind the slots.
+// TMEM: Qa tile [0, 32K); slot s: S' at col_slot0 + 64 s (dS, bf16, over its first 32 columns); dQa behind the slots.
 template <int KATOMS, int DVH, int OUTW>
 __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dq_cc_kernel(
     const __grid_constant__ CUtensorMap tm_q_stat, const __grid_constant__ CUtensorMap tm_k_strm,
     const float* __restrict__ v, const float* __restrict__ d_o, const float* __restrict__ delta, float* __restrict__ dqa, int L,
-    int KD, int NQ, int C1, int nqt, int nitems, int dbg, long long* __restrict__ tl_buf) {
+    int KD, int NQ, int C1, int nqt, int nitems, long long* __restrict__ tl_buf) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   typedef CbSmem<KATOMS, CB_BN * DVH, CB_BM * OUTW, DVH + 1> Smem;
   Smem& sm = *reinterpret_cast<Smem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -712,26 +684,26 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dq_cc_kernel(
 
   if (warp == CB_W_TMA) {
     if (lane == 0)
-      cb_producer<KATOMS>(sm, &tm_q_stat, &tm_k_strm, v, DVH, nullptr, 0, d_o, DVH, delta, 1, L, nqt, ntiles, my_items, dbg, tl);
+      cb_producer<KATOMS>(sm, &tm_q_stat, &tm_k_strm, v, DVH, nullptr, 0, d_o, DVH, delta, 1, L, nqt, ntiles, my_items, tl);
   } else if (warp == CB_W_S || warp == CB_W_S2) {
     cb_score_issuer<KATOMS>(sm, tmem, pl, C1 >> 4, ntiles, my_items, warp == CB_W_S ? 0 : 1, warp == CB_W_S ? tl : nullptr);
   } else if (warp == CB_W_G) {
-    cb_grad_issuer<KATOMS>(sm, tmem, pl, tc::idesc_bf16_f32(CB_BM, NQ) | (1u << 16), ntiles, my_items, dbg, tl);
+    cb_grad_issuer<KATOMS>(sm, tmem, pl, tc::idesc_bf16_f32(CB_BM, NQ) | (1u << 16), ntiles, my_items, tl);
   } else {
     const int wg = warp >> 2;
     const int rowi = (warp & 3) * 32 + lane;
     const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
     const int NS = pl.NS;
-    auto stage_stat = [&](int it) {                   // WG0: stationary tile of item `it` -> its TMEM buffer
+    auto stage_stat = [&](int it) {                   // WG0: stationary tile of item `it` -> TMEM
       tc::mbar_wait(&sm.bar_stat, it & 1);
-      stationary_to_tmem<KATOMS>(sm.stat, tlane + (uint32_t)((it & (pl.QB - 1)) * KATOMS * 32), rowi);
+      stationary_to_tmem<KATOMS>(sm.stat, tlane, rowi);
       tc::mbar_arrive(&sm.bar_a_ready);
     };
     if (wg == 0) stage_stat(0);
     uint32_t rs[2][32], pd[32];
     Ring rst, rsl;
     int tcur = 0;                                     // global tile index the rings stand at
-    const bool bulk_out = (KD & 3) == 0 && !(dbg & 32);
+    const bool bulk_out = (KD & 3) == 0;
     for (int it = 0; it < my_items; ++it) {
       const int item = blockIdx.x + it * gridDim.x, bn = item / nqt, qt = item - bn * nqt, q0 = qt * CB_BM;
       const int qi = q0 + rowi;
@@ -759,7 +731,6 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dq_cc_kernel(
         const bool tail = nvalid < CB_BN;
         long long* const tw = (warp & 3) == 0 ? tl : nullptr;
         TL_STAMP(tw, 7, it * ntiles + j);
-        if (lane == 0) tc::hb(8 + warp, it * 1000 + j);
         tc::mbar_wait(&sm.bar_s_full[slot], rsl.ph);
         tc::tc_fence_after();
         TL_STAMP(tw, 8, it * ntiles + j);
@@ -770,48 +741,31 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dq_cc_kernel(
         tc::tmem_ld_x32(tslot + 32, rs[1]);
         TL_STAMP(tw, 9, it * ntiles + j);
         const uint32_t vt = smem_u32(sm.side[st]);
-        if (dbg & 9) {
-          tc::tmem_ld_wait();
-          tc::tmem_ld_landed(rs[1]);
-          if (dbg & 8) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) pd[i] = rs[0][i];
-          } else {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) pd[i] = tc::pack_bf16x2(__uint_as_float(rs[0][i]) * ndelta, __uint_as_float(rs[1][i]) * go[0]);
-          }
-        } else {
-          if (tail) dq_cc_chunk<DVH, true, 0>(rs[0], pd, vt, nvalid, go, ndelta);
-          else dq_cc_chunk<DVH, false, 0>(rs[0], pd, vt, nvalid, go, ndelta);
-          tc::tmem_ld_wait();
-          tc::tmem_ld_landed(rs[1]);
-          if (tail) dq_cc_chunk<DVH, true, 1>(rs[1], pd, vt, nvalid, go, ndelta);
-          else dq_cc_chunk<DVH, false, 1>(rs[1], pd, vt, nvalid, go, ndelta);
-        }
+        if (tail) dq_cc_chunk<DVH, true, 0>(rs[0], pd, vt, nvalid, go, ndelta);
+        else dq_cc_chunk<DVH, false, 0>(rs[0], pd, vt, nvalid, go, ndelta);
+        tc::tmem_ld_wait();
+        tc::tmem_ld_landed(rs[1]);
+        if (tail) dq_cc_chunk<DVH, true, 1>(rs[1], pd, vt, nvalid, go, ndelta);
+        else dq_cc_chunk<DVH, false, 1>(rs[1], pd, vt, nvalid, go, ndelta);
         TL_STAMP(tw, 10, it * ntiles + j);
         tc::tmem_st_x32(tslot, pd);                    // dS (bf16) over S'[0,32): all of S' is in registers
         tc::tmem_st_wait();
         tc::tc_fence_before();
         tc::mbar_arrive(&sm.bar_p_ready[slot]);
         tc::mbar_arrive(&sm.bar_empty[st]);            // value tile consumed
-        if (lane == 0) tc::hb(8 + warp, 500000 + it * 1000 + j);
         TL_STAMP(tw, 11, it * ntiles + j);
       }
       // ---- drain dQa (warpgroup 0 alone; the others go straight on with the next item's tiles, so the score slots are full
       //      again when the accumulator is released): TMEM -> shared staging tile -> one bulk store of nrows x KD floats ----
       if (wg == 0) {
         TL_STAMP(tl, 12, it * 4 + 0);
-        if (lane == 0) tc::hb(24 + warp, 1000 + it);
         if (it + 1 < my_items) {                       // single stationary buffer: refill once the item's score MMAs are done
           tc::mbar_wait(&sm.bar_s_done, it & 1);
           tc::tc_fence_after();
-          if (lane == 0) tc::hb(24 + warp, 2000 + it);
           stage_stat(it + 1);
         }
-        if (lane == 0) tc::hb(24 + warp, 3000 + it);
         tc::mbar_wait(&sm.bar_final, it & 1);
         tc::tc_fence_after();
-        if (lane == 0) tc::hb(24 + warp, 4000 + it);
         TL_STAMP(tl, 12, it * 4 + 1);
         if (bulk_out) {
           if (threadIdx.x == 0) bulk_wait_read();      // the previous item's store has finished reading the staging tile
@@ -836,7 +790,6 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dq_cc_kernel(
           tc::fence_proxy_async();
           asm volatile("bar.sync 1, 128;" ::: "memory");
           if (threadIdx.x == 0) bulk_s2g(dqa + ((size_t)bn * L + q0) * KD, sm.out, (uint32_t)(min(CB_BM, L - q0) * KD * 4));
-          if (lane == 0) tc::hb(24 + warp, 5000 + it);
           TL_STAMP(tl, 12, it * 4 + 3);
         } else {
           for (int c0 = 0; c0 < NQ; c0 += 32) {
@@ -861,22 +814,20 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dq_cc_kernel(
 }
 
 // ---- key-stationary: dK, dV ------------------------------------------------------------------------
-// TMEM: Ka buffers [0, QB*32K); slot s: S'^T at col_slot0 + 64 s (dS^T, bf16, over its first 32 columns); dK (32) behind the slots.
-// SS = 1: the stationary Ka tile stays in shared memory (SS-mode score MMAs, double-buffered by item parity); its TMEM columns
-// become score slots: 7 instead of 5 (the pipeline is bound by tiles in flight / chain latency, see cb_plan).
-template <int KATOMS, int DVH, int SS>
+// TMEM: Ka tile [0, 32K); slot s: S'^T at col_slot0 + 64 s (dS^T, bf16, over its first 32 columns); dK (32) behind the slots.
+template <int KATOMS, int DVH>
 __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dkv_cc_kernel(
     const __grid_constant__ CUtensorMap tm_k_stat, const __grid_constant__ CUtensorMap tm_q_strm,
     const float* __restrict__ v, const float* __restrict__ d_o, const float* __restrict__ delta, float* __restrict__ dk,
     float* __restrict__ dv, bf16* __restrict__ dqkvh, int KPq, int nh, int L, int dkh, int C1, int nqt, int nitems) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  typedef CbSmem<KATOMS, CB_BN * (DVH + 1), 0, DVH, SS ? 2 : 1> Smem;
+  typedef CbSmem<KATOMS, CB_BN * (DVH + 1), 0, DVH> Smem;
   Smem& sm = *reinterpret_cast<Smem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   constexpr int ST = Smem::ST;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int ntiles = (L + CB_BN - 1) / CB_BN;
   const int my_items = (nitems - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-  const CbPlan pl = cb_plan(KATOMS, 32, ST, ntiles, SS ? 0 : 1);
+  const CbPlan pl = cb_plan(KATOMS, 32, ST, ntiles);
   __shared__ float dv_xch[2][CB_NWG][CB_BM][DVH];       // dV partial of every tile class (j % 3), by item parity
 
   cb_init<KATOMS>(sm, warp, lane, &tm_k_stat, &tm_q_strm, nqt, v, DVH, nullptr, 0, L);
@@ -884,11 +835,11 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dkv_cc_kernel(
 
   if (warp == CB_W_TMA) {
     if (lane == 0)
-      cb_producer<KATOMS>(sm, &tm_k_stat, &tm_q_strm, d_o, DVH, delta, 1, v, DVH, nullptr, 0, L, nqt, ntiles, my_items, 0);
+      cb_producer<KATOMS>(sm, &tm_k_stat, &tm_q_strm, d_o, DVH, delta, 1, v, DVH, nullptr, 0, L, nqt, ntiles, my_items);
   } else if (warp == CB_W_S || warp == CB_W_S2) {
     cb_score_issuer<KATOMS>(sm, tmem, pl, C1 >> 4, ntiles, my_items, warp == CB_W_S ? 0 : 1);
   } else if (warp == CB_W_G) {
-    cb_grad_issuer<KATOMS>(sm, tmem, pl, tc::idesc_bf16_f32(CB_BM, 32) | (1u << 16), ntiles, my_items, 0);
+    cb_grad_issuer<KATOMS>(sm, tmem, pl, tc::idesc_bf16_f32(CB_BM, 32) | (1u << 16), ntiles, my_items);
   } else {
     const int wg = warp >> 2;
     const int rowi = (warp & 3) * 32 + lane;
@@ -896,10 +847,8 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dkv_cc_kernel(
     const int NS = pl.NS;
     auto stage_stat = [&](int it) {
       tc::mbar_wait(&sm.bar_stat, it & 1);
-      if (!SS) {
-        stationary_to_tmem<KATOMS>(sm.stat, tlane + (uint32_t)((it & (pl.QB - 1)) * KATOMS * 32), rowi);
-        tc::mbar_arrive(&sm.bar_a_ready);
-      }
+      stationary_to_tmem<KATOMS>(sm.stat, tlane, rowi);
+      tc::mbar_arrive(&sm.bar_a_ready);
     };
     if (wg == 0) stage_stat(0);
     uint32_t rs[2][32], pd[32];
@@ -910,7 +859,7 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dkv_cc_kernel(
       const int item = blockIdx.x + it * gridDim.x, bn = item / nqt, qt = item - bn * nqt, k0 = qt * CB_BM;
       const int kj = k0 + rowi;
       const size_t row = (size_t)bn * L + kj;
-      if (wg != 0 || SS) tc::mbar_wait(&sm.bar_stat, it & 1);   // this row's v came with the stationary tile
+      if (wg != 0) tc::mbar_wait(&sm.bar_stat, it & 1);   // this row's v came with the stationary tile
       float vk[DVH], dvacc[DVH];
 #pragma unroll
       for (int e = 0; e < DVH; ++e) { vk[e] = kj < L ? sm.rowside[it & 1][rowi * DVH + e] : 0.f; dvacc[e] = 0.f; }
@@ -953,7 +902,7 @@ __global__ void __launch_bounds__(CB_THREADS, 1) attn_bwd_dkv_cc_kernel(
       for (int e = 0; e < DVH; ++e) dv_xch[it & 1][cls][rowi][e] = dvacc[e];
       tc::mbar_arrive(&sm.bar_dv);
       if (wg > 0) continue;
-      if (!SS && it + 1 < my_items) {                  // single stationary TMEM buffer: refill once the item's score MMAs are done
+      if (it + 1 < my_items) {                         // single stationary TMEM buffer: refill once the item's score MMAs are done
         tc::mbar_wait(&sm.bar_s_done, it & 1);
         tc::tc_fence_after();
         stage_stat(it + 1);
@@ -1032,7 +981,7 @@ int launch_fwd_cc(const Dims& d, const AugLayout& a, const void* qa, const void*
   auto kern = attn_fwd_cc_kernel<KATOMS, DVH>;
   AACONV_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int nqt = cdiv(d.L, CF_BM), nitems = nqt * d.BN;
-  kern<<<std::min(nitems, sm_count()), CF_THREADS, smem, AACONV_ST(st)>>>(tq, tk, v, o, lse, d.L, a.C1, nqt, nitems, g_attn_dbg_mode);
+  kern<<<std::min(nitems, sm_count()), CF_THREADS, smem, AACONV_ST(st)>>>(tq, tk, v, o, lse, d.L, a.C1, nqt, nitems);
   AACONV_LAUNCH_OK("attn_fwd_cc");
   return 0;
 }
@@ -1043,7 +992,7 @@ int launch_bwd_dq_cc(const Dims& d, const AugLayout& a, const CUtensorMap& tq_st
   const size_t smem = sizeof(CbSmem<KATOMS, CB_BN * DVH, CB_BM * OUTW, DVH + 1>) + 1024;
   auto kern = attn_bwd_dq_cc_kernel<KATOMS, DVH, OUTW>;
   AACONV_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<grid, CB_THREADS, smem, AACONV_ST(st)>>>(tq_stat, tk_strm, v, d_o, delta, dqa, d.L, a.KD, a.NQ, a.C1, nqt, nitems, g_attn_dbg_mode, g_attn_dbg);
+  kern<<<grid, CB_THREADS, smem, AACONV_ST(st)>>>(tq_stat, tk_strm, v, d_o, delta, dqa, d.L, a.KD, a.NQ, a.C1, nqt, nitems, g_attn_dbg);
   AACONV_LAUNCH_OK("attn_bwd_dq_cc");
   return 0;
 }
@@ -1063,22 +1012,12 @@ int launch_bwd_cc(const Dims& d, const AugLayout& a, const void* qa, const void*
   AACONV_TRY(make_aug_map(d, qa, a.KP, CB_BN, &tq_strm));
   const int nqt = cdiv(d.L, CB_BM), nitems = nqt * d.BN;
   const int grid = std::min(nitems, sm_count());
-  static const bool dkv_ss = [] { const char* e = getenv("AACONV_DKV_SS"); return e ? atoi(e) != 0 : false; }();   // A/B (profiles/r02_attn_ab.md): SS mode measured slower (167 vs 162 us), default off
-  if (dkv_ss && KATOMS <= 2) {
-    const size_t smem = sizeof(CbSmem<KATOMS, CB_BN * (DVH + 1), 0, DVH, 2>) + 1024;
-    auto kern = attn_bwd_dkv_cc_kernel<KATOMS, DVH, 1>;
-    AACONV_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, CB_THREADS, smem, AACONV_ST(st)>>>(tk_stat, tq_strm, v, d_o, delta, dk, dv, static_cast<bf16*>(dqkvh), KPq, d.nh, d.L, d.dkh, a.C1,
-                                         nqt, nitems);
-    AACONV_LAUNCH_OK("attn_bwd_dkv_cc");
-  } else {
-    const size_t smem = sizeof(CbSmem<KATOMS, CB_BN * (DVH + 1), 0, DVH>) + 1024;
-    auto kern = attn_bwd_dkv_cc_kernel<KATOMS, DVH, 0>;
-    AACONV_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, CB_THREADS, smem, AACONV_ST(st)>>>(tk_stat, tq_strm, v, d_o, delta, dk, dv, static_cast<bf16*>(dqkvh), KPq, d.nh, d.L, d.dkh, a.C1,
-                                         nqt, nitems);
-    AACONV_LAUNCH_OK("attn_bwd_dkv_cc");
-  }
+  const size_t smem = sizeof(CbSmem<KATOMS, CB_BN * (DVH + 1), 0, DVH>) + 1024;
+  auto kern = attn_bwd_dkv_cc_kernel<KATOMS, DVH>;
+  AACONV_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<grid, CB_THREADS, smem, AACONV_ST(st)>>>(tk_stat, tq_strm, v, d_o, delta, dk, dv, static_cast<bf16*>(dqkvh), KPq, d.nh, d.L, d.dkh, a.C1,
+                                                  nqt, nitems);
+  AACONV_LAUNCH_OK("attn_bwd_dkv_cc");
   typedef CcOutw<KATOMS> W;
   if (a.KD <= W::MID) return launch_bwd_dq_cc<KATOMS, DVH, W::MID>(d, a, tq_stat, tk_strm, v, d_o, delta, dqa, nqt, nitems, grid, st);
   return launch_bwd_dq_cc<KATOMS, DVH, W::MAX>(d, a, tq_stat, tk_strm, v, d_o, delta, dqa, nqt, nitems, grid, st);
@@ -1109,7 +1048,7 @@ bool cc_smem_fits(int KD) {
                         ? smem_fits(attn_bwd_dq_cc_kernel<KATOMS, DVH, W::MID>, sizeof(CbSmem<KATOMS, CB_BN * DVH, CB_BM * W::MID, DVH + 1>) + 1024)
                         : smem_fits(attn_bwd_dq_cc_kernel<KATOMS, DVH, W::MAX>, sizeof(CbSmem<KATOMS, CB_BN * DVH, CB_BM * W::MAX, DVH + 1>) + 1024);
     r = dq && smem_fits(attn_fwd_cc_kernel<KATOMS, DVH>, sizeof(CfSmem<KATOMS, DVH>) + 1024) &&
-        smem_fits(attn_bwd_dkv_cc_kernel<KATOMS, DVH, 0>, sizeof(CbSmem<KATOMS, CB_BN * (DVH + 1), 0, DVH>) + 1024);
+        smem_fits(attn_bwd_dkv_cc_kernel<KATOMS, DVH>, sizeof(CbSmem<KATOMS, CB_BN * (DVH + 1), 0, DVH>) + 1024);
   }
   return r;
 }
@@ -1129,16 +1068,9 @@ int cc_attn_supported(const Dims& d) {
   return 0;
 }
 
-// ablation (tools/attn_ablate.py; results are WRONG): AACONV_ABL_NKS = score k-steps, AACONV_ABL_NQ = width of the dQa accumulator
-static AugLayout ablated(AugLayout a) {
-  if (const char* e = getenv("AACONV_ABL_NKS")) a.C1 = 16 * atoi(e);
-  if (const char* e = getenv("AACONV_ABL_NQ")) a.NQ = atoi(e);
-  return a;
-}
-
 int cc_attn_fwd(const Dims& d, const void* qa, const void* ka, const float* v, float* o, float* lse, cudaStream_t st) {
   AACONV_TRY(cc_attn_supported(d));
-  const AugLayout a = ablated(aug_layout(d));
+  const AugLayout a = aug_layout(d);
   const int K = a.KP / 64;
   if (d.dvh == 1) {
     if (K == 1) return launch_fwd_cc<1, 1>(d, a, qa, ka, v, o, lse, st);
@@ -1153,7 +1085,7 @@ int cc_attn_fwd(const Dims& d, const void* qa, const void* ka, const float* v, f
 int cc_attn_bwd(const Dims& d, const void* qa, const void* ka, const float* v, const float* d_o, const float* delta, float* dqa,
                 float* dk, float* dv, void* dqkvh, int KPq, cudaStream_t st) {
   AACONV_TRY(cc_attn_supported(d));
-  const AugLayout a = ablated(aug_layout(d));
+  const AugLayout a = aug_layout(d);
   const int K = a.KP / 64;
   if (d.dvh == 1) {
     if (K == 1) return launch_bwd_cc<1, 1>(d, a, qa, ka, v, d_o, delta, dqa, dk, dv, dqkvh, KPq, st);

@@ -1,7 +1,6 @@
 // Operand builders and relative-logit adjoints around the tcgen05 attention kernels (bf16 path).
 //
 //   aug_build_fwd   q,k,v (fp32, head-split) -> augmented bf16 operands Qa, Ka (layout in attn_tc_bwd.cu)
-//   aug_patch_bwd   fills the backward-only columns of Qa in place: -lse (hi/lo), dO, -delta (hi/lo), delta = dO.o
 //   rel_bwd         dQa -> total dq (content + relative part) written as bf16 into the packed dqkv operand of the
 //                   projection GEMMs, and the key_rel_w / key_rel_h gradients
 //
@@ -15,7 +14,6 @@
 //   dq_rel    [rows x dkh]     = dR[rows x 2N-1] . T^T                      dR[row, r] = dAq[row, r + x - (N-1)]
 //   dT^T      [2N-1 x dkh]    += dR^T[2N-1 x rows] . Q[rows x dkh]          (accumulated in registers, fixed order)
 #include <algorithm>
-#include <cstdlib>
 #include <cuda_bf16.h>
 #include "tc_common.cuh"
 #include "bf16_path.cuh"
@@ -250,38 +248,13 @@ __global__ void __launch_bounds__(256) aug_build_fwd_kernel(const BuildP p) {
   }
 }
 
-// ------------------------------------------------------------------------------------------------
-// backward patch of Qa
-// ------------------------------------------------------------------------------------------------
-__global__ void aug_patch_bwd_kernel(const float* __restrict__ lse, const float* __restrict__ d_o,
-                                     const float* __restrict__ o, bf16* __restrict__ qa, float* __restrict__ delta_out,
-                                     size_t rows, int dvh, int KD, int C1, int KP) {
-  const size_t row = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= rows) return;
-  bf16* dst = qa + row * KP;
-  bf16 hi, lo;
-  split_bf16(-lse[row] * LOG2E, hi, lo);
-  dst[KD] = hi;
-  dst[KD + 1] = lo;
-  float delta = 0.f;
-  for (int e = 0; e < dvh; ++e) {
-    const float g = d_o[row * dvh + e];
-    delta = fmaf(g, o[row * dvh + e], delta);
-    dst[C1 + e] = __float2bfloat16(g);
-  }
-  split_bf16(-delta, hi, lo);
-  dst[C1 + dvh] = hi;
-  dst[C1 + dvh + 1] = lo;
-  delta_out[row] = delta;
-}
-
 constexpr int OBP_THREADS = 128;   // 25600 pixels at Transition 1 -> 200 CTAs (256 threads left 48 of 148 SMs idle)
 // ------------------------------------------------------------------------------------------------
 // out_proj adjoint + backward patch of Qa in ONE pass over the pixels (small value widths: dv = NH * DVH <= 16)
 //   dO[b,n,l,e] = sum_c Wout[c, n*dvh+e] dy[b, Cc+c, l]        (attn_aug_conv.py:92 adjoint, data)
 //   dWout[c,j] += dy[b, Cc+c, l] * o[b, n(j), l, e(j)]          (weight; per-block partials, summed in block order by
 //                                                                out_w_reduce_kernel: deterministic)
-//   delta[b,n,l] = dO . o;  Qa columns -lse (hi/lo), dO, -delta (hi/lo) as in aug_patch_bwd_kernel
+//   delta[b,n,l] = dO . o;  the backward-only columns of Qa: -lse (hi/lo), dO, -delta (hi/lo)
 // Replaces four launches (out_bwd_data, out_bwd_weight, splitk_reduce, aug_patch_bwd: 56 us at Transition 1) whose
 // work is 25600 pixels x 8 channels.
 // ------------------------------------------------------------------------------------------------
@@ -471,9 +444,7 @@ size_t aug_build_smem(const Dims& d) {
 int aug_build_fwd(const Dims& d, const float* q, const float* k, const float* v, const float* krw, const float* krh,
                   void* qa, void* ka, cudaStream_t st) {
   AACONV_TRY(aug_supported(d));
-  // AACONV_AUG_BUILD=legacy keeps the mma.sync builder (A/B runs, tools/aug_ab.py)
-  static const bool legacy = [] { const char* e = getenv("AACONV_AUG_BUILD"); return e && e[0] == 'l'; }();
-  if (!legacy && aug_build_tc_supported(d) == 0) return aug_build_tc(d, q, k, v, krw, krh, qa, ka, st);
+  if (aug_build_tc_supported(d) == 0) return aug_build_tc(d, q, k, v, krw, krh, qa, ka, st);
   const AugLayout a = aug_layout(d);
   BuildP p;
   p.q = q; p.k = k; p.v = v; p.krw = krw; p.krh = krh;
@@ -489,15 +460,6 @@ int aug_build_fwd(const Dims& d, const float* q, const float* k, const float* v,
   const int grid = std::min(p.ntiles, 148 * per_sm);
   aug_build_fwd_kernel<<<grid, 256, smem, AACONV_ST(st)>>>(p);
   AACONV_LAUNCH_OK("aug_build_fwd");
-  return 0;
-}
-
-int aug_patch_bwd(const Dims& d, const float* lse, const float* d_o, const float* o, void* qa, float* delta, cudaStream_t st) {
-  const AugLayout a = aug_layout(d);
-  const size_t rows = (size_t)d.BN * d.L;
-  const unsigned grid = (unsigned)((rows + 255) / 256);
-  aug_patch_bwd_kernel<<<grid, 256, 0, AACONV_ST(st)>>>(lse, d_o, o, static_cast<bf16*>(qa), delta, rows, d.dvh, a.KD, a.C1, a.KP);
-  AACONV_LAUNCH_OK("aug_patch_bwd");
   return 0;
 }
 
@@ -911,9 +873,7 @@ size_t rel_bwd_partial_floats(const Dims& d) {
 int rel_bwd(const Dims& d, const float* dqa, const float* q, const float* krw, const float* krh, float* dq, void* dqkvh,
             int KPq, float* dkrw, float* dkrh, float* partial, cudaStream_t st) {
   AACONV_TRY(rel_bwd_supported(d));
-  // AACONV_REL_BWD=legacy keeps the mma.sync kernel (A/B runs, tools/stage_ab.py)
-  static const bool legacy = [] { const char* e = getenv("AACONV_REL_BWD"); return e && e[0] == 'l'; }();
-  if (!legacy && !dq && dqkvh && rel_bwd_tc_supported(d, KPq) == 0) {
+  if (!dq && dqkvh && rel_bwd_tc_supported(d, KPq) == 0) {
     const int RP = cdiv(std::max(d.RW, d.RH), 16) * 16, DK8 = cdiv(d.dkh, 8) * 8;
     int nparts = 0;
     AACONV_TRY(rel_bwd_tc(d, dqa, q, krw, krh, dqkvh, KPq, partial, RP, DK8, &nparts, st));

@@ -10,7 +10,6 @@
 // TMA tensor stores.  Persistent CTAs: TMA warp (q tiles), MMA warp (two TMEM accumulator buffers), one or two epilogue warpgroups.
 // Reference rows a4-a6 (attn_aug_conv.py:55-63,77-86).
 #include <algorithm>
-#include <cstdlib>
 #include "tc_common.cuh"
 #include "bf16_path.cuh"
 
@@ -105,7 +104,7 @@ template <int W, int H, int DKH>
 __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_kernel(
     const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_qa, const __grid_constant__ CUtensorMap tm_ka,
     const float* __restrict__ kg, const float* __restrict__ vg, const float* __restrict__ krw, const float* __restrict__ krh,
-    int L, int dvh, int tiles_per_bn, int ntiles, int dbg) {
+    int L, int dvh, int tiles_per_bn, int ntiles, uint32_t dep_zero /* always 0: see tc::mbar_arrive_after */) {
   typedef AbCfg<W, H, DKH> C;
   typedef AbSmem<C> Smem;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -167,7 +166,6 @@ __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_ker
         const int tile = blockIdx.x + i * gridDim.x, bn = tile / tiles_per_bn, l0 = (tile - bn * tiles_per_bn) * AB_BM;
         const int s = i % ST;
         tc::mbar_wait(&sm.bar_empty[s], ((i / ST) & 1) ^ 1);
-        if (dbg & 16) { tc::mbar_arrive(&sm.bar_full[s]); continue; }   // ablation: no q loads
         tc::mbar_arrive_expect_tx(&sm.bar_full[s], AB_BM * 128);
         tc::tma_load_3d(sm.q[s], &tm_q, &sm.bar_full[s], 0, l0, bn);
       }
@@ -184,12 +182,10 @@ __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_ker
       if (tc::elect_one()) {
         const uint32_t a = tc::desc_lo_k(smem_u32(sm.q[s]));
         const uint32_t d0 = tmem + buf * C::TCOLS;
-        if (!(dbg & 32)) {
 #pragma unroll
-          for (int ks = 0; ks < C::KSTEPS; ++ks) mma_ss_tf32(d0, tc::desc64(a + ks * 2), tc::desc64(bw + ks * 2), idw, ks > 0);
+        for (int ks = 0; ks < C::KSTEPS; ++ks) mma_ss_tf32(d0, tc::desc64(a + ks * 2), tc::desc64(bw + ks * 2), idw, ks > 0);
 #pragma unroll
-          for (int ks = 0; ks < C::KSTEPS; ++ks) mma_ss_tf32(d0 + C::NW, tc::desc64(a + ks * 2), tc::desc64(bh + ks * 2), idh, ks > 0);
-        }
+        for (int ks = 0; ks < C::KSTEPS; ++ks) mma_ss_tf32(d0 + C::NW, tc::desc64(a + ks * 2), tc::desc64(bh + ks * 2), idh, ks > 0);
         tc::mma_commit(&sm.bar_tfull[buf]);
       }
       __syncwarp();
@@ -214,7 +210,7 @@ __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_ker
       float kf[DKH];
 #pragma unroll
       for (int e = 0; e < DKH; e += 4) {
-        const float4 t4 = (dbg & 8) ? make_float4(0.f, 0.f, 0.f, 0.f) : __ldg(reinterpret_cast<const float4*>(kg + grow * DKH + e));
+        const float4 t4 = __ldg(reinterpret_cast<const float4*>(kg + grow * DKH + e));
         kf[e] = t4.x; kf[e + 1] = t4.y; kf[e + 2] = t4.z; kf[e + 3] = t4.w;
       }
       float vf[14];
@@ -224,14 +220,8 @@ __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_ker
       tc::mbar_wait(&sm.bar_tfull[buf], (i >> 1) & 1);
       tc::tc_fence_after();
       uint32_t aq[W / 2], bq[H / 2];
-      if (dbg & 2) {
-#pragma unroll
-        for (int j = 0; j < W / 2; ++j) aq[j] = j;
-#pragma unroll
-        for (int j = 0; j < H / 2; ++j) bq[j] = j;
-      }
       // ---- W axis: R_w row -> private shared row (bf16) -> window [W-1-x, 2W-1-x) ----
-      if (!(dbg & 2)) {
+      {
         const uint32_t tcol = tlane + buf * C::TCOLS;
 #pragma unroll
         for (int b0 = 0; b0 < C::NW; b0 += 64) {            // at most 64 columns in flight (registers)
@@ -254,7 +244,7 @@ __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_ker
         for (int j = 0; j < W / 2; ++j) aq[j] = __funnelshift_r(wd[j], wd[j + 1], fs);
       }
       // ---- H axis ----
-      if (!(dbg & 2)) {
+      {
         const uint32_t tcol = tlane + buf * C::TCOLS + C::NW;
 #pragma unroll
         for (int b0 = 0; b0 < C::NH; b0 += 64) {
@@ -294,7 +284,7 @@ __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_ker
         uint32_t fold = 0u;
 #pragma unroll
         for (int c = 0; c < DKH / 2; ++c) fold ^= qp[c];
-        tc::mbar_arrive_after(&sm.bar_empty[s], fold & ((uint32_t)dbg & 0x40000000u));
+        tc::mbar_arrive_after(&sm.bar_empty[s], fold & dep_zero);
       }
       // ---- Qa row: [ c q | c Aq | c Bq | 0 (lse slots, backward) | 0 .. ] -> staging tile -> TMA store ----
       if (leader) bulk_wait_read0();                 // the previous tile's Ka store has finished READING the staging tile
@@ -309,11 +299,11 @@ __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_ker
 #pragma unroll
       for (int ch = 0; ch < C::KP / 8; ++ch) {
         const uint32_t dst = stg0 + (ch >> 3) * (AB_BM * 128) + ((((uint32_t)ch & 7) ^ swz) << 4);
-        if (!(dbg & 4)) sts128(dst, qa_word(4 * ch), qa_word(4 * ch + 1), qa_word(4 * ch + 2), qa_word(4 * ch + 3));
+        sts128(dst, qa_word(4 * ch), qa_word(4 * ch + 1), qa_word(4 * ch + 2), qa_word(4 * ch + 3));
       }
       tc::fence_proxy_async();
       wg_sync();
-      if (leader && !(dbg & 1)) {
+      if (leader) {
 #pragma unroll
         for (int a = 0; a < C::KATOMS; ++a) tma_store_3d(&tm_qa, sm.stg[wg][a], a * 64, l0, bn);
         bulk_commit();
@@ -343,11 +333,11 @@ __global__ void __launch_bounds__(AbCfg<W, H, DKH>::THREADS, 1) aug_build_tc_ker
 #pragma unroll
       for (int ch = 0; ch < C::KP / 8; ++ch) {
         const uint32_t dst = stg0 + (ch >> 3) * (AB_BM * 128) + ((((uint32_t)ch & 7) ^ swz) << 4);
-        if (!(dbg & 4)) sts128(dst, kw[4 * ch], kw[4 * ch + 1], kw[4 * ch + 2], kw[4 * ch + 3]);
+        sts128(dst, kw[4 * ch], kw[4 * ch + 1], kw[4 * ch + 2], kw[4 * ch + 3]);
       }
       tc::fence_proxy_async();
       wg_sync();
-      if (leader && !(dbg & 1)) {
+      if (leader) {
 #pragma unroll
         for (int a = 0; a < C::KATOMS; ++a) tma_store_3d(&tm_ka, sm.stg[wg][a], a * 64, l0, bn);
         bulk_commit();
@@ -390,8 +380,7 @@ int launch_aug_build_tc(const Dims& d, const float* q, const float* k, const flo
   auto kern = aug_build_tc_kernel<W, H, DKH>;
   AACONV_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int tiles_per_bn = cdiv(d.L, AB_BM), ntiles = tiles_per_bn * d.BN;
-  static const int dbg = [] { const char* e = getenv("AACONV_AB_DBG"); return e ? atoi(e) : 0; }();   // ablation bits (results wrong)
-  kern<<<std::min(ntiles, sm_count_ab()), C::THREADS, smem, AACONV_ST(st)>>>(tq, tqa, tka, k, v, krw, krh, d.L, d.dvh, tiles_per_bn, ntiles, dbg);
+  kern<<<std::min(ntiles, sm_count_ab()), C::THREADS, smem, AACONV_ST(st)>>>(tq, tqa, tka, k, v, krw, krh, d.L, d.dvh, tiles_per_bn, ntiles, 0u);
   AACONV_LAUNCH_OK("aug_build_tc");
   return 0;
 }
@@ -492,7 +481,8 @@ template <int W, int H, int DKH>
 __global__ void __launch_bounds__(192, 1) rel_bwd_tc_kernel(const float* __restrict__ dqa, const float* __restrict__ qg,
                                                             const float* __restrict__ krw, const float* __restrict__ krh,
                                                             bf16* __restrict__ dqkvh, float* __restrict__ partial, int L, int nh,
-                                                            int KPq, int RP, int DK8, float qscale, int tiles_per_bn, int ntiles, int dbg) {
+                                                            int KPq, int RP, int DK8, float qscale, int tiles_per_bn, int ntiles,
+                                                            uint32_t dep_zero /* always 0: see tc::mbar_arrive_after */) {
   typedef RbCfg<W, H, DKH> C;
   typedef RbSmem<C> Smem;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -512,7 +502,7 @@ __global__ void __launch_bounds__(192, 1) rel_bwd_tc_kernel(const float* __restr
     tc::mbar_init(&sm.bar_a_ready, 128);
     tc::mbar_init(&sm.bar_done, 1);
     tc::fence_barrier_init();
-    for (int i = 0; i < ST && i < my_tiles && !(dbg & 4); ++i) {
+    for (int i = 0; i < ST && i < my_tiles; ++i) {
       int bn, l0;
       const int nrows = tile_rows(i, bn, l0);
       tc::mbar_arrive_expect_tx(&sm.bar_full[i], nrows * C::KD * 4);
@@ -555,10 +545,10 @@ __global__ void __launch_bounds__(192, 1) rel_bwd_tc_kernel(const float* __restr
 
   if (warp == 4) {
     if (lane == 0) {
-      for (int i = (dbg & 4) ? 0 : ST; i < my_tiles; ++i) {
+      for (int i = ST; i < my_tiles; ++i) {
         int bn, l0;
         const int nrows = tile_rows(i, bn, l0), s = i % ST;
-        if (i >= ST) tc::mbar_wait(&sm.bar_empty[s], ((i / ST) & 1) ^ 1);
+        tc::mbar_wait(&sm.bar_empty[s], ((i / ST) & 1) ^ 1);
         tc::mbar_arrive_expect_tx(&sm.bar_full[s], nrows * C::KD * 4);
         bulk_g2s_1d(sm.in[s], dqa + ((size_t)bn * L + l0) * C::KD, nrows * C::KD * 4, &sm.bar_full[s]);
       }
@@ -591,7 +581,6 @@ __global__ void __launch_bounds__(192, 1) rel_bwd_tc_kernel(const float* __restr
   } else {
     // ===================== row owners =====================
     const int r = threadIdx.x;
-    const uint32_t zmask = (uint32_t)dbg & 0x40000000u;          // 0 at run time; the compiler cannot know
     const uint32_t tlane = tmem + ((uint32_t)(warp * 32) << 16);
     const uint32_t swz = (uint32_t)(r & 7);
     const uint32_t arow = smem_u32(sm.a[0]) + r * 128, qrow = smem_u32(sm.qt) + r * 128;
@@ -599,7 +588,6 @@ __global__ void __launch_bounds__(192, 1) rel_bwd_tc_kernel(const float* __restr
     bf16* dst_prev = nullptr;
     auto finish_prev = [&](int iprev) {              // D1 of tile iprev -> dq_total -> bf16 store
       tc::mbar_wait(&sm.bar_done, iprev & 1);
-      if (dbg & 1) { const long long t0 = clock64(); while (clock64() - t0 < 3000) {} }
       tc::tc_fence_after();
       uint32_t d1[32];
       tc::tmem_ld_x32(tlane + COL_D1, d1);
@@ -649,7 +637,7 @@ __global__ void __launch_bounds__(192, 1) rel_bwd_tc_kernel(const float* __restr
         for (int j = 1; j <= W / 2; ++j) fold ^= pa[j];
 #pragma unroll
         for (int j = 1; j <= H / 2; ++j) fold ^= pb[j];
-        tc::mbar_arrive_after(&sm.bar_empty[s], fold & zmask);
+        tc::mbar_arrive_after(&sm.bar_empty[s], fold & dep_zero);
       }
       // ---- the previous tile's products are done: its D1 leaves, and the A / q tiles may be rewritten ----
       if (i > 0) finish_prev(i - 1);
@@ -692,7 +680,6 @@ __global__ void __launch_bounds__(192, 1) rel_bwd_tc_kernel(const float* __restr
         sts128(qrow + (((uint32_t)ch ^ swz) << 4), w4[0], w4[1], w4[2], w4[3]);
       }
       tc::fence_proxy_async();
-      if (dbg & 2) asm volatile("bar.sync 2, 128;" ::: "memory");
       tc::mbar_arrive(&sm.bar_a_ready);
     }
     if (my_tiles > 0) {
@@ -731,9 +718,8 @@ int launch_rel_bwd_tc(const Dims& d, const float* dqa, const float* q, const flo
   AACONV_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int tiles_per_bn = cdiv(d.L, AB_BM), ntiles = tiles_per_bn * d.BN;
   const int grid = std::min(ntiles, sm_count_ab());
-  static const int dbg = [] { const char* e = getenv("AACONV_RB_DBG"); return e ? atoi(e) : 0; }();   // debugging experiments
   kern<<<grid, 192, smem, AACONV_ST(st)>>>(dqa, q, krw, krh, static_cast<bf16*>(dqkvh), partial, d.L, d.nh, KPq, RP, DK8, d.qscale,
-                                           tiles_per_bn, ntiles, dbg);
+                                           tiles_per_bn, ntiles, 0u);
   AACONV_LAUNCH_OK("rel_bwd_tc");
   *grid_out = grid;
   return 0;

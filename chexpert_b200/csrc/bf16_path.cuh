@@ -28,8 +28,7 @@ int rel_bwd_tc(const Dims& d, const float* dqa, const float* q, const float* krw
 int rel_bwd_reduce(const Dims& d, const float* partial, int nparts, int RP, int DK8, float* dkrw, float* dkrh, cudaStream_t st);
 // (B,nh,L,L) softmax map from the bf16 operands and the bf16 forward kernel's lse (visualise path)
 int aug_weights(const Dims& d, const void* qa, const void* ka, const float* lse, float* weights, cudaStream_t st);
-int aug_patch_bwd(const Dims& d, const float* lse, const float* d_o, const float* o, void* qa, float* delta, cudaStream_t st);
-// out_proj adjoint (dO, dWout) + the patch above in one pass (nh = 8, dv/nh <= 2); partial: out_bwd_patch_partial_floats
+// out_proj adjoint (dO, dWout) + the backward-only columns of Qa (-lse, dO, -delta) in one pass (nh = 8, dv/nh <= 2); partial: out_bwd_patch_partial_floats
 int out_bwd_patch_supported(const Dims& d);
 size_t out_bwd_patch_partial_floats(const Dims& d);
 int out_bwd_patch(const Dims& d, const float* dy, const float* o, const float* lse, const float* wout, float* d_o, float* delta,

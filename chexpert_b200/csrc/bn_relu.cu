@@ -21,7 +21,6 @@
 //   eval      bn_eval    grid (C, G): BatchNorm2d in eval mode, relu(x s + t) from the running statistics, the apply loop of bn_apply
 //                        (aaconv_bn_relu_eval's NCHW -> NCHW variant: stem norm0, norm5, layers the channels-last tiles cannot take)
 #include <algorithm>
-#include <cstdlib>
 #include <cuda_bf16.h>
 #include "common.cuh"
 
@@ -359,12 +358,12 @@ __global__ void __launch_bounds__(256) bn_bwd_dx_kernel(const T* __restrict__ x,
 }
 
 // host: group size, thread layout and whether every plane of every tensor can be accessed four elements at a time
+constexpr int kBnTarget = 8192;   // elements per CTA
 template <class T>
 Geo make_geo(int B, int C, int HW, long long xbs, const void* p0, const void* p1, const void* p2) {
   Geo g;
   g.B = B; g.HW = HW; g.xbs = xbs;
-  static const int target = [] { const char* e = getenv("AACONV_BN_TARGET"); return e ? atoi(e) : 8192; }();   // elements per CTA (A/B)
-  g.bpb = std::max(1, std::min(B, target / std::max(HW, 1)));
+  g.bpb = std::max(1, std::min(B, kBnTarget / std::max(HW, 1)));
   g.G = (B + g.bpb - 1) / g.bpb;
   const size_t al = sizeof(T) * 4;                        // bytes of one four-element access (16 for fp32, 8 for bf16)
   const uintptr_t bits = reinterpret_cast<uintptr_t>(p0) | reinterpret_cast<uintptr_t>(p1) | reinterpret_cast<uintptr_t>(p2) |

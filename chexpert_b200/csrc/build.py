@@ -12,12 +12,10 @@ from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SOURCES = ['api.cu', 'runtime.cu', 'prologue.cu', 'bn_relu.cu', 'bn_cl.cu', 'fp32_gemms.cu', 'fp32_attn.cu', 'fp32_path.cu', 'bce.cu', 'eval_ops.cu', 'bf16_path.cu', 'tc_host.cu', 'aug_ops.cu', 'aug_tc.cu', 'attn_tc.cu', 'attn_cc.cu', 'attn_tc_bwd.cu', 'gemm_tc.cu', 'prep.cu', 'cam.cu']
-LIB = os.path.join(HERE, os.environ.get('AACONV_BUILD_NAME', 'libaaconv_b200.so'))
-EXTRA = os.environ.get('AACONV_BUILD_FLAGS', '').split()     # experiment variants: AACONV_BUILD_NAME=libx.so AACONV_BUILD_FLAGS='-DAACONV_CF_NWG=4'
-NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
-FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
-         '-Xcompiler', '-fPIC', '--use_fast_math=false', '-Xptxas', '-v']
-FLAGS = [f for f in FLAGS if f != '--use_fast_math=false']
+LIB = os.path.join(HERE, 'libaaconv_b200.so')
+BUILD_DIR = os.path.join(HERE, 'build')
+NVCC = '/usr/local/cuda/bin/nvcc'
+FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '-Xcompiler', '-fPIC', '-Xptxas', '-v']
 
 
 def _digest():
@@ -31,18 +29,17 @@ def _digest():
 
 
 def build(force=False, verbose=True):
-    bdir = 'build' if not EXTRA else 'build_' + os.path.basename(LIB)
-    stamp = os.path.join(HERE, bdir, 'stamp')
+    stamp = os.path.join(BUILD_DIR, 'stamp')
     dig = _digest()
     if not force and os.path.exists(LIB) and os.path.exists(stamp) and open(stamp).read() == dig:
         return LIB
-    os.makedirs(os.path.join(HERE, bdir), exist_ok=True)
+    os.makedirs(BUILD_DIR, exist_ok=True)
 
     def cc(src):
-        obj = os.path.join(HERE, bdir, src.replace('.cu', '.o'))
-        cmd = [NVCC, *FLAGS, *EXTRA, '-c', os.path.join(HERE, src), '-o', obj]
+        obj = os.path.join(BUILD_DIR, src.replace('.cu', '.o'))
+        cmd = [NVCC, *FLAGS, '-c', os.path.join(HERE, src), '-o', obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
-        log = os.path.join(HERE, bdir, src + '.log')
+        log = os.path.join(BUILD_DIR, src + '.log')
         open(log, 'w').write(r.stdout + r.stderr)
         if r.returncode:
             raise RuntimeError(f'nvcc failed for {src}:\n{r.stdout}\n{r.stderr}')

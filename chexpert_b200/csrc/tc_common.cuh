@@ -38,7 +38,11 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 // are asynchronous (only a later USE of their destination registers waits for them), the arrive is not ordered behind them,
 // and the producer's TMA write may then overwrite the stage while the last loads are still queued -- seen as run-to-run
 // differences in the last-loaded 16-byte chunks of rel_bwd_tc's rows (single-stage configuration, 512 px).
-// dep_zero = (xor of the loaded registers) & zmask with zmask == 0 at run time but unknown to the compiler.
+// dep_zero = (xor of the loaded registers) & zmask with zmask == 0 at run time but unknown to the compiler.  The kernels that
+// use it (aug_build_tc_kernel, rel_bwd_tc_kernel) take zmask as their last argument, `uint32_t dep_zero`, which every launch
+// passes as 0.  It must stay a kernel argument: with a literal 0 (or anything else the compiler can prove is 0) the fold is
+// deleted and the arrive issues right after the last ld.shared again; as a parameter it reaches the arrive's operand through
+// a LOP3 of the loaded registers and the parameter (cuobjdump -sass: LOP3.LUT -> VIADD -> SYNCS.ARRIVE.TRANS64).
 __device__ __forceinline__ void mbar_arrive_after(uint64_t* bar, uint32_t dep_zero) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(1u + dep_zero) : "memory");
 }
@@ -59,9 +63,7 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
 // Bounded wait: a protocol bug traps (-> launch error at the next sync) instead of hanging the GPU.  In "soft" mode
 // (aaconv_debug_set_mode bit 16; debugging only) a timed-out wait is logged to a device buffer and treated as satisfied, so
 // the kernel ends and the host can read WHICH barriers were stuck (aaconv_debug_read_mbar_log).
-#ifndef AACONV_MBAR_SPIN_LIMIT
-#define AACONV_MBAR_SPIN_LIMIT (1u << 26)
-#endif
+constexpr uint32_t MBAR_SPIN_LIMIT = 1u << 26;
 static __device__ unsigned long long* g_mbar_log = nullptr;   // mapped pinned host memory: [0] = count, [1..64] = records
 static __device__ unsigned g_mbar_soft = 0;                   // (survives a later fault of the kernel)
 static __device__ __noinline__ void mbar_timeout(uint32_t bar, uint32_t parity) {
@@ -75,19 +77,10 @@ static __device__ __noinline__ void mbar_timeout(uint32_t bar, uint32_t parity) 
          bar, parity);
   __trap();
 }
-// debugging heartbeat (soft mode only): last position of a role of CTA 0, readable after a fault
-// (compiled in with -DAACONV_DEBUG_HB only: the flag test is a global load per call)
-__device__ __forceinline__ void hb(int slot, unsigned long long v) {
-#ifdef AACONV_DEBUG_HB
-  if (g_mbar_soft && g_mbar_log && blockIdx.x == 0) reinterpret_cast<volatile unsigned long long*>(g_mbar_log)[1 + slot] = v;
-#else
-  (void)slot; (void)v;
-#endif
-}
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   uint32_t spins = 0;
   while (!mbar_try_wait(bar, parity)) {
-    if ((++spins & 0xFFFFFu) == 0 && (spins >= AACONV_MBAR_SPIN_LIMIT || g_mbar_soft)) {   // flag read once per 2^20 polls
+    if ((++spins & 0xFFFFFu) == 0 && (spins >= MBAR_SPIN_LIMIT || g_mbar_soft)) {   // flag read once per 2^20 polls
       mbar_timeout(smem_u32(bar), parity);
       break;
     }
@@ -99,7 +92,7 @@ __device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity
   uint32_t spins = 0;
   while (!mbar_try_wait(bar, parity)) {
     __nanosleep(40);
-    if (++spins > (AACONV_MBAR_SPIN_LIMIT >> 4)) { mbar_timeout(smem_u32(bar), parity); break; }
+    if (++spins > (MBAR_SPIN_LIMIT >> 4)) { mbar_timeout(smem_u32(bar), parity); break; }
   }
 }
 
@@ -247,13 +240,6 @@ __device__ __forceinline__ void issue_ts_ksteps(uint32_t d_main, uint32_t d_extr
     mma_ts(d_main, a_tmem + ks * 8, desc64(b_lo + (ks >> 2) * B_ATOM + (ks & 3) * 2), idesc, ks > 0 ? 1u : 0u);
   if (EXTRA) mma_ts(d_extra, a_tmem + NKS * 8, desc64(b_lo + (NKS >> 2) * B_ATOM + (NKS & 3) * 2), idesc, 0u);
 }
-// the same with A in shared memory (K-major, 64-column atoms A_ATOM descriptor units apart)
-template <int NKS, uint32_t A_ATOM, uint32_t B_ATOM>
-__device__ __forceinline__ void issue_ss_ksteps(uint32_t d_main, uint32_t a_lo, uint32_t b_lo, uint32_t idesc) {
-#pragma unroll
-  for (int ks = 0; ks < NKS; ++ks)
-    mma_ss(d_main, desc64(a_lo + (ks >> 2) * A_ATOM + (ks & 3) * 2), desc64(b_lo + (ks >> 2) * B_ATOM + (ks & 3) * 2), idesc, ks > 0 ? 1u : 0u);
-}
 template <int EXTRA, uint32_t B_ATOM>
 __device__ __forceinline__ void issue_ts_ksteps_n(int nks, uint32_t d_main, uint32_t d_extra, uint32_t a_tmem, uint32_t b_lo, uint32_t idesc) {
   switch (nks) {   // warp-uniform
@@ -294,28 +280,6 @@ __device__ __forceinline__ float ex2f(float x) {
   return y;
 }
 
-// 2^x on the FMA / ALU pipes (no MUFU): round-to-nearest split x = n + f, f in [-0.5, 0.5], degree-3 minimax polynomial for
-// 2^f (max relative error 7.5e-5, far inside the bf16 budget of everything these exponentials feed), exponent added in the
-// integer domain -- the FlashAttention-4 trick for loops bound by MUFU.EX2 (16 / clk / SM).  x is clamped at -126 (result
-// 2^-126 instead of 0: these terms are sums' far tails); callers guarantee x < 127.
-// MEASURED (B200, T1, B=16, round 1): moving 1 of every 4 exponentials here made all three attention kernels 3-6 % SLOWER
-// (fwd 131 -> 135 us, dK/dV 170 -> 178, dQa 153 -> 162): with three math warps per scheduler the loops are bound by the
-// dependent-issue latency of each warp's own instruction stream, not by MUFU throughput, and the polynomial adds ~9
-// instructions per element.  Kept behind AACONV_EX2_POLY_OF_4 (default 0 = every exponential on MUFU).
-__device__ __forceinline__ float ex2_poly(float x) {
-  x = fmaxf(x, -126.f);
-  const float t = x + 12582912.f;                    // 1.5 * 2^23: the integer part lands in the low mantissa bits
-  const float f = x - (t - 12582912.f);
-  float p = fmaf(f, 0.0551716610789299f, 0.2426111251115799f);
-  p = fmaf(f, p, 0.6932609677314758f);
-  p = fmaf(f, p, 0.9999280571937561f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(t) << 23));
-}
-#ifndef AACONV_EX2_POLY_OF_4
-#define AACONV_EX2_POLY_OF_4 0
-#endif
-// element u (0..3) of an unrolled group of four: the last EX2_POLY_OF_4 of them take the polynomial
-__device__ __forceinline__ float ex2_mixed(float x, int u) { return u >= 4 - AACONV_EX2_POLY_OF_4 ? ex2_poly(x) : ex2f(x); }
 
 }  // namespace tc
 

@@ -14,7 +14,6 @@ chexpert.py:90-123,504-518) loads strictly into this model and vice versa.  The 
 """
 from collections import OrderedDict
 
-import os
 
 import torch
 import torch.nn as nn
@@ -221,7 +220,7 @@ class BufferedDenseBlock(nn.ModuleDict):
                                         drop_rate=drop_rate))
         self.num_input_features, self.growth_rate, self.num_layers = num_input_features, growth_rate, num_layers
         self.out_channels = num_input_features + num_layers * growth_rate
-        self.inner_channels_last = os.environ.get('AACONV_INNER_CL', '1') != '0'   # AACONV_INNER_CL=0: NCHW inside the layers (A/B, profiles/r02_b_scaling.md)
+        self.inner_channels_last = True   # False: NCHW inside the layers, the route taken when slice_ok / cl_ok fail
         self.fused_eval = bool(fused_eval)
 
     def _forward_eval(self, feats, buf, slice_ok):

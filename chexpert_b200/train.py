@@ -40,7 +40,7 @@ class TrainStep:
 
     def __init__(self, device, size=320, precision='bf16', lr=1e-4, raw_labels=True, bucket_mb=25.0, seed=0,
                  autocast=True, channels_last=False, cuda_graph=False, graph_after=2, buffered=False, fused_prologue=False,
-                 batched_casts=True, arch='aadensenet121'):
+                 arch='aadensenet121'):
         torch.manual_seed(seed)
         self.device = torch.device(device)
         # arch (densenet.build_model): 'aadensenet121' or the reference's baseline 'densenet121'; the optimizer is the same for both
@@ -59,7 +59,7 @@ class TrainStep:
         # Multi-rank: the bucket all-reduces are captured too.  That needs the thread-local capture mode (NCCL's watchdog
         # thread polls events during the capture; the default global mode hung at 2 GPUs) and, at exit, the graph has to go
         # before the process group (release()).
-        # batched_casts: under autocast every cuDNN convolution casts its fp32 weight to bf16 in forward and its bf16 weight
+        # Weight casts: under autocast every cuDNN convolution casts its fp32 weight to bf16 in forward and its bf16 weight
         # gradient back to fp32 in backward -- ~360 three-microsecond kernels per step (9 % of the captured step).  Same
         # arithmetic, two launches: all conv weights are cast at once into bf16 shadows (torch._foreach_copy_), the model runs
         # on the shadows (torch.func.functional_call), and the shadows' gradients are cast back at once.
@@ -71,7 +71,7 @@ class TrainStep:
                     m._nbt_batched = True
                     self._nbt.append(m.num_batches_tracked)
         self._sh = None
-        if batched_casts and self.autocast:
+        if self.autocast:
             self._setup_shadows()
         # Gradient exchange (world > 1): packed and all-reduced after backward, inside the CUDA graph.  Exchanging under backward
         # measured slower on B200s under the CUDA graph (one hook per bucket: 2504 vs 2777 images/s at 2 GPUs; one hook per

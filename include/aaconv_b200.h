@@ -257,11 +257,9 @@ int aaconv_grad_cam(const void* x, int dtype, int B, int C, int h, int w, int64_
  *   aaconv_profile_end    stop; fills ms[i] = device time of launch i (its own start -> stop event) and the
  *                         '\n'-joined kernel names; returns the number of entries written (<= max_entries). */
 long long aaconv_launch_count(void);
-/* Debug hooks of the attention kernels (tools/attn_timeline.py, tools/attn_ablate.py); both default to off.
+/* Debug hooks of the attention kernels (tools/attn_timeline.py, tools/dbg_shape.py); both default to off.
  *   aaconv_debug_set_timeline  device buffer of 16 x 96 int64: clock64 stamps of one persistent CTA of the dQa kernel (NULL = off)
- *   aaconv_debug_set_mode      ablation bits: 1 no MUFU, 2 no global traffic after the first tiles, 4 no gradient MMAs,
- *                              8 no math, 32 dQa drain without the bulk store -- results are WRONG when bits 1-8 are set; 16 = soft
- *                              mbarrier timeouts (see aaconv_debug_read_mbar_log)                                          */
+ *   aaconv_debug_set_mode      16 = soft mbarrier timeouts (see aaconv_debug_read_mbar_log), 0 = off; other bits are ignored */
 void aaconv_debug_set_timeline(void* device_buffer);
 void aaconv_debug_set_mode(int mode);
 /*   aaconv_debug_read_mbar_log  with mode bit 16 set, a timed-out mbarrier wait in the small-value-width attention kernels is

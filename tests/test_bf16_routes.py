@@ -22,16 +22,6 @@ from tests.helpers import _bf16_grad_close, _bf16_output_close, _fp32_close, aut
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, 'chexpert_b200', 'csrc')
 
-# environment switches the library reads once per process; any of them moves shapes onto experiment routes
-_ENV = [k for k in os.environ if k in ('AACONV_AUG_BUILD', 'AACONV_REL_BWD', 'AACONV_DKV_SS') or k.startswith('AACONV_ABL_')]
-
-
-def gpu_route(f):
-    """GPU test on the production routes: skipped when an experiment switch is set"""
-    f = pytest.mark.skipif(bool(_ENV), reason=f'{", ".join(_ENV)} set: the library would run experiment routes, not these')(f)
-    return pytest.mark.gpu(f)
-
-
 # one entry per decision of the bf16 path: option -> kernels that run only on that option
 DECISIONS = {
     'builder': {'tc': ('aug_build_tc',), 'mma': ('aug_build_fwd',)},
@@ -116,7 +106,6 @@ EXCLUDED = {
     'out_fwd_f32': 'fp32 path only (the bf16 path applies out_proj in out_proj_fwd)',
     'out_bwd_data_f32': 'fp32 path only (the bf16 path fuses it into out_bwd_patch / out_bwd_data_patch)',
     'rel_weight_grad_f32': 'fp32 path only (the bf16 path uses rel_bwd / aug_rel_weight_grad)',
-    'aug_patch_bwd': 'no caller: superseded by out_bwd_patch / out_bwd_data_patch',
 }
 # kernels every bf16 case runs; boundary variants add their own below
 ALWAYS = ('out_proj_fwd',)
@@ -266,7 +255,7 @@ def _check_values(case, precision, y, w, dx, grads, x_bf16=False, fused=False, o
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize('precision', ['bf16', 'fp32'])
 @pytest.mark.parametrize('cid', list(CASES))
-@gpu_route
+@pytest.mark.gpu
 def test_route_matches_oracle(cid, precision):
     case = CASES[cid]
     if precision == 'fp32' and case.fp32_rejects:
@@ -286,7 +275,7 @@ BOUNDARY_VARIANTS = [(cid, prec, xb, fu) for cid in ('ffma_gemm', 'T3_288') for 
 
 
 @pytest.mark.parametrize('cid,precision,x_bf16,fused', BOUNDARY_VARIANTS)
-@gpu_route
+@pytest.mark.gpu
 def test_boundary_variant_matches_oracle(cid, precision, x_bf16, fused):
     case = CASES[cid]
     y, w, dx, grads, ran = _run(case, precision, x_bf16, fused)
@@ -299,7 +288,7 @@ def test_boundary_variant_matches_oracle(cid, precision, x_bf16, fused):
 # 2. contracts: backward twice on one saved block, partial gradients, batch independence
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize('cid', ['T2_512', 'dvh2_cc_k2', 'w128_outw_max'])
-@gpu_route
+@pytest.mark.gpu
 def test_backward_twice_is_bit_identical(cid):
     """The saved block is patched in place by backward (the backward-only columns of Qa) and the direct path clears its
     packed dq/dk/dv operand first: a retained graph must give the same gradients on the second call, bit for bit."""
@@ -325,7 +314,7 @@ PARTIAL = {'x_frozen': ('conv.weight', 'in_proj_qkv.weight', 'out_proj.weight', 
 
 @pytest.mark.parametrize('which', list(PARTIAL))
 @pytest.mark.parametrize('cid', ['dvh2_cc_k2', 'w128_outw_max'])
-@gpu_route
+@pytest.mark.gpu
 def test_partial_gradients_bf16(cid, which):
     """Gradients that are not requested are not written (NULL members of aaconv_param_grads) and come back None; the
     requested ones still meet the gate."""
@@ -345,7 +334,7 @@ def test_partial_gradients_bf16(cid, which):
 
 
 @pytest.mark.parametrize('cid', ['T2_512', 'dvh2_cc_k2'])
-@gpu_route
+@pytest.mark.gpu
 def test_batch_independence_bf16(cid):
     """Sample b of a batched call equals the same sample run alone, bit for bit (y and dx)."""
     case = CASES[cid]

@@ -1,6 +1,6 @@
 """Clock64 timeline of one persistent CTA (blockIdx.x == 40) of attn_bwd_dq_cc_kernel through the debug hook (GPU box).
 
-python tools/attn_timeline.py [ablation mode]  -> per-tile stamps relative to the first one (cycles); column = global tile
+python tools/attn_timeline.py [debug mode: 16 = soft mbarrier timeouts]  -> per-tile stamps relative to the first one (cycles); column = global tile
 index of the CTA (item * ntiles + tile).  Events (chexpert_b200/csrc/attn_cc.cu, TL_STAMP):
    0 S: loop top   1 S: K tile landed   2 S: slot free   3 S: issued+committed     4 G: loop top   5 G: dS ready   6 G: issued
    7 WG: waiting for S'   8 WG: S' ready   9 WG: S' in registers   10 WG: math done   11 WG: dS stored, arrived
